@@ -20,6 +20,9 @@ no data-path collective).
              bandwidth; `roofline_fp32` is the binding one (SURVEY 8d): algorithmic FLOPs / launch time against an FFMA
              microkernel measured in the same run.
 `cpu_baseline` the CPU oracle (fp32 build, OpenMP over envs, all host cores) on a bounded sample, rank 0, N = 1 only.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (rank 0's shard) as DIR/<name>.npy, so that
+two builds run with the same arguments, and therefore the same seeded inputs, can be compared output for output.
 """
 from __future__ import annotations
 
@@ -68,6 +71,43 @@ def algorithmic_flops(dims, depth, n_frames, I, L):
     f += Jp + 40 * nefc + nsolve * 4 * P + nmul * 4 * P + 3 * (2 * Jp + 6 * nefc)
     f += I * (2 * Jp + 12 * nefc + (2 + 3 * L) * 8 * nefc + 12 * nv) + 6 * nv + 40
     return n_frames * f
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# output dump
+# ------------------------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 << 20
+
+
+def host_copy(arrays, prefix=""):
+    """Flat {name: numpy array} copy of a (nested) dict of tensors / arrays; '/' in names becomes '.'."""
+    out = {}
+    for k, v in arrays.items():
+        name = prefix + k.replace("/", ".")
+        if isinstance(v, dict):
+            out.update(host_copy(v, name + "."))
+        else:
+            out[name] = v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v)
+    return out
+
+
+def dump_outputs(path, arrays, seed=0):
+    """Writes `arrays` (from `host_copy`) as <path>/<name>.npy: float32 stays float32, everything else becomes float64 (exact
+    for the integer outputs).  At most DUMP_BYTES in all: arrays are visited smallest first and each may use an equal share of
+    the budget left; those within their share are written whole, larger ones as a fixed, seeded sample of their elements
+    (flattened, in index order) that depends only on the seed and the array's size."""
+    flat = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES
+    order = sorted(flat, key=lambda k: (flat[k].nbytes, k))
+    for i, k in enumerate(order):
+        v = flat[k]
+        share = left // (len(order) - i)
+        if v.nbytes > share:
+            keep = max(1, share // v.itemsize)
+            v = v.reshape(-1)[np.unique(np.random.default_rng(seed).integers(0, v.size, size=keep))]
+        left -= v.nbytes
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -335,6 +375,8 @@ def run_ours(args):
     clocks = sampler.finish()
     launches = eng.launches - launches0
     done_frac = float(out["done"].mean())
+    # the next state and outputs of the last timed step, before the roofline loop below steps on
+    last = host_copy({**{k: a_st[k] for k in pkg("_lib").STATE_F + ("cur_frame", "sub_clip_frame")}, **out}) if args.dump_outputs and rank == 0 else None
 
     # ---- per-launch duration of the fused kernel for the roofline (events bracket every launch on its stream; the
     # clock sampler is off), and the solver counters of the executed-FLOP model ---------------------------------------
@@ -394,6 +436,8 @@ def run_ours(args):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     ms_total, e2e_ms_total, kernel_ms = red["ms"], red["e2e"], red["kern"]
     value = total * K / (ms_total * 1e-3)
     e2e_value = total * K / (e2e_ms_total * 1e-3)
@@ -495,7 +539,9 @@ def run_pair(args):
     qpos = np.tile(model.arrays["qpos0"], (B, 1)).astype(np.float32) + (1e-3 * rng.standard_normal((B, model.nq))).astype(np.float32)
     a, b = eng.alloc_state(B), eng.alloc_state(B)
     a["qpos"].copy_(torch.tensor(qpos, device=dev))
-    ctrl = torch.rand(W + K, B, model.nu, device=dev) * 2 - 1
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(67280421310721)  # torch's default CUDA seed: the controls this workload has always drawn, on every rank
+    ctrl = torch.rand(W + K, B, model.nu, generator=gen, device=dev) * 2 - 1
     stats = torch.zeros(B, 4, dtype=torch.int32, device=dev)
     host_ctrl = torch.empty(K, B, model.nu).pin_memory()
     host_ctrl.copy_(ctrl[W:].cpu())
@@ -519,6 +565,8 @@ def run_pair(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, host_copy({**{k: a[k] for k in lib.STATE_F}, "stats": stats}))
     dctrl = torch.empty(B, model.nu, device=dev)
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0.record()
@@ -572,6 +620,7 @@ def run_train(args, sgd: bool):
             if sgd:
                 host_metric.copy_(tr.learner.ws["metrics"], non_blocking=True)
             torch.cuda.current_stream().synchronize()
+        return data
     for _ in range(min(W, 3)):
         one(False)
     torch.cuda.synchronize()
@@ -585,9 +634,15 @@ def run_train(args, sgd: bool):
         one(False)
     e1.record()
     for _ in range(K):
-        one(True)
+        data = one(True)
     e2.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        # next_observation[:-1] is observation[1:] (one buffer): only its last row is new
+        last = {"rollout": dict(data, next_observation=data["next_observation"][-1:])}
+        if sgd:
+            last.update(policy=tr.learner.policy_params(), value=tr.learner.value_params(), loss_metrics=tr.learner.ws["metrics"])
+        dump_outputs(args.dump_outputs, host_copy(last))
     total = B * world * unroll
     launches = tr.rollout.launches + tr.sgd_launches - l0  # the captured update's kernels are counted per replay
 
@@ -613,7 +668,12 @@ def main():
     ap.add_argument("--envs-per-gpu", type=int, default=0, help="default: the workload's BASELINE.json size")
     ap.add_argument("--workload", default="rodent", choices=sorted(WORKLOADS), help="rodent = the config the metric is quoted on")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

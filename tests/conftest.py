@@ -12,7 +12,14 @@ for p in (ROOT, os.path.join(ROOT, "oracle")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
-REFERENCE = "/root/reference"  # present in the build container only; never required
+# a checkout of the original VNL-Brax-Imitation project (its MJCF assets): optional, the tests that read it skip without it
+REFERENCE = os.environ.get("VNL_REFERENCE")
+
+
+def reference_asset(name):
+    """Path of assets/<name> in the VNL_REFERENCE checkout, or None."""
+    path = os.path.join(REFERENCE, "assets", name) if REFERENCE else None
+    return path if path and os.path.exists(path) else None
 
 
 def pytest_configure(config):

@@ -1,12 +1,10 @@
 """G1-G3 of SURVEY Appendix G: the MJCF compiler and clip preprocessing against the ONLY numeric
 pins the reference holds -- the derived fields of clips/transform_snips_groom.p (committed as
 tests/golden/rodent_clip_golden.npz by tools/build_fixtures.py)."""
-import os
-
 import numpy as np
 import pytest
 
-from conftest import REFERENCE, pkg
+from conftest import pkg, reference_asset
 
 mjcf = pkg("mjcf")
 clipm = pkg("clip")
@@ -94,22 +92,44 @@ def test_velocity_pipeline_from_qpos(golden):
     assert np.abs(np.clip(v[:, 6:], -20, 20) - golden["joints_velocity"]).max() < 1e-5
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "assets", "rodent.xml")), reason="reference checkout absent")
+@pytest.mark.skipif(reference_asset("rodent.xml") is None, reason="no VNL_REFERENCE checkout of the original project")
 def test_packaged_model_is_the_compiled_reference_asset(rodent):
-    m2 = mjcf.load_rodent(os.path.join(REFERENCE, "assets", "rodent.xml"))
+    m2 = mjcf.load_rodent(reference_asset("rodent.xml"))
     m = rodent["model"]
     assert m2.body_names == m.body_names and m2.jnt_names == m.jnt_names
     for k, v in m.arrays.items():
         assert np.array_equal(np.asarray(m2.arrays[k]), np.asarray(v)), k
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "assets", "humanoid.xml")), reason="reference checkout absent")
 def test_humanoid_dims():
-    m = mjcf.load_humanoid(os.path.join(REFERENCE, "assets", "humanoid.xml"))
+    """humanoid.xml as compiled by tools/build_fixtures.py into the packaged model."""
+    m, _ = pkg("envs.humanoid").packaged_humanoid()
     d = pkg("model_blob").model_dims(m)
     assert (m.nbody, m.njnt, m.nq, m.nv, m.nu, m.na) == (17, 22, 28, 27, 21, 0)
     assert (d["ncon"], d["nlimit"], d["nefc"]) == (10, 21, 61)
     assert not m.eulerdamp and abs(m.timestep - 0.005) < 1e-12 and abs(m.impratio - 100.0) < 1e-9
+
+
+def test_load_humanoid_recipe(tmp_path):
+    """mjcf.load_humanoid on an MJCF file (envs/humanoid.py:40-54): compiled as written (no rescale), CG 6 x 6, eulerdamp
+    disabled even where the file enables it."""
+    import xml.etree.ElementTree as ET
+    xml = ('<mujoco model="h"><option timestep="0.005" impratio="100"><flag eulerdamp="enable"/></option><worldbody>'
+           '<geom name="floor" type="plane" size="5 5 0.1"/><body name="torso" pos="0 0 1.3"><freejoint name="root"/>'
+           '<geom name="t" type="capsule" fromto="0 -.07 0 0 .07 0" size=".07"/><body name="arm" pos="0 0.2 0">'
+           '<joint name="sh" type="hinge" axis="0 1 0" range="-60 60" damping="1"/>'
+           '<geom name="a" type="capsule" fromto="0 0 0 0 0 -0.3" size="0.04"/></body></body></worldbody>'
+           '<actuator><motor name="m" joint="sh" gear="40"/></actuator></mujoco>')
+    path = tmp_path / "h.xml"
+    path.write_text(xml)
+    m = mjcf.load_humanoid(str(path))
+    want = mjcf.compile_model(ET.fromstring(xml), name="humanoid", solver="cg", iterations=6, ls_iterations=6, eulerdamp=False)
+    assert not m.eulerdamp and abs(m.timestep - 0.005) < 1e-12 and abs(m.impratio - 100.0) < 1e-9
+    assert (m.solver, m.iterations, m.ls_iterations) == (want.solver, 6, 6) and (m.nq, m.nv, m.nu) == (8, 7, 1)
+    assert m.body_names == want.body_names and m.arrays.keys() == want.arrays.keys()
+    for k, v in want.arrays.items():
+        assert np.array_equal(np.asarray(m.arrays[k]), np.asarray(v)), k
+    assert np.allclose(m.arrays["jnt_range"][1], np.deg2rad([-60, 60]))  # degrees by default, as in humanoid.xml
 
 
 def test_rescale_rule_only_touches_explicit_attributes():

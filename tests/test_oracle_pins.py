@@ -190,7 +190,7 @@ def test_contact_parameter_mixing_of_the_rodent_floor_pairs(rodent):
     the floor (class collision_floor) keeps priority 0.  mj_contactParam / mjCPair::Compile: the higher priority wins outright,
     equal priority -> element-wise max friction and solmix-weighted solref.  The expectation is re-derived from the XML with
     an independent default resolver and compared with the compiled pair tables the kernel and the oracle consume."""
-    import os
+    from conftest import reference_asset
     m = rodent["model"]
     A = m.arrays
     n = len(A["pair_geom1"])
@@ -203,9 +203,9 @@ def test_contact_parameter_mixing_of_the_rodent_floor_pairs(rodent):
     assert np.allclose(A["pair_solref"], [0.005, 1.0]) and np.allclose(A["pair_solimp"], [0.9, 0.95, 0.001, 0.5, 2.0])
     assert set(np.round(fr[:, 0], 9).tolist()) <= {0.7, 1.5} and np.allclose(fr[:, 2], 0.005) and np.allclose(fr[:, 3], 0.0001)
     assert np.allclose(A["pair_includemargin"], 0.0)
-    path = os.path.join("/root/reference", "assets", "rodent.xml")
-    if not os.path.exists(path):
-        pytest.skip("reference checkout absent (GPU box): the XML-derived expectation needs rodent.xml")
+    path = reference_asset("rodent.xml")
+    if path is None:
+        pytest.skip("no VNL_REFERENCE checkout: the XML-derived expectation needs the original project's rodent.xml")
     prm = _xml_geom_params(ET.parse(path).getroot())
     npaw = 0
     for p in range(n):

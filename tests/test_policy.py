@@ -136,9 +136,8 @@ def test_torch_restatement_matches_numpy():
     np.testing.assert_allclose(r["log_prob"].numpy(), lp, atol=5e-4)
 
 
-def test_policy_refuses_to_run_without_gpu():
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+def test_policy_refuses_to_run_without_gpu(monkeypatch):
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)  # also on a GPU machine
     params = pol.init_params(np.random.default_rng(0), pol.param_shapes(**RODENT))
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         pol.IntentionPolicy(params)
