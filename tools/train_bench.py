@@ -5,6 +5,8 @@ GEMMs, Adam) with the gradient all-reduce over NCCL at N > 1 -- timed phase by p
     python tools/train_bench.py                                             # 1 GPU
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/train_bench.py
   env: ENVS (8192) MINIBATCHES (32) UPDATES (16) STEPS (2) GRAPH (1) X3 (0)
+       ENV=rodent|humanoid (rodent) -- the tracking env; CLIP=standing|moving (standing) -- the humanoid's packaged stand-in clip
+       (`envs.humanoid.packaged_humanoid(moving=...)`; the rodent always tracks its packaged clip)
   PROFILE=1 (with GRAPH=0): after the warm-up step, ONE eager minibatch update between cudaProfilerStart / Stop and exit -- the region
   `ncu --profile-from-start off --metrics gpu__time_duration.sum` lists (tools/make_profiles.py summarises the csv)."""
 import importlib
@@ -20,12 +22,18 @@ sys.path.insert(0, ROOT)
 import bench  # noqa: E402
 
 
-def build(dev, rank, world, B, unroll, nmb, nup, graph=True, x3=False):
+def build(dev, rank, world, B, unroll, nmb, nup, graph=True, x3=False, env_name="rodent", clip="standing"):
     P = lambda n: importlib.import_module("vnl-brax-imitation_b200." + n)
     sh, pol, lrn = P("sharding"), P("policy"), P("learner")
-    env = bench.make_env("rodent", str(dev))
+    if env_name not in ("rodent", "humanoid") or clip not in ("standing", "moving"):
+        raise ValueError("ENV must be rodent or humanoid, CLIP standing or moving")
+    if env_name == "humanoid":
+        model, ref = P("envs.humanoid").packaged_humanoid(moving=clip == "moving")
+        env = P("envs").HumanoidTracking(model=model, reference_clip=ref, device=str(dev))
+    else:
+        env = bench.make_env("rodent", str(dev))
     eng = env.engine
-    qpos, qvel, start = bench.workload_draws("rodent", env, B * world, *sh.shard_range(B * world, rank, world))
+    qpos, qvel, start = bench.workload_draws(env_name, env, B * world, *sh.shard_range(B * world, rank, world))
     s0 = env.reset_from(qpos, qvel, start)
     rng = np.random.default_rng(0)  # the same initial networks on every rank (key_policy / key_value are global, train.py:190-192)
     pp = pol.init_params(rng, pol.param_shapes(eng.traj_size, eng.obs_size, env.action_size))
@@ -48,7 +56,8 @@ def main():
     B, unroll = int(os.environ.get("ENVS", 8192)), 20
     nmb, nup, steps = int(os.environ.get("MINIBATCHES", 32)), int(os.environ.get("UPDATES", 16)), int(os.environ.get("STEPS", 2))
     graph, x3 = os.environ.get("GRAPH", "1") == "1", os.environ.get("X3", "0") == "1"
-    tr = build(dev, rank, world, B, unroll, nmb, nup, graph, x3)
+    env_name, clip = os.environ.get("ENV", "rodent"), os.environ.get("CLIP", "standing")
+    tr = build(dev, rank, world, B, unroll, nmb, nup, graph, x3, env_name, clip)
     ev = lambda: torch.cuda.Event(enable_timing=True)
     m = tr.training_step()  # warm-up: graph captures
     torch.cuda.synchronize()
@@ -86,12 +95,14 @@ def main():
     torch.cuda.synchronize()
     m = tr.learner.metrics_dict()
     red = sh.reduce_scalars(dict(ms=w0.elapsed_time(w1), ro=t_ro, sgd=t_sgd), op="max", device=dev)
-    res = {"config": "rodent PPO training_step: %d envs/GPU x unroll %d; SGD phase %d updates x %d minibatches of %d rows (%s, %s)" % (
-               B, unroll, nup, nmb, unroll * B // nmb, "3xTF32" if x3 else "TF32", "CUDA graph per minibatch update" if graph else "eager"),
+    what = env_name if env_name == "rodent" else "%s (%s clip)" % (env_name, clip)
+    res = {"config": "%s PPO training_step: %d envs/GPU x unroll %d; SGD phase %d updates x %d minibatches of %d rows (%s, %s)" % (
+               what, B, unroll, nup, nmb, unroll * B // nmb, "3xTF32" if x3 else "TF32", "CUDA graph per minibatch update" if graph else "eager"),
            "n_gpus": world, "training_env_steps_per_s": world * B * unroll * steps / (red["ms"] * 1e-3), "ms_per_training_step": red["ms"] / steps,
            "rollout_ms": red["ro"] / steps, "sgd_phase_ms": red["sgd"] / steps, "ms_per_minibatch_update": red["sgd"] / steps / (nup * nmb),
            "minibatch_updates_per_training_step": nup * nmb, "last_metrics": m}
-    flops = 6.0 * 1630397 * (unroll * B // nmb)  # fwd + bwd of both networks per minibatch update
+    nparams = sum(int(np.prod(s)) for s in tr.learner.shapes.values())  # 1630397 for the rodent
+    flops = 6.0 * nparams * (unroll * B // nmb)  # fwd + bwd of both networks per minibatch update
     res["sgd_tflops_dense"] = flops * nup * nmb / (red["sgd"] / steps * 1e-3) / 1e12
     if world > 1:
         import torch.distributed as dist

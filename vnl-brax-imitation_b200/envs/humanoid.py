@@ -22,6 +22,9 @@ from .rodent import METRIC_KEYS
 _DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "data")
 
 HUMANOID_ENV_ARGS = dict(solver="cg", iterations=6, ls_iterations=6)  # configs/env_config.yaml:1-8
+# the episode metrics of the reference env (humanoid.py:121-128): the rodent's without the appendage term; the step kernel still
+# writes all of METRIC_KEYS (column "rapp" unused)
+HUMANOID_METRIC_KEYS = tuple(k for k in METRIC_KEYS if k != "rapp")
 
 
 def packaged_humanoid(moving: bool = False):
@@ -94,11 +97,16 @@ class HumanoidTracking:
     def observation_size(self) -> int:
         return self._obs_size
 
+    @property
+    def metric_keys(self):
+        """Names of `State.metrics` (columns METRIC_KEYS.index(name) of the step kernel's metrics output)."""
+        return HUMANOID_METRIC_KEYS
+
     def _wrap(self, st, out) -> State:
         ps = PipelineState({k: st[k] for k in ("qpos", "qvel", "act", "qacc_warmstart", "xpos", "xquat", "subtree_com",
                                               "qfrc_actuator")})
         m = out["metrics"]
-        metrics = {k: m[:, i] for i, k in enumerate(METRIC_KEYS) if k != "rapp"}  # humanoid.py:121-128
+        metrics = {k: m[:, METRIC_KEYS.index(k)] for k in HUMANOID_METRIC_KEYS}
         info = dict(cur_frame=st["cur_frame"], sub_clip_frame=st["sub_clip_frame"], traj=out["traj"], termination_error=m[:, 6],
                     solver_stats=out["stats"])
         return State(ps, out["obs"], out["reward"], out["done"], metrics, info)

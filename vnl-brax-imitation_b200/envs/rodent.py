@@ -132,6 +132,11 @@ class RodentTracking:
         return self._obs_size
 
     @property
+    def metric_keys(self):
+        """Names of `State.metrics` (columns METRIC_KEYS.index(name) of the step kernel's metrics output)."""
+        return METRIC_KEYS
+
+    @property
     def backend(self) -> str:
         return "vnl_b200"
 

@@ -37,6 +37,9 @@ class Evaluator:
         self._Rollout = Rollout
         dev = eval_env.device
         f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)
+        # the env's metric names (the humanoid has no appendage term); the step kernel writes every column of METRIC_KEYS, all of
+        # which are folded, and only the env's own are reported
+        self.metric_keys = tuple(getattr(eval_env, "metric_keys", METRIC_KEYS))
         self.episode_metrics, self.active, self.episode_steps = f(self.B, len(METRIC_KEYS) + 1), f(self.B), f(self.B)
         self.rollout = None
 
@@ -65,11 +68,11 @@ class Evaluator:
         self.torch.cuda.synchronize(self.env.device)  # eval_metrics.active_episodes.block_until_ready()
         epoch_eval_time = time.time() - t0
         em = self.episode_metrics.cpu().numpy()
-        names = list(METRIC_KEYS) + ["reward"]
+        cols = [(n, METRIC_KEYS.index(n)) for n in self.metric_keys] + [("reward", len(METRIC_KEYS))]
         metrics = {}
         for fn in (np.mean, np.std):
             suffix = "_std" if fn is np.std else ""
-            metrics.update({f"eval/episode_{n}{suffix}": (float(fn(em[:, i])) if aggregate_episodes else em[:, i].copy()) for i, n in enumerate(names)})
+            metrics.update({f"eval/episode_{n}{suffix}": (float(fn(em[:, i])) if aggregate_episodes else em[:, i].copy()) for n, i in cols})
         metrics["eval/avg_episode_length"] = float(np.mean(self.episode_steps.cpu().numpy()))
         metrics["eval/epoch_eval_time"] = epoch_eval_time
         metrics["eval/sps"] = self._steps_per_unroll / epoch_eval_time

@@ -59,6 +59,36 @@ _POLICY_TENSORS = ("encoder/hidden_0/kernel", "encoder/hidden_0/bias", "encoder/
                    "decoder/hidden_2/kernel", "decoder/hidden_2/bias")
 
 
+def learner_shapes(policy_shapes: Dict[str, tuple], value_shapes: Dict[str, tuple]) -> Dict[str, tuple]:
+    """Shapes of the learner's tensors in flat-buffer order: "policy/" + _POLICY_TENSORS (the two encoder heads as one
+    [e2, 2 L] tensor), then "value/" + VALUE_ORDER."""
+    e2, L = policy_shapes["encoder/fc2_mean/kernel"]
+    shapes = {}
+    for k in _POLICY_TENSORS:
+        if k == "encoder/heads/kernel":
+            shapes["policy/" + k] = (e2, 2 * L)
+        elif k == "encoder/heads/bias":
+            shapes["policy/" + k] = (2 * L,)
+        else:
+            shapes["policy/" + k] = tuple(policy_shapes[k])
+    for k in VALUE_ORDER:
+        shapes["value/" + k] = tuple(value_shapes[k])
+    return shapes
+
+
+def flat_layout(shapes: Dict[str, tuple]):
+    """(offsets, row strides, total floats) of the flat parameter buffer.  Every tensor starts 16-byte aligned; a matrix whose
+    column count is not a multiple of 4 is a GEMM operand with rows of tk.ld4(cols) floats (the padding columns are never written
+    and stay 0 in parameters, gradients and Adam moments).  A single-column matrix (the value head [n, 1]) is read by row kernels,
+    not by TMA, and stays dense.  A 1-D tensor counts as one row."""
+    offsets, strides, off = {}, {}, 0
+    for k, s in shapes.items():
+        ld = tk.ld4(s[1]) if len(s) == 2 and s[1] > 1 else s[-1]
+        offsets[k], strides[k] = off, ld
+        off += tk.ld4(s[0] * ld if len(s) == 2 else s[0])
+    return offsets, strides, off
+
+
 class PPOLearner:
     """Flat parameter / gradient / Adam buffers + the workspaces of one minibatch shape (T x Bm rows).
 
@@ -88,43 +118,35 @@ class PPOLearner:
         self.obs, self.nu = k4 - self.L, nlog // 2
         self.widths = dict(e1=e1, e2=e2, d1=d1, d2=d2)
         self.vh = [value_params["hidden_0/kernel"].shape[1], value_params["hidden_1/kernel"].shape[1]]
-        if max(e1, e2, d1, d2) > 256 or self.nu > 32 or any(w % 4 for w in (e1, e2, d1, d2, self.obs, 2 * self.nu, self.L)):
+        # any width up to the kernels' limits: operands whose width is not a multiple of 4 floats get padded row strides (tk.ld4).
+        # The encoder heads [mean | logvar] are read as dense rows of 2 L floats by the reparameterisation kernels (L even), and the
+        # value MLP's swish passes are elementwise over dense rows (hidden widths multiples of 4).
+        if max(e1, e2, d1, d2) > 256 or self.nu > 32 or self.L % 2 or any(w % 4 for w in self.vh):
             raise ValueError("layer sizes not supported by the update kernels")
         # ---- flat buffers -------------------------------------------------------------------------------------------------
-        shapes = {}
-        for k in _POLICY_TENSORS:
-            if k == "encoder/heads/kernel":
-                shapes["policy/" + k] = (e2, 2 * self.L)
-            elif k == "encoder/heads/bias":
-                shapes["policy/" + k] = (2 * self.L,)
-            else:
-                shapes["policy/" + k] = tuple(P[k].shape)
-        for k in VALUE_ORDER:
-            shapes["value/" + k] = tuple(value_params[k].shape)
-        self.shapes, self.offsets, off = shapes, {}, 0
-        for k, s in shapes.items():
-            self.offsets[k] = off
-            off += (int(np.prod(s)) + 3) // 4 * 4  # 16-byte aligned tensors (TMA operands)
+        shapes = learner_shapes({k: v.shape for k, v in P.items()}, {k: v.shape for k, v in value_params.items()})
+        self.shapes = shapes
+        self.offsets, self.strides, off = flat_layout(shapes)
         self.nparams = off
         self.n_policy = self.offsets["value/hidden_0/kernel"]  # the policy bucket = [0, n_policy)
         z = lambda n, dt=t.float32: t.zeros(n, dtype=dt, device=dev)
         self.params, self.grads, self.m, self.v = z(off), z(off), z(off), z(off)
         self.step_dev, self.bc_dev = z(1, t.int32), z(2)
-        self.p = {k: self.params[self.offsets[k]:self.offsets[k] + int(np.prod(s))].view(*s) for k, s in shapes.items()}
-        self.g = {k: self.grads[self.offsets[k]:self.offsets[k] + int(np.prod(s))].view(*s) for k, s in shapes.items()}
+        self.p, self.g = self.views(self.params), self.views(self.grads)
         self.load_params(policy_params, value_params)
         # ---- workspaces of one minibatch ---------------------------------------------------------------------------------
         R, Bm, L, nu = self.R, self.Bm, self.L, self.nu
         f = lambda *s: t.zeros(*s, dtype=t.float32, device=dev)
-        self.ld_traj = (self.traj + 3) // 4 * 4
+        fp = lambda rows, n: tk.padded(rows, n, dev)  # TMA operands of any width (row stride tk.ld4(n))
+        self.ld_traj = tk.ld4(self.traj)
         W = self.widths
         self.ws = dict(
-            h0pre=f(R, e1), h0=f(R, e1), s0=f(R, 2), h1pre=f(R, e2), h1=f(R, e2), s1=f(R, 2), heads=f(R, 2 * L),
-            dec_in=f(R, L + self.obs), d0pre=f(R, d1), d0=f(R, d1), s2=f(R, 2), d1pre=f(R, d2), d1=f(R, d2), s3=f(R, 2), logits=f(R, 2 * nu),
-            vin=f(R + Bm, self.obs), v0pre=f(R + Bm, self.vh[0]), v0=f(R + Bm, self.vh[0]), v1pre=f(R + Bm, self.vh[1]), v1=f(R + Bm, self.vh[1]),
+            h0pre=fp(R, e1), h0=fp(R, e1), s0=f(R, 2), h1pre=fp(R, e2), h1=fp(R, e2), s1=f(R, 2), heads=f(R, 2 * L),
+            dec_in=fp(R, L + self.obs), d0pre=fp(R, d1), d0=fp(R, d1), s2=f(R, 2), d1pre=fp(R, d2), d1=fp(R, d2), s3=f(R, 2), logits=fp(R, 2 * nu),
+            vin=fp(R + Bm, self.obs), v0pre=f(R + Bm, self.vh[0]), v0=f(R + Bm, self.vh[0]), v1pre=f(R + Bm, self.vh[1]), v1=f(R + Bm, self.vh[1]),
             val=f(R + Bm), target_lp=f(R), ent=f(R), termination=f(R), rewards_s=f(R), vs=f(R), adv=f(R),
-            dlogits=f(R, 2 * nu), dval=f(R), dd1=f(R, d2), dd1pre=f(R, d2), dd0=f(R, d1), dd0pre=f(R, d1), ddec_in=f(R, L + self.obs),
-            dheads=f(R, 2 * L), dh1=f(R, e2), dh1pre=f(R, e2), dh0=f(R, e1), dh0pre=f(R, e1),
+            dlogits=fp(R, 2 * nu), dval=f(R), dd1=fp(R, d2), dd1pre=fp(R, d2), dd0=fp(R, d1), dd0pre=fp(R, d1), ddec_in=fp(R, L + self.obs),
+            dheads=f(R, 2 * L), dh1=fp(R, e2), dh1pre=fp(R, e2), dh0=fp(R, e1), dh0pre=fp(R, e1),
             dv1pre=f(R, self.vh[1]), dv0=f(R, self.vh[0]), dv0pre=f(R, self.vh[0]),
             metrics=f(8), scratch2=f(2))
         self.obs_mean, self.obs_std = f(self.obs), t.ones(self.obs, dtype=t.float32, device=dev)
@@ -138,6 +160,14 @@ class PPOLearner:
         del W
 
     # ---- parameters -----------------------------------------------------------------------------------------------------
+    def views(self, flat) -> Dict[str, "torch.Tensor"]:
+        """The tensors of a flat buffer (params, grads, m or v) in their flax shapes, as views with the layout's row strides."""
+        out = {}
+        for k, s in self.shapes.items():
+            o = self.offsets[k]
+            out[k] = flat[o:o + s[0] * self.strides[k]].view(s[0], self.strides[k])[:, :s[1]] if len(s) == 2 else flat[o:o + s[0]]
+        return out
+
     def load_params(self, policy_params, value_params) -> None:
         t = self.torch
         up = lambda a: t.as_tensor(np.ascontiguousarray(a, dtype=np.float32), device=self.device)
@@ -240,7 +270,6 @@ class PPOLearner:
         traj, obs = batch["traj"], batch["observation"]
         assert traj.shape == (R, self.ld_traj) and obs.shape == (R, self.obs) and traj.is_contiguous() and obs.is_contiguous()
         # ---- forward: policy --------------------------------------------------------------------------------------------
-        Ld = self.L + self.obs
         # The two networks are independent up to the loss rows and again after them: the value network runs on `self.branch`
         # (fork / join by stream events, which a CUDA-graph capture records as two parallel chains), so the policy's small,
         # latency-bound GEMMs (40-80 CTAs each) fill the SMs the value GEMMs leave idle between their waves.
@@ -248,45 +277,47 @@ class PPOLearner:
         V = lambda k: p["value/" + k]
         GV = lambda k: g["value/" + k]
         RB = R + Bm
+        ld = lambda x: x.stride(0)  # every row stride comes from the tensor (padded operands: tk.ld4 of the width)
+        nxt, vin, dec_in = batch["next_observation_last"], ws["vin"], ws["dec_in"]
         self.branch.wait_stream(main)
         with t.cuda.stream(self.branch):
             sb = tk.stream(self.params)
-            chk(L_.vnl_obs_normalize(ptr(obs), self.obs, R, self.obs, ptr(self.obs_mean), ptr(self.obs_std), ptr(ws["vin"]), self.obs, sb), "normalize")
-            chk(L_.vnl_obs_normalize(ptr(batch["next_observation_last"]), self.obs, Bm, self.obs, ptr(self.obs_mean), ptr(self.obs_std),
-                                     ptr(ws["vin"]) + 4 * R * self.obs, self.obs, sb), "normalize")
+            chk(L_.vnl_obs_normalize(ptr(obs), ld(obs), R, self.obs, ptr(self.obs_mean), ptr(self.obs_std), ptr(vin), ld(vin), sb), "normalize")
+            chk(L_.vnl_obs_normalize(ptr(nxt), ld(nxt), Bm, self.obs, ptr(self.obs_mean), ptr(self.obs_std), ptr(vin) + 4 * R * ld(vin), ld(vin), sb),
+                "normalize")
             # value forward (baseline rows + the Bm bootstrap rows in one pass)
-            self._fwd(ws["vin"], RB, V("hidden_0/kernel"), V("hidden_0/bias"), ws["v0pre"], act=ws["v0"])  # swish in the GEMM epilogue
+            self._fwd(vin, RB, V("hidden_0/kernel"), V("hidden_0/bias"), ws["v0pre"], act=ws["v0"])  # swish in the GEMM epilogue
             self._fwd(ws["v0"], RB, V("hidden_1/kernel"), V("hidden_1/bias"), ws["v1pre"], act=ws["v1"])
-            chk(L_.vnl_rowdot(ptr(ws["v1"]), self.vh[1], RB, self.vh[1], ptr(V("hidden_2/kernel")), ptr(V("hidden_2/bias")), ptr(ws["val"]), sb), "rowdot")
-        chk(L_.vnl_obs_normalize(ptr(obs), self.obs, R, self.obs, ptr(self.obs_mean), ptr(self.obs_std), ptr(ws["dec_in"]) + 4 * self.L, Ld, st), "normalize")
+            chk(L_.vnl_rowdot(ptr(ws["v1"]), ld(ws["v1"]), RB, self.vh[1], ptr(V("hidden_2/kernel")), ptr(V("hidden_2/bias")), ptr(ws["val"]), sb), "rowdot")
+        chk(L_.vnl_obs_normalize(ptr(obs), ld(obs), R, self.obs, ptr(self.obs_mean), ptr(self.obs_std), ptr(dec_in) + 4 * self.L, ld(dec_in), st), "normalize")
 
         def relu_ln(pre, name, out, stats):
             n = pre.shape[1]
-            chk(L_.vnl_relu_ln_fwd(ptr(pre), n, R, n, ptr(P(name + "/scale")), ptr(P(name + "/bias")), ptr(out), n, ptr(stats), st), "relu_ln_fwd")
+            chk(L_.vnl_relu_ln_fwd(ptr(pre), ld(pre), R, n, ptr(P(name + "/scale")), ptr(P(name + "/bias")), ptr(out), ld(out), ptr(stats), st), "relu_ln_fwd")
         self._fwd(traj, R, P("encoder/hidden_0/kernel"), P("encoder/hidden_0/bias"), ws["h0pre"])
         relu_ln(ws["h0pre"], "encoder/LayerNorm_0", ws["h0"], ws["s0"])
         self._fwd(ws["h0"], R, P("encoder/hidden_1/kernel"), P("encoder/hidden_1/bias"), ws["h1pre"])
         relu_ln(ws["h1pre"], "encoder/LayerNorm_1", ws["h1"], ws["s1"])
         self._fwd(ws["h1"], R, P("encoder/heads/kernel"), P("encoder/heads/bias"), ws["heads"])
-        chk(L_.vnl_reparam_fwd(ptr(ws["heads"]), ptr(batch["eps_z"]), R, self.L, ptr(ws["dec_in"]), Ld, st), "reparam")
-        self._fwd(ws["dec_in"], R, P("decoder/hidden_0/kernel"), P("decoder/hidden_0/bias"), ws["d0pre"])
+        chk(L_.vnl_reparam_fwd(ptr(ws["heads"]), ptr(batch["eps_z"]), R, self.L, ptr(dec_in), ld(dec_in), st), "reparam")
+        self._fwd(dec_in, R, P("decoder/hidden_0/kernel"), P("decoder/hidden_0/bias"), ws["d0pre"])
         relu_ln(ws["d0pre"], "decoder/LayerNorm_0", ws["d0"], ws["s2"])
         self._fwd(ws["d0"], R, P("decoder/hidden_1/kernel"), P("decoder/hidden_1/bias"), ws["d1pre"])
         relu_ln(ws["d1pre"], "decoder/LayerNorm_1", ws["d1"], ws["s3"])
         self._fwd(ws["d1"], R, P("decoder/hidden_2/kernel"), P("decoder/hidden_2/bias"), ws["logits"])
         # ---- loss -------------------------------------------------------------------------------------------------------------
-        chk(L_.vnl_ppo_rows(ptr(ws["logits"]), 2 * nu, ptr(batch["raw_action"]), ptr(batch["eps_ent"]), R, nu, ptr(batch["discount"]),
+        chk(L_.vnl_ppo_rows(ptr(ws["logits"]), ld(ws["logits"]), ptr(batch["raw_action"]), ptr(batch["eps_ent"]), R, nu, ptr(batch["discount"]),
                             ptr(batch["truncation"]), ptr(batch["reward"]), float(hp["reward_scaling"]), ptr(ws["target_lp"]), ptr(ws["ent"]),
                             ptr(ws["termination"]), ptr(ws["rewards_s"]), st), "ppo_rows")
         main.wait_stream(self.branch)  # join: GAE needs the values
         chk(self._gae.vnl_gae(self.T, Bm, ptr(batch["truncation"]), ptr(ws["termination"]), ptr(ws["rewards_s"]), ptr(ws["val"]), ptr(ws["val"]) + 4 * R,
                          float(hp["gae_lambda"]), float(hp["discounting"]), ptr(ws["vs"]), ptr(ws["adv"]), st), "gae")
-        chk(L_.vnl_ppo_loss_bwd(ptr(ws["logits"]), 2 * nu, ptr(batch["raw_action"]), ptr(batch["eps_ent"]), R, nu, ptr(ws["target_lp"]),
+        chk(L_.vnl_ppo_loss_bwd(ptr(ws["logits"]), ld(ws["logits"]), ptr(batch["raw_action"]), ptr(batch["eps_ent"]), R, nu, ptr(ws["target_lp"]),
                                 ptr(batch["log_prob"]), ptr(ws["ent"]), ptr(ws["adv"]), ptr(ws["vs"]), ptr(ws["val"]), float(hp["clipping_epsilon"]),
-                                float(hp["entropy_cost"]), int(bool(hp["normalize_advantage"])), ptr(ws["dlogits"]), 2 * nu, ptr(ws["dval"]),
+                                float(hp["entropy_cost"]), int(bool(hp["normalize_advantage"])), ptr(ws["dlogits"]), ld(ws["dlogits"]), ptr(ws["dval"]),
                                 ptr(ws["metrics"]), ptr(ws["scratch2"]), st), "ppo_loss_bwd")
         self.launches += 13  # row kernels of the forward pass and the loss (GEMMs count themselves)
-        colsum = lambda x, n, out, w=None: chk(L_.vnl_colsum(ptr(x), x.shape[1] if x.dim() == 2 else n, R, n, None if w is None else ptr(w), ptr(out),
+        colsum = lambda x, n, out, w=None: chk(L_.vnl_colsum(ptr(x), ld(x) if x.dim() == 2 else n, R, n, None if w is None else ptr(w), ptr(out),
                                                              tk.stream(self.params)), "colsum")
         # ---- backward ------------------------------------------------------------------------------------------------------------
         # Each network's backward is a serial CHAIN (dgrad -> activation backward -> dgrad ...) with LEAVES hanging off it (the weight
@@ -302,7 +333,7 @@ class PPOLearner:
 
         def value_head_leaves():
             sl = tk.stream(self.params)
-            chk(L_.vnl_colsum(ptr(ws["v1"]), self.vh[1], R, self.vh[1], ptr(ws["dval"]), ptr(GV("hidden_2/kernel")), sl), "colsum")
+            chk(L_.vnl_colsum(ptr(ws["v1"]), ld(ws["v1"]), R, self.vh[1], ptr(ws["dval"]), ptr(GV("hidden_2/kernel")), sl), "colsum")
             chk(L_.vnl_colsum(ptr(ws["dval"]), 1, R, 1, None, ptr(GV("hidden_2/bias")), sl), "colsum")
         leaf(self.leaf_v, main, value_head_leaves)
         with t.cuda.stream(self.branch):
@@ -312,13 +343,13 @@ class PPOLearner:
                                                 colsum(ws["dv1pre"], self.vh[1], GV("hidden_1/bias"))))
         with t.cuda.stream(self.branch):
             self._dgrad(ws["dv1pre"], R, V("hidden_1/kernel"), ws["dv0pre"], pre=ws["v0pre"], tmp=ws["dv0"])  # swish' in the GEMM epilogue
-            self._wgrad(ws["vin"], ws["dv0pre"], R, GV("hidden_0/kernel"))
+            self._wgrad(vin, ws["dv0pre"], R, GV("hidden_0/kernel"))
             colsum(ws["dv0pre"], self.vh[0], GV("hidden_0/bias"))
 
         # policy (its gradient bucket goes to the exchange as soon as it is complete)
         def relu_ln_bwd(dy, pre, stats, name, dpre, dense):  # also leaves the bias gradient of the dense layer in front (column sums of dpre)
             n = pre.shape[1]
-            chk(L_.vnl_relu_ln_bwd(ptr(dy), n, ptr(pre), n, ptr(stats), ptr(P(name + "/scale")), R, n, ptr(dpre), n, ptr(G(name + "/scale")),
+            chk(L_.vnl_relu_ln_bwd(ptr(dy), ld(dy), ptr(pre), ld(pre), ptr(stats), ptr(P(name + "/scale")), R, n, ptr(dpre), ld(dpre), ptr(G(name + "/scale")),
                                    ptr(G(name + "/bias")), ptr(G(dense + "/bias")), st), "relu_ln_bwd")
         lp = lambda fn: leaf(self.leaf_p, main, fn)
         lp(lambda: (self._wgrad(ws["d1"], ws["dlogits"], R, G("decoder/hidden_2/kernel")), colsum(ws["dlogits"], 2 * nu, G("decoder/hidden_2/bias"))))
@@ -327,10 +358,10 @@ class PPOLearner:
         lp(lambda: self._wgrad(ws["d0"], ws["dd1pre"], R, G("decoder/hidden_1/kernel")))
         self._dgrad(ws["dd1pre"], R, P("decoder/hidden_1/kernel"), ws["dd0"])
         relu_ln_bwd(ws["dd0"], ws["d0pre"], ws["s2"], "decoder/LayerNorm_0", ws["dd0pre"], "decoder/hidden_0")
-        lp(lambda: self._wgrad(ws["dec_in"], ws["dd0pre"], R, G("decoder/hidden_0/kernel")))
+        lp(lambda: self._wgrad(dec_in, ws["dd0pre"], R, G("decoder/hidden_0/kernel")))
         self._dgrad(ws["dd0pre"], R, P("decoder/hidden_0/kernel"), ws["ddec_in"])
         kl_coef = float(hp["kl_weight"]) / float(R * self.L)
-        chk(L_.vnl_heads_bwd(ptr(ws["ddec_in"]), Ld, ptr(ws["heads"]), ptr(batch["eps_z"]), R, self.L, kl_coef, ptr(ws["dheads"]),
+        chk(L_.vnl_heads_bwd(ptr(ws["ddec_in"]), ld(ws["ddec_in"]), ptr(ws["heads"]), ptr(batch["eps_z"]), R, self.L, kl_coef, ptr(ws["dheads"]),
                              ptr(ws["metrics"]) + 16, st), "heads_bwd")
         lp(lambda: (self._wgrad(ws["h1"], ws["dheads"], R, G("encoder/heads/kernel")), colsum(ws["dheads"], 2 * self.L, G("encoder/heads/bias"))))
         self._dgrad(ws["dheads"], R, P("encoder/heads/kernel"), ws["dh1"])

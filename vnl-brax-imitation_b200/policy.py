@@ -230,11 +230,14 @@ class PrecisePolicy:
         d2, nlog = params["decoder/hidden_2/kernel"].shape
         self.traj_size, self.obs_size, self.latent, self.action_size = traj, k4 - latent, latent, nlog // 2
         self.widths = (e1, e2, 2 * latent, d1, d2, nlog)
-        if max(self.widths) > 1024 or self.action_size > 32 or any(w % 4 for w in self.widths) or self.obs_size % 4 or latent % 4:
+        # GEMM operands of any width get padded row strides (tk.ld4); the encoder heads [mean | logvar] are read as dense rows of
+        # 2 latent floats by the reparameterisation kernel (latent even)
+        if max(self.widths) > 1024 or self.action_size > 32 or latent % 2:
             raise ValueError("layer sizes not supported by the fp32 policy path")
         f = lambda *sh: torch.zeros(*sh, dtype=torch.float32, device=self.device)
-        self.W = {"e0": f(traj, e1), "e1": f(e1, e2), "eh": f(e2, 2 * latent), "d0": f(k4, d1), "d1": f(d1, d2), "d2": f(d2, nlog)}
-        self.Wsplit = {k: (torch.empty_like(v), torch.empty_like(v)) for k, v in self.W.items()}
+        fp = lambda rows, n: tk.padded(rows, n, self.device)
+        self.W = {"e0": fp(traj, e1), "e1": fp(e1, e2), "eh": f(e2, 2 * latent), "d0": fp(k4, d1), "d1": fp(d1, d2), "d2": fp(d2, nlog)}
+        self.Wsplit = {k: (tk.like(v), tk.like(v)) for k, v in self.W.items()}
         self.b = {"e0": f(e1), "e1": f(e2), "eh": f(2 * latent), "d0": f(d1), "d1": f(d2), "d2": f(nlog)}
         self.ln = {k: (f(n), f(n)) for k, n in (("e0", e1), ("e1", e2), ("d0", d1), ("d1", d2))}
         self.blob_dev = self.W["e0"]  # an address that identifies "the parameters" for capturers (rollout.Rollout)
@@ -289,13 +292,14 @@ class PrecisePolicy:
         if B not in self.bufs:
             t = self.torch
             f = lambda *s: t.zeros(*s, dtype=t.float32, device=self.device)
+            fp = lambda rows, n: self.tk.padded(rows, n, self.device)  # GEMM operands: row stride tk.ld4(n)
             e1, e2, h2, d1, d2, nlog = self.widths
-            ld = (self.traj_size + 3) // 4 * 4
-            b = dict(traj=f(B, ld), idx=t.arange(B, dtype=t.int32, device=self.device), pre0=f(B, e1), h0=f(B, e1), pre1=f(B, e2), h1=f(B, e2),
-                     heads=f(B, h2), dec_in=f(B, self.latent + self.obs_size), pre2=f(B, d1), h2=f(B, d1), pre3=f(B, d2), h3=f(B, d2), st=f(B, 2))
+            b = dict(traj=f(B, self.tk.ld4(self.traj_size)), idx=t.arange(B, dtype=t.int32, device=self.device), pre0=fp(B, e1), h0=fp(B, e1), pre1=fp(B, e2),
+                     h1=fp(B, e2), heads=f(B, h2), dec_in=fp(B, self.latent + self.obs_size), pre2=fp(B, d1), h2=fp(B, d1), pre3=fp(B, d2), h3=fp(B, d2),
+                     st=f(B, 2))
             if self.x3:
                 for k in ("traj", "h0", "h1", "dec_in", "h2", "h3"):
-                    b[k + "_hi"], b[k + "_lo"] = t.empty_like(b[k]), t.empty_like(b[k])
+                    b[k + "_hi"], b[k + "_lo"] = self.tk.like(b[k]), self.tk.like(b[k])
             self.bufs[B] = b
         return self.bufs[B]
 
@@ -326,20 +330,21 @@ class PrecisePolicy:
         b, st, ptr = self._buffers(B), tk.stream(traj), (lambda x: None if x is None else x.data_ptr())
         chk = tk.check
         with t.cuda.device(self.device):
-            chk(L_.vnl_gather_rows(ptr(traj), 1, B, self.traj_size, ptr(b["idx"]), B, ptr(b["traj"]), b["traj"].shape[1], st), "pad traj")
-            Ld = self.latent + self.obs_size
-            chk(L_.vnl_obs_normalize(ptr(obs), self.obs_size, B, self.obs_size, ptr(self.obs_mean), ptr(self.obs_std), ptr(b["dec_in"]) + 4 * self.latent, Ld, st), "normalize")
-            relu_ln = lambda pre, name, dst: chk(L_.vnl_relu_ln_fwd(ptr(pre), pre.shape[1], B, pre.shape[1], ptr(self.ln[name][0]), ptr(self.ln[name][1]), ptr(dst), dst.shape[1], ptr(b["st"]), st), "relu_ln")
+            ld = lambda x: x.stride(0)  # row strides come from the tensors (padded operands: tk.ld4 of the width)
+            dec_in = b["dec_in"]
+            chk(L_.vnl_gather_rows(ptr(traj), 1, B, self.traj_size, ptr(b["idx"]), B, ptr(b["traj"]), ld(b["traj"]), st), "pad traj")
+            chk(L_.vnl_obs_normalize(ptr(obs), ld(obs), B, self.obs_size, ptr(self.obs_mean), ptr(self.obs_std), ptr(dec_in) + 4 * self.latent, ld(dec_in), st), "normalize")
+            relu_ln = lambda pre, name, dst: chk(L_.vnl_relu_ln_fwd(ptr(pre), ld(pre), B, pre.shape[1], ptr(self.ln[name][0]), ptr(self.ln[name][1]), ptr(dst), ld(dst), ptr(b["st"]), st), "relu_ln")
             self._dense(b, "traj", B, "e0", b["pre0"]); relu_ln(b["pre0"], "e0", b["h0"])
             self._dense(b, "h0", B, "e1", b["pre1"]); relu_ln(b["pre1"], "e1", b["h1"])
             self._dense(b, "h1", B, "eh", b["heads"])
-            chk(L_.vnl_reparam_fwd(ptr(b["heads"]), ptr(eps_z), B, self.latent, ptr(b["dec_in"]), Ld, st), "reparam")
+            chk(L_.vnl_reparam_fwd(ptr(b["heads"]), ptr(eps_z), B, self.latent, ptr(dec_in), ld(dec_in), st), "reparam")
             self._dense(b, "dec_in", B, "d0", b["pre2"]); relu_ln(b["pre2"], "d0", b["h2"])
             self._dense(b, "h2", B, "d1", b["pre3"]); relu_ln(b["pre3"], "d1", b["h3"])
             self._dense(b, "h3", B, "d2", out["logits"])
             if rand_action is not None and rand_action.dim() == 2:
                 rand_action = rand_action[0].contiguous()
-            chk(L_.vnl_policy_sample(ptr(out["logits"]), 2 * self.action_size, ptr(eps_a), ptr(rand_action), B, self.action_size, ptr(out["action"]),
+            chk(L_.vnl_policy_sample(ptr(out["logits"]), ld(out["logits"]), ptr(eps_a), ptr(rand_action), B, self.action_size, ptr(out["action"]),
                                      ptr(out["raw_action"]), ptr(out["log_prob"]), ptr(out["rand_log_prob"]) if rand_action is not None else None, st),
                 "policy_sample")
             if heads:

@@ -75,8 +75,9 @@ class Rollout:
         # carry: the next unroll starts from the last state / obs / traj / done
         self.done_prev.copy_(self.done[self.T - 1])
         if cur != self.cur:  # odd T: bring the state back to the buffer the (captured) launches read first
-            for k, v in self.state[cur].items():
-                self.state[self.cur][k].copy_(v)
+            # (its keys: without a clip index in the first state -- single-clip envs such as the humanoid -- there is no clip_id to restore)
+            for k, v in self.state[self.cur].items():
+                v.copy_(self.state[cur][k])
 
     def generate_unroll(self, eps_z=None, eps_a=None) -> Dict[str, "torch.Tensor"]:
         """One unroll; returns views of the transition buffers, named as brax's Transition (acting.py:50-57):

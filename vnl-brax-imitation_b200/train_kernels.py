@@ -58,17 +58,43 @@ def _ptrs(ts):
     return (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
 
 
-def split(x):
-    """(hi, lo) of the 3xTF32 scheme."""
+# ---- row strides of GEMM operands --------------------------------------------------------------------------------------
+# A TMA tensor map needs a row stride that is a multiple of 16 bytes, so every operand of `gemm` with a width n that is not a
+# multiple of 4 floats lives in a zeroed [rows, ld4(n)] buffer and is passed as its [rows, n] view: the kernels take the row
+# stride (`ld`) from `x.stride(0)`, and TMA never reads the padding columns (it fills out-of-range elements with zeros).  For
+# widths that are multiples of 4 the rule is the identity.
+def ld4(n: int) -> int:
+    """Row stride in floats of an operand of width n (also the 16-byte alignment of a tensor in a flat buffer)."""
+    return (int(n) + 3) // 4 * 4
+
+
+def padded(rows: int, n: int, device, dtype=None):
+    """Zeroed [rows, ld4(n)] buffer returned as its [rows, n] view (stride(0) == ld4(n))."""
     import torch
-    hi, lo = torch.empty_like(x), torch.empty_like(x)
-    check(lib().vnl_split_tf32(x.data_ptr(), x.numel(), hi.data_ptr(), lo.data_ptr(), stream(x)), "vnl_split_tf32")
-    return hi, lo
+    return torch.zeros(int(rows), ld4(n), dtype=dtype or torch.float32, device=device)[:, :int(n)]
+
+
+def like(x):
+    """Uninitialised tensor with x's shape AND strides (torch.empty_like of a row-padded view would be dense)."""
+    import torch
+    return torch.empty_strided(x.size(), x.stride(), dtype=x.dtype, device=x.device)
+
+
+def _extent(x) -> int:
+    """Floats from x's first to its last element (the padding between rows of a row-padded view included)."""
+    return 1 + sum((s - 1) * st for s, st in zip(x.shape, x.stride())) if x.numel() else 0
+
+
+def split(x):
+    """(hi, lo) of the 3xTF32 scheme, with x's row stride."""
+    hi, lo = like(x), like(x)
+    return split_into(x, hi, lo)
 
 
 def split_into(x, hi, lo):
-    """3xTF32 split into preallocated tensors (no allocation: CUDA-graph capturable)."""
-    check(lib().vnl_split_tf32(x.data_ptr(), x.numel(), hi.data_ptr(), lo.data_ptr(), stream(x)), "vnl_split_tf32")
+    """3xTF32 split into preallocated tensors of x's strides (no allocation: CUDA-graph capturable)."""
+    assert hi.stride() == x.stride() and lo.stride() == x.stride()
+    check(lib().vnl_split_tf32(x.data_ptr(), _extent(x), hi.data_ptr(), lo.data_ptr(), stream(x)), "vnl_split_tf32")
     return hi, lo
 
 
