@@ -51,6 +51,23 @@ def test_flat_layout_pads_only_the_humanoid_logit_kernel():
     assert [tk.ld4(w) for w in (55, 119, 42, 630, 232, 60)] == [56, 120, 44, 632, 232, 60]
 
 
+@pytest.mark.parametrize("dims", [(795, 232, 30), (630, 55, 21)], ids=["rodent", "humanoid"])
+def test_precise_policy_layout_is_the_learners_policy_bucket(dims, monkeypatch):
+    """PrecisePolicy's flat parameter buffer has the keys, offsets and row strides of the learner's policy bucket, and its size
+    n_policy (the policy is built on the CPU in one-pass TF32: laying out and packing needs no kernel)."""
+    import torch
+    lrn, pol = pkg("learner"), pkg("policy")
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: True)
+    shapes = pol.param_shapes(*dims)
+    p = pol.PrecisePolicy(pol.init_params(np.random.default_rng(0), shapes), device="cpu", precision="tf32")
+    offsets, strides, _ = lrn.flat_layout(lrn.learner_shapes(shapes, lrn.value_param_shapes(dims[1])))
+    bucket = [k for k in offsets if k.startswith("policy/")]
+    assert ["policy/" + k for k in p.p] == bucket and p.blob_dev.numel() == offsets["value/hidden_0/kernel"]
+    for k, x in p.p.items():
+        assert x.data_ptr() - p.blob_dev.data_ptr() == 4 * offsets["policy/" + k], k
+        assert x.dim() == 1 or x.stride(0) == strides["policy/" + k], k
+
+
 def test_learner_size_checks_keep_the_real_limits(monkeypatch):
     """Odd widths are accepted; what the kernels cannot do is refused before any device work."""
     import torch
@@ -240,6 +257,29 @@ def test_humanoid_updates_keep_the_padding_zero():
     assert torch.isfinite(L.params).all()
 
 
+@pytest.mark.gpu
+def test_precise_policy_parameters_equal_the_learners_policy_bucket():
+    """After two updates, `policy.load_params(learner.policy_params())` on a policy built from other parameters leaves its flat
+    parameter buffer equal to the learner's [0, n_policy) bit for bit, padding included, and its 3xTF32 splits equal to the split
+    of that bucket."""
+    import torch
+    lrn, pol, tk = pkg("learner"), pkg("policy"), pkg("train_kernels")
+    P, V = _params(4)
+    L = lrn.PPOLearner(P, V, T, BM, x3=True)
+    for step in range(2):
+        batch, mean, std = _batch(30 + step, L.policy_params(), L.value_params())
+        L.set_normalizer(mean, std)
+        L.update(batch)
+    p = pol.PrecisePolicy(_params(5)[0], "cuda:0")
+    p.load_params(L.policy_params())
+    torch.cuda.synchronize()
+    bits = lambda x: x.view(torch.int32)
+    bucket = L.params[:L.n_policy]
+    assert p.blob_dev.shape == bucket.shape and torch.equal(bits(p.blob_dev), bits(bucket))
+    for got, want in zip(p.blob_split, tk.split(bucket)):
+        assert torch.equal(bits(got), bits(want))
+
+
 # ---- the fp32-class rollout policy --------------------------------------------------------------------------------------
 def _policy_case(B, seed):
     import torch
@@ -254,16 +294,18 @@ def _policy_case(B, seed):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("B", [1, 130, 4096])
-def test_humanoid_precise_policy_matches_fp32_network(B):
-    """3xTF32 against the float64 network: logits 3e-5, log-prob 1e-3 (tests/test_policy.py)."""
+def test_humanoid_precise_policy_in_the_learners_layout_matches_fp32_network(B):
+    """3xTF32 against the float64 network: logits 3e-5, log-prob 1e-3 (tests/test_policy.py).  The logit kernel keeps its padded
+    row stride in the flat parameter buffer and both split buffers, and so does the cached forward's decoder input."""
     import torch
     pol = pkg("policy")
     params, x, mean, std = _policy_case(B, 40 + B % 7)
     p = pol.PrecisePolicy(params, "cuda:0", mean, std)
-    assert p.W["d2"].stride(0) == 44 and p.Wsplit["d2"][0].stride(0) == 44 and p.Wsplit["d2"][1].stride(0) == 44
+    k = "decoder/hidden_2/kernel"
+    assert p.p[k].stride(0) == 44 and p.splits[0][k].stride(0) == 44 and p.splits[1][k].stride(0) == 44
     act, out = p(x["traj"], x["obs"], x["eps_z"], x["eps_a"], x["rand"])
     torch.cuda.synchronize()
-    assert p.bufs[B]["dec_in"].stride(0) == 120 and out["logits"].is_contiguous()
+    assert p.bufs[B]["fwd"].ws["dec_in"].stride(0) == 120 and out["logits"].is_contiguous()
     d = lambda k: x[k].double()
     ref = pol.reference_forward(params, d("traj"), d("obs"), d("eps_z"), d("eps_a"), d("rand")[None].expand(B, -1), mean.double(), std.double())
     assert float((out["logits"].double() - ref["logits"]).abs().max()) < 3e-5 * max(1.0, float(ref["logits"].abs().max()))

@@ -21,7 +21,6 @@ from typing import Dict, Optional
 
 import numpy as np
 
-from . import policy as pol
 from . import ppo as gae_mod
 from . import train_kernels as tk
 
@@ -59,20 +58,27 @@ _POLICY_TENSORS = ("encoder/hidden_0/kernel", "encoder/hidden_0/bias", "encoder/
                    "decoder/hidden_2/kernel", "decoder/hidden_2/bias")
 
 
-def learner_shapes(policy_shapes: Dict[str, tuple], value_shapes: Dict[str, tuple]) -> Dict[str, tuple]:
-    """Shapes of the learner's tensors in flat-buffer order: "policy/" + _POLICY_TENSORS (the two encoder heads as one
-    [e2, 2 L] tensor), then "value/" + VALUE_ORDER."""
+def policy_widths(policy_params) -> Dict[str, int]:
+    """Layer widths of the intention network, read from its flax tree."""
+    traj, e1 = policy_params["encoder/hidden_0/kernel"].shape
+    e2, latent = policy_params["encoder/fc2_mean/kernel"].shape
+    k4, d1 = policy_params["decoder/hidden_0/kernel"].shape
+    d2, nlog = policy_params["decoder/hidden_2/kernel"].shape
+    return dict(traj=traj, obs=k4 - latent, latent=latent, e1=e1, e2=e2, d1=d1, d2=d2, nu=nlog // 2)
+
+
+def policy_tensor_shapes(policy_shapes: Dict[str, tuple]) -> Dict[str, tuple]:
+    """Shapes of _POLICY_TENSORS from the flax tree's: the two encoder heads as one [e2, 2 L] tensor."""
     e2, L = policy_shapes["encoder/fc2_mean/kernel"]
-    shapes = {}
-    for k in _POLICY_TENSORS:
-        if k == "encoder/heads/kernel":
-            shapes["policy/" + k] = (e2, 2 * L)
-        elif k == "encoder/heads/bias":
-            shapes["policy/" + k] = (2 * L,)
-        else:
-            shapes["policy/" + k] = tuple(policy_shapes[k])
-    for k in VALUE_ORDER:
-        shapes["value/" + k] = tuple(value_shapes[k])
+    heads = {"encoder/heads/kernel": (e2, 2 * L), "encoder/heads/bias": (2 * L,)}
+    return {k: heads[k] if k in heads else tuple(policy_shapes[k]) for k in _POLICY_TENSORS}
+
+
+def learner_shapes(policy_shapes: Dict[str, tuple], value_shapes: Dict[str, tuple]) -> Dict[str, tuple]:
+    """Shapes of the learner's tensors in flat-buffer order: "policy/" + _POLICY_TENSORS (policy_tensor_shapes), then
+    "value/" + VALUE_ORDER."""
+    shapes = {"policy/" + k: s for k, s in policy_tensor_shapes(policy_shapes).items()}
+    shapes.update(("value/" + k, tuple(value_shapes[k])) for k in VALUE_ORDER)
     return shapes
 
 
@@ -87,6 +93,103 @@ def flat_layout(shapes: Dict[str, tuple]):
         offsets[k], strides[k] = off, ld
         off += tk.ld4(s[0] * ld if len(s) == 2 else s[0])
     return offsets, strides, off
+
+
+def flat_views(flat, shapes: Dict[str, tuple]) -> Dict[str, "torch.Tensor"]:
+    """The tensors of a flat buffer laid out by flat_layout(shapes), as views in their shapes with the layout's row strides."""
+    offsets, strides, _ = flat_layout(shapes)
+    out = {}
+    for k, s in shapes.items():
+        o = offsets[k]
+        out[k] = flat[o:o + s[0] * strides[k]].view(s[0], strides[k])[:, :s[1]] if len(s) == 2 else flat[o:o + s[0]]
+    return out
+
+
+def pack_policy(views: Dict[str, "torch.Tensor"], policy_params: Dict[str, np.ndarray]) -> None:
+    """Copies a flax tree into the policy views (keyed by _POLICY_TENSORS), fc2_mean | fc2_logvar merged into the encoder heads."""
+    import torch
+    for k, x in views.items():
+        a = np.concatenate([policy_params[k.replace("heads", h)] for h in ("fc2_mean", "fc2_logvar")], -1) if "/heads/" in k else policy_params[k]
+        x.copy_(torch.as_tensor(np.ascontiguousarray(a, dtype=np.float32), device=x.device))
+
+
+def export_policy(views: Dict[str, "torch.Tensor"]) -> Dict[str, np.ndarray]:
+    """The flax tree of the policy views (keyed by _POLICY_TENSORS) on the host, the encoder heads split into fc2_mean | fc2_logvar."""
+    out = {}
+    for k, x in views.items():
+        a = x.detach().cpu().numpy()
+        if "/heads/" in k:
+            L = a.shape[-1] // 2
+            out[k.replace("heads", "fc2_mean")], out[k.replace("heads", "fc2_logvar")] = a[..., :L].copy(), a[..., L:].copy()
+        else:
+            out[k] = a.copy()
+    return out
+
+
+def splitk(K: int, x3: bool) -> int:
+    """Split-K of a product over K: 3xTF32 accumulates in chains of <= 8 K blocks of 32 (the tensor core's accumulator truncates)."""
+    return max(1, ((K + 31) // 32 + 7) // 8) if x3 else 1
+
+
+class PolicyForward:
+    """The intention network's forward pass over `rows` rows, for the learner's minibatch and policy.PrecisePolicy's rollout call.
+    Owns the workspaces `ws` (GEMM operands with tk.ld4 row strides) and, in 3xTF32, the hi / lo copies of each GEMM's left operand."""
+    LAUNCHES = 12  # normalise, 6 GEMMs (3xTF32 splits counted with their GEMM), 4 relu + LayerNorm, reparameterisation
+
+    @staticmethod
+    def check(w: Dict[str, int]) -> None:
+        # the forward kernels' limits: vnl_relu_ln_fwd rows of <= 1024 floats, vnl_policy_sample <= 32 actions; the encoder heads
+        # [mean | logvar] are read as dense rows of 2 latent floats by the reparameterisation kernels (latent even)
+        if max(w["e1"], w["e2"], 2 * w["latent"], w["d1"], w["d2"]) > 1024 or w["nu"] > 32 or w["latent"] % 2:
+            raise ValueError("layer sizes not supported by the policy forward kernels")
+
+    def __init__(self, widths: Dict[str, int], rows: int, device, x3: bool):
+        import torch
+        self.check(widths)
+        self.w = w = widths
+        self.rows, self.x3 = int(rows), bool(x3)
+        f = lambda n: torch.zeros(self.rows, n, dtype=torch.float32, device=device)
+        fp = lambda n: tk.padded(self.rows, n, device)
+        self.ws = dict(h0pre=fp(w["e1"]), h0=fp(w["e1"]), s0=f(2), h1pre=fp(w["e2"]), h1=fp(w["e2"]), s1=f(2), heads=f(2 * w["latent"]),
+                       dec_in=fp(w["latent"] + w["obs"]), d0pre=fp(w["d1"]), d0=fp(w["d1"]), s2=f(2), d1pre=fp(w["d2"]), d1=fp(w["d2"]), s3=f(2))
+        self.hilo = {}
+        if self.x3:
+            lhs = {k: self.ws[k] for k in ("h0", "h1", "dec_in", "d0", "d1")}
+            lhs["traj"] = torch.empty(self.rows, tk.ld4(w["traj"]), dtype=torch.float32, device=device)  # the callers' traj rows
+            self.hilo = {k: (tk.like(x), tk.like(x)) for k, x in lhs.items()}
+
+    def __call__(self, P, traj, obs, mean, std, eps_z, logits, splits=None) -> None:
+        """Enqueues normalise, e0, e1, heads, reparam, d0, d1, d2 (relu + LayerNorm after the hidden layers) on the current stream.
+        P: parameter views keyed by _POLICY_TENSORS; traj: rows of stride tk.ld4(traj); logits [rows, 2 nu]: the output, any row
+        stride; splits: (hi, lo) views of P in 3xTF32 (without them each GEMM splits its weight)."""
+        L_, ws, w, R, chk, st = tk.lib(), self.ws, self.w, self.rows, tk.check, tk.stream(logits)
+        ptr = lambda x: x.data_ptr()
+        ld = lambda x: x.stride(0)  # every row stride comes from the tensor (padded operands: tk.ld4 of the width)
+        lhs = dict(ws, traj=traj)
+
+        def dense(src, name, out):
+            x, W = lhs[src], P[name + "/kernel"]
+            K, N = W.shape
+            parts = None
+            if self.x3:
+                xs = tk.split_into(x, *self.hilo[src])
+                parts = (xs, (splits[0][name + "/kernel"], splits[1][name + "/kernel"]) if splits else tk.split(W))
+            tk.gemm(x, 0, W, 1, out, R, N, K, bias=P[name + "/bias"], x3=self.x3, splitk=splitk(K, self.x3), parts=parts)
+
+        def hidden(src, net, i, pre, out, stats):  # net/hidden_i, then relu + net/LayerNorm_i
+            pre, out, ln = ws[pre], ws[out], f"{net}/LayerNorm_{i}"
+            dense(src, f"{net}/hidden_{i}", pre)
+            chk(L_.vnl_relu_ln_fwd(ptr(pre), ld(pre), R, pre.shape[1], ptr(P[ln + "/scale"]), ptr(P[ln + "/bias"]), ptr(out), ld(out),
+                                   ptr(ws[stats]), st), "relu_ln_fwd")
+        dec_in = ws["dec_in"]
+        chk(L_.vnl_obs_normalize(ptr(obs), ld(obs), R, w["obs"], ptr(mean), ptr(std), ptr(dec_in) + 4 * w["latent"], ld(dec_in), st), "normalize")
+        hidden("traj", "encoder", 0, "h0pre", "h0", "s0")
+        hidden("h0", "encoder", 1, "h1pre", "h1", "s1")
+        dense("h1", "encoder/heads", ws["heads"])
+        chk(L_.vnl_reparam_fwd(ptr(ws["heads"]), ptr(eps_z), R, w["latent"], ptr(dec_in), ld(dec_in), st), "reparam")
+        hidden("dec_in", "decoder", 0, "d0pre", "d0", "s2")
+        hidden("d0", "decoder", 1, "d1pre", "d1", "s3")
+        dense("d1", "decoder/hidden_2", logits)
 
 
 class PPOLearner:
@@ -110,21 +213,17 @@ class PPOLearner:
                        gae_lambda=gae_lambda, clipping_epsilon=clipping_epsilon, normalize_advantage=normalize_advantage, kl_weight=kl_weight,
                        b1=adam_b1, b2=adam_b2, eps=adam_eps)
         self.x3 = bool(x3)
-        P = policy_params
-        self.traj, e1 = P["encoder/hidden_0/kernel"].shape
-        e2, self.L = P["encoder/fc2_mean/kernel"].shape
-        k4, d1 = P["decoder/hidden_0/kernel"].shape
-        d2, nlog = P["decoder/hidden_2/kernel"].shape
-        self.obs, self.nu = k4 - self.L, nlog // 2
-        self.widths = dict(e1=e1, e2=e2, d1=d1, d2=d2)
+        self.widths = w = policy_widths(policy_params)
+        self.traj, self.obs, self.L, self.nu = w["traj"], w["obs"], w["latent"], w["nu"]
+        e1, e2, d1, d2 = w["e1"], w["e2"], w["d1"], w["d2"]
         self.vh = [value_params["hidden_0/kernel"].shape[1], value_params["hidden_1/kernel"].shape[1]]
-        # any width up to the kernels' limits: operands whose width is not a multiple of 4 floats get padded row strides (tk.ld4).
-        # The encoder heads [mean | logvar] are read as dense rows of 2 L floats by the reparameterisation kernels (L even), and the
-        # value MLP's swish passes are elementwise over dense rows (hidden widths multiples of 4).
-        if max(e1, e2, d1, d2) > 256 or self.nu > 32 or self.L % 2 or any(w % 4 for w in self.vh):
+        # the backward kernels' limits (PolicyForward checks the forward's): any policy width up to 256 (tk.ld4 row strides), value
+        # hidden widths multiples of 4 (the swish passes are elementwise over dense rows)
+        if max(e1, e2, d1, d2) > 256 or any(v % 4 for v in self.vh):
             raise ValueError("layer sizes not supported by the update kernels")
+        self.fwd = PolicyForward(w, self.R, dev, self.x3)
         # ---- flat buffers -------------------------------------------------------------------------------------------------
-        shapes = learner_shapes({k: v.shape for k, v in P.items()}, {k: v.shape for k, v in value_params.items()})
+        shapes = learner_shapes({k: v.shape for k, v in policy_params.items()}, {k: v.shape for k, v in value_params.items()})
         self.shapes = shapes
         self.offsets, self.strides, off = flat_layout(shapes)
         self.nparams = off
@@ -132,17 +231,16 @@ class PPOLearner:
         z = lambda n, dt=t.float32: t.zeros(n, dtype=dt, device=dev)
         self.params, self.grads, self.m, self.v = z(off), z(off), z(off), z(off)
         self.step_dev, self.bc_dev = z(1, t.int32), z(2)
-        self.p, self.g = self.views(self.params), self.views(self.grads)
+        self.p, self.g = flat_views(self.params, shapes), flat_views(self.grads, shapes)
+        self.pp, self.gp = ({k: views["policy/" + k] for k in _POLICY_TENSORS} for views in (self.p, self.g))  # keyed as the policy's
         self.load_params(policy_params, value_params)
         # ---- workspaces of one minibatch ---------------------------------------------------------------------------------
         R, Bm, L, nu = self.R, self.Bm, self.L, self.nu
         f = lambda *s: t.zeros(*s, dtype=t.float32, device=dev)
         fp = lambda rows, n: tk.padded(rows, n, dev)  # TMA operands of any width (row stride tk.ld4(n))
         self.ld_traj = tk.ld4(self.traj)
-        W = self.widths
         self.ws = dict(
-            h0pre=fp(R, e1), h0=fp(R, e1), s0=f(R, 2), h1pre=fp(R, e2), h1=fp(R, e2), s1=f(R, 2), heads=f(R, 2 * L),
-            dec_in=fp(R, L + self.obs), d0pre=fp(R, d1), d0=fp(R, d1), s2=f(R, 2), d1pre=fp(R, d2), d1=fp(R, d2), s3=f(R, 2), logits=fp(R, 2 * nu),
+            self.fwd.ws, logits=fp(R, 2 * nu),
             vin=fp(R + Bm, self.obs), v0pre=f(R + Bm, self.vh[0]), v0=f(R + Bm, self.vh[0]), v1pre=f(R + Bm, self.vh[1]), v1=f(R + Bm, self.vh[1]),
             val=f(R + Bm), target_lp=f(R), ent=f(R), termination=f(R), rewards_s=f(R), vs=f(R), adv=f(R),
             dlogits=fp(R, 2 * nu), dval=f(R), dd1=fp(R, d2), dd1pre=fp(R, d2), dd0=fp(R, d1), dd0pre=fp(R, d1), ddec_in=fp(R, L + self.obs),
@@ -157,77 +255,47 @@ class PPOLearner:
         self.leaf_p, self.leaf_v = t.cuda.Stream(device=dev), t.cuda.Stream(device=dev)  # weight / bias gradients: leaves of the backward chains
         self._gae = gae_mod._bind(tk.lib())
         self._pending = None
-        del W
 
     # ---- parameters -----------------------------------------------------------------------------------------------------
-    def views(self, flat) -> Dict[str, "torch.Tensor"]:
-        """The tensors of a flat buffer (params, grads, m or v) in their flax shapes, as views with the layout's row strides."""
-        out = {}
-        for k, s in self.shapes.items():
-            o = self.offsets[k]
-            out[k] = flat[o:o + s[0] * self.strides[k]].view(s[0], self.strides[k])[:, :s[1]] if len(s) == 2 else flat[o:o + s[0]]
-        return out
+    @staticmethod
+    def _value(views) -> Dict[str, np.ndarray]:
+        return {k: views["value/" + k].detach().cpu().numpy().copy() for k in VALUE_ORDER}
 
     def load_params(self, policy_params, value_params) -> None:
-        t = self.torch
-        up = lambda a: t.as_tensor(np.ascontiguousarray(a, dtype=np.float32), device=self.device)
-        for k in _POLICY_TENSORS:
-            if k == "encoder/heads/kernel":
-                self.p["policy/" + k].copy_(t.cat([up(policy_params["encoder/fc2_mean/kernel"]), up(policy_params["encoder/fc2_logvar/kernel"])], 1))
-            elif k == "encoder/heads/bias":
-                self.p["policy/" + k].copy_(t.cat([up(policy_params["encoder/fc2_mean/bias"]), up(policy_params["encoder/fc2_logvar/bias"])]))
-            else:
-                self.p["policy/" + k].copy_(up(policy_params[k]))
+        pack_policy(self.pp, policy_params)
         for k in VALUE_ORDER:
-            self.p["value/" + k].copy_(up(value_params[k]))
+            self.p["value/" + k].copy_(self.torch.as_tensor(np.ascontiguousarray(value_params[k], dtype=np.float32), device=self.device))
 
     def set_normalizer(self, mean, std) -> None:
         self.obs_mean.copy_(self.torch.as_tensor(mean, dtype=self.torch.float32))
         self.obs_std.copy_(self.torch.as_tensor(std, dtype=self.torch.float32))
 
-    def _export(self, src, prefix) -> Dict[str, np.ndarray]:
-        out = {}
-        L = self.L
-        for k in (_POLICY_TENSORS if prefix == "policy/" else VALUE_ORDER):
-            a = src[prefix + k].detach().cpu().numpy()
-            if k == "encoder/heads/kernel":
-                out["encoder/fc2_mean/kernel"], out["encoder/fc2_logvar/kernel"] = a[:, :L].copy(), a[:, L:].copy()
-            elif k == "encoder/heads/bias":
-                out["encoder/fc2_mean/bias"], out["encoder/fc2_logvar/bias"] = a[:L].copy(), a[L:].copy()
-            else:
-                out[k] = a.copy()
-        return out
-
     def policy_params(self):
-        return self._export(self.p, "policy/")
+        return export_policy(self.pp)
 
     def value_params(self):
-        return self._export(self.p, "value/")
+        return self._value(self.p)
 
     def policy_grads(self):
-        return self._export(self.g, "policy/")
+        return export_policy(self.gp)
 
     def value_grads(self):
-        return self._export(self.g, "value/")
+        return self._value(self.g)
 
     # ---- the three products of a dense layer -------------------------------------------------------------------------------
-    def _splitk(self, K: int) -> int:
-        kb = (K + 31) // 32
-        return max(1, (kb + 7) // 8) if self.x3 else 1  # 3xTF32: accumulation chains of <= 8 K blocks (the accumulator truncates)
-
-    def _fwd(self, x, rows, W, b, out, act=None):  # out[rows, out] = x[rows, in] . W[in, out] + b;  act = swish(out) from the same epilogue
+    def _fwd(self, x, rows, W, b, out, act):  # out[rows, out] = x[rows, in] . W[in, out] + b;  act = swish(out) from the same epilogue
         K, N = W.shape
-        sk = self._splitk(K)
-        fused = act is not None and sk <= 1 and N % 32 == 0
+        sk = splitk(K, self.x3)
+        fused = sk <= 1 and N % 32 == 0
         tk.gemm(x, 0, W, 1, out, rows, N, K, bias=b, x3=self.x3, splitk=sk, epilogue=1 if fused else 0, aux=act if fused else None)
         self.launches += 1
-        if act is not None and not fused:
+        if not fused:
             tk.check(tk.lib().vnl_swish_fwd(out.data_ptr(), rows * N, act.data_ptr(), tk.stream(out)), "swish")
             self.launches += 1
 
     def _dgrad(self, dy, rows, W, out, pre=None, tmp=None):  # out[rows, in] = dy[rows, out] . W[in, out]^T  (* swish'(pre) in the epilogue)
         N, K = W.shape
-        sk = self._splitk(K)
+        sk = splitk(K, self.x3)
         if pre is None:
             tk.gemm(dy, 0, W, 0, out, rows, N, K, x3=self.x3, splitk=sk)
         elif sk <= 1 and N % 32 == 0:
@@ -242,12 +310,12 @@ class PPOLearner:
         M, N = gW.shape
         tiles = ((M + 127) // 128) * ((N + (127 if N > 64 else 63)) // (128 if N > 64 else 64))
         kb = (rows + 31) // 32
-        sk = max(self._splitk(rows), min(max(1, 148 // tiles), max(1, kb // 4)))
+        sk = max(splitk(rows, self.x3), min(max(1, 148 // tiles), max(1, kb // 4)))
         if N % 256 == 0 and M >= 256:  # 256 x 256 tiles (vnl_gemm.cu picks them when tiles x splits still fill the machine)
             tb = ((M + 255) // 256) * (N // 256)
             skb = min(max(1, 148 // tb), max(1, kb // 4))
             if tb * skb >= 96:
-                sk = max(self._splitk(rows), skb)
+                sk = max(splitk(rows, self.x3), skb)
         tk.gemm(x, 1, dy, 1, gW, M, N, rows, x3=self.x3, splitk=sk, zero=False)  # self.grads was zeroed at the top of the evaluation
         self.launches += 1
 
@@ -289,22 +357,8 @@ class PPOLearner:
             self._fwd(vin, RB, V("hidden_0/kernel"), V("hidden_0/bias"), ws["v0pre"], act=ws["v0"])  # swish in the GEMM epilogue
             self._fwd(ws["v0"], RB, V("hidden_1/kernel"), V("hidden_1/bias"), ws["v1pre"], act=ws["v1"])
             chk(L_.vnl_rowdot(ptr(ws["v1"]), ld(ws["v1"]), RB, self.vh[1], ptr(V("hidden_2/kernel")), ptr(V("hidden_2/bias")), ptr(ws["val"]), sb), "rowdot")
-        chk(L_.vnl_obs_normalize(ptr(obs), ld(obs), R, self.obs, ptr(self.obs_mean), ptr(self.obs_std), ptr(dec_in) + 4 * self.L, ld(dec_in), st), "normalize")
-
-        def relu_ln(pre, name, out, stats):
-            n = pre.shape[1]
-            chk(L_.vnl_relu_ln_fwd(ptr(pre), ld(pre), R, n, ptr(P(name + "/scale")), ptr(P(name + "/bias")), ptr(out), ld(out), ptr(stats), st), "relu_ln_fwd")
-        self._fwd(traj, R, P("encoder/hidden_0/kernel"), P("encoder/hidden_0/bias"), ws["h0pre"])
-        relu_ln(ws["h0pre"], "encoder/LayerNorm_0", ws["h0"], ws["s0"])
-        self._fwd(ws["h0"], R, P("encoder/hidden_1/kernel"), P("encoder/hidden_1/bias"), ws["h1pre"])
-        relu_ln(ws["h1pre"], "encoder/LayerNorm_1", ws["h1"], ws["s1"])
-        self._fwd(ws["h1"], R, P("encoder/heads/kernel"), P("encoder/heads/bias"), ws["heads"])
-        chk(L_.vnl_reparam_fwd(ptr(ws["heads"]), ptr(batch["eps_z"]), R, self.L, ptr(dec_in), ld(dec_in), st), "reparam")
-        self._fwd(dec_in, R, P("decoder/hidden_0/kernel"), P("decoder/hidden_0/bias"), ws["d0pre"])
-        relu_ln(ws["d0pre"], "decoder/LayerNorm_0", ws["d0"], ws["s2"])
-        self._fwd(ws["d0"], R, P("decoder/hidden_1/kernel"), P("decoder/hidden_1/bias"), ws["d1pre"])
-        relu_ln(ws["d1pre"], "decoder/LayerNorm_1", ws["d1"], ws["s3"])
-        self._fwd(ws["d1"], R, P("decoder/hidden_2/kernel"), P("decoder/hidden_2/bias"), ws["logits"])
+        self.fwd(self.pp, traj, obs, self.obs_mean, self.obs_std, batch["eps_z"], ws["logits"])
+        self.launches += PolicyForward.LAUNCHES
         # ---- loss -------------------------------------------------------------------------------------------------------------
         chk(L_.vnl_ppo_rows(ptr(ws["logits"]), ld(ws["logits"]), ptr(batch["raw_action"]), ptr(batch["eps_ent"]), R, nu, ptr(batch["discount"]),
                             ptr(batch["truncation"]), ptr(batch["reward"]), float(hp["reward_scaling"]), ptr(ws["target_lp"]), ptr(ws["ent"]),
@@ -316,7 +370,7 @@ class PPOLearner:
                                 ptr(batch["log_prob"]), ptr(ws["ent"]), ptr(ws["adv"]), ptr(ws["vs"]), ptr(ws["val"]), float(hp["clipping_epsilon"]),
                                 float(hp["entropy_cost"]), int(bool(hp["normalize_advantage"])), ptr(ws["dlogits"]), ld(ws["dlogits"]), ptr(ws["dval"]),
                                 ptr(ws["metrics"]), ptr(ws["scratch2"]), st), "ppo_loss_bwd")
-        self.launches += 13  # row kernels of the forward pass and the loss (GEMMs count themselves)
+        self.launches += 7  # row kernels of the value forward and the loss, and the zeroing (GEMMs and the policy forward count themselves)
         colsum = lambda x, n, out, w=None: chk(L_.vnl_colsum(ptr(x), ld(x) if x.dim() == 2 else n, R, n, None if w is None else ptr(w), ptr(out),
                                                              tk.stream(self.params)), "colsum")
         # ---- backward ------------------------------------------------------------------------------------------------------------

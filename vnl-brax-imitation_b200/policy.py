@@ -15,6 +15,8 @@ from typing import Dict, Optional, Sequence
 import numpy as np
 
 from . import _lib
+from . import learner as lrn
+from . import train_kernels as tk
 
 # flax parameter tree of IntentionNetwork, in the order vnl_policy_pack takes the arrays
 PARAM_ORDER = (
@@ -84,8 +86,20 @@ def init_params(rng: np.random.Generator, shapes: Dict[str, tuple], perturb: flo
     return out
 
 
+def alloc_outputs(policy, B: int, heads: bool = False):
+    """The output tensors of one call of `policy` (IntentionPolicy or PrecisePolicy: their `alloc_outputs` method) for B rows."""
+    t, nu = policy.torch, policy.action_size
+    f = lambda *s: t.empty(*s, dtype=t.float32, device=policy.device)
+    out = {"action": f(B, nu), "raw_action": f(B, nu), "logits": f(B, 2 * nu), "log_prob": f(B), "rand_log_prob": f(B)}
+    if heads:
+        out["z_mean"], out["z_logvar"] = f(B, policy.latent), f(B, policy.latent)
+    return out
+
+
 class IntentionPolicy:
     """Device-resident packed parameters + the `policy(traj, obs, draws)` call of the rollout."""
+
+    alloc_outputs = alloc_outputs
 
     def __init__(self, params: Dict[str, np.ndarray], device: str = "cuda:0", obs_mean=None, obs_std=None):
         import torch
@@ -95,16 +109,12 @@ class IntentionPolicy:
         self.torch = torch
         self.lib = _bind(_lib.load_library())
         self.device = torch.device(device)
-        sh = {k: params[k].shape for k in PARAM_ORDER}
-        traj, e1 = sh["encoder/hidden_0/kernel"]
-        e2, latent = sh["encoder/fc2_mean/kernel"]
-        k4, d1 = sh["decoder/hidden_0/kernel"]
-        d2, nlog = sh["decoder/hidden_2/kernel"]
-        self.dims = VnlPolicyDims(traj, k4 - latent, latent, e1, e2, d1, d2, nlog // 2)
+        w = lrn.policy_widths(params)
+        self.dims = VnlPolicyDims(**w)
         rc = self.lib.vnl_policy_check(ctypes.byref(self.dims))
         if rc:
             raise ValueError(f"layer sizes not supported by the policy kernel ({rc})")
-        self.traj_size, self.obs_size, self.latent, self.action_size = traj, k4 - latent, latent, nlog // 2
+        self.traj_size, self.obs_size, self.latent, self.action_size = w["traj"], w["obs"], w["latent"], w["nu"]
         self.load_params(params)
         self.set_normalizer(obs_mean, obs_std)
         self.launches = 0
@@ -156,14 +166,6 @@ class IntentionPolicy:
         """Called by a capturer (rollout.Rollout) once the operand addresses are baked into a CUDA graph."""
         self._norm_pinned = True
 
-    def alloc_outputs(self, B: int, heads: bool = False):
-        t, nu = self.torch, self.action_size
-        f = lambda *s: t.empty(*s, dtype=t.float32, device=self.device)
-        out = {"action": f(B, nu), "raw_action": f(B, nu), "logits": f(B, 2 * nu), "log_prob": f(B), "rand_log_prob": f(B)}
-        if heads:
-            out["z_mean"], out["z_logvar"] = f(B, self.latent), f(B, self.latent)
-        return out
-
     def __call__(self, traj, obs, eps_z, eps_a, rand_action=None, out: Optional[dict] = None, heads: bool = False):
         """One launch: (action [B,nu], extras) as `policy(trajectories, observations, key)` of ppo_networks.py:55-83.
         eps_z [B,latent], eps_a [B,nu]: standard-normal draws; rand_action [B,nu]: the uniform(-1,1) draw (optional).
@@ -208,40 +210,34 @@ class IntentionPolicy:
 class PrecisePolicy:
     """The same `policy(traj, obs, draws)` call as IntentionPolicy at the REFERENCE's precision (fp32 network, VERDICT r1 / ADVICE r1:
     the bf16 kernel's behaviour log-probs are 0.05-0.35 away from the fp32 network the learner re-evaluates, the size of the PPO
-    clip range).  Runs the learner's forward kernels: `vnl_gemm_tf32` on the tensor cores -- `precision="3xtf32"` (default, fp32-class:
-    log-probs within ~1e-4 of an fp32 / float64 evaluation) or `"tf32"` (one pass, what XLA runs for the reference on a GPU) -- plus
-    relu + LayerNorm, reparameterisation and `vnl_policy_sample`.  ~25 launches instead of one (0.25 ms at 8192 envs beside a 7.7 ms
-    env step), all CUDA-graph capturable: every buffer is allocated once per batch size, weights and their 3xTF32 splits are
-    refreshed in place by `load_params`.  Drop-in for IntentionPolicy in rollout.Rollout (same attributes and call)."""
+    clip range).  Runs the learner's forward pass (learner.PolicyForward: `vnl_gemm_tf32` in `precision="3xtf32"`, the default,
+    fp32-class: log-probs within ~1e-4 of an fp32 / float64 evaluation, or `"tf32"`, one pass as XLA runs the reference on a GPU), then
+    `vnl_policy_sample`.  ~25 launches instead of one (0.25 ms at 8192 envs beside a 7.7 ms env step), all CUDA-graph capturable: the
+    parameters are one flat buffer `blob_dev` laid out as the learner's policy bucket, refreshed in place with its 3xTF32 splits by
+    `load_params`; the workspaces are allocated once per batch size.  Drop-in for IntentionPolicy in rollout.Rollout."""
+
+    alloc_outputs = alloc_outputs
 
     def __init__(self, params: Dict[str, np.ndarray], device: str = "cuda:0", obs_mean=None, obs_std=None, precision: str = "3xtf32"):
         import torch
 
-        from . import train_kernels as tk
         if not torch.cuda.is_available():
             raise RuntimeError("vnl_b200 policy needs a CUDA device (sm_100a); there is no CPU fallback")
         if precision not in ("3xtf32", "tf32"):
             raise ValueError("precision must be '3xtf32' or 'tf32'")
-        self.torch, self.tk, self.x3 = torch, tk, precision == "3xtf32"
+        self.torch, self.x3 = torch, precision == "3xtf32"
         self.device = torch.device(device)
-        traj, e1 = params["encoder/hidden_0/kernel"].shape
-        e2, latent = params["encoder/fc2_mean/kernel"].shape
-        k4, d1 = params["decoder/hidden_0/kernel"].shape
-        d2, nlog = params["decoder/hidden_2/kernel"].shape
-        self.traj_size, self.obs_size, self.latent, self.action_size = traj, k4 - latent, latent, nlog // 2
-        self.widths = (e1, e2, 2 * latent, d1, d2, nlog)
-        # GEMM operands of any width get padded row strides (tk.ld4); the encoder heads [mean | logvar] are read as dense rows of
-        # 2 latent floats by the reparameterisation kernel (latent even)
-        if max(self.widths) > 1024 or self.action_size > 32 or latent % 2:
-            raise ValueError("layer sizes not supported by the fp32 policy path")
-        f = lambda *sh: torch.zeros(*sh, dtype=torch.float32, device=self.device)
-        fp = lambda rows, n: tk.padded(rows, n, self.device)
-        self.W = {"e0": fp(traj, e1), "e1": fp(e1, e2), "eh": f(e2, 2 * latent), "d0": fp(k4, d1), "d1": fp(d1, d2), "d2": fp(d2, nlog)}
-        self.Wsplit = {k: (tk.like(v), tk.like(v)) for k, v in self.W.items()}
-        self.b = {"e0": f(e1), "e1": f(e2), "eh": f(2 * latent), "d0": f(d1), "d1": f(d2), "d2": f(nlog)}
-        self.ln = {k: (f(n), f(n)) for k, n in (("e0", e1), ("e1", e2), ("d0", d1), ("d1", d2))}
-        self.blob_dev = self.W["e0"]  # an address that identifies "the parameters" for capturers (rollout.Rollout)
-        self.obs_mean, self.obs_std = f(self.obs_size), torch.ones(self.obs_size, dtype=torch.float32, device=self.device)
+        self.widths = w = lrn.policy_widths(params)
+        self.traj_size, self.obs_size, self.latent, self.action_size = w["traj"], w["obs"], w["latent"], w["nu"]
+        lrn.PolicyForward.check(w)
+        shapes = lrn.policy_tensor_shapes({k: v.shape for k, v in params.items()})
+        # The parameters keep ONE address for the life of the policy: `rollout.Rollout` captures `blob_dev.data_ptr()` into its CUDA
+        # graph, so `load_params` after a PPO update must land in the same buffer.
+        self.blob_dev = torch.zeros(lrn.flat_layout(shapes)[2], dtype=torch.float32, device=self.device)
+        self.p = lrn.flat_views(self.blob_dev, shapes)
+        self.blob_split = (tk.like(self.blob_dev), tk.like(self.blob_dev))  # its 3xTF32 hi / lo
+        self.splits = tuple(lrn.flat_views(x, shapes) for x in self.blob_split)
+        self.obs_mean, self.obs_std = (torch.full((self.obs_size,), v, dtype=torch.float32, device=self.device) for v in (0.0, 1.0))
         self._identity = True
         self.bufs = {}
         self.launches = 0
@@ -249,19 +245,9 @@ class PrecisePolicy:
         self.set_normalizer(obs_mean, obs_std)
 
     def load_params(self, params) -> None:
-        t = self.torch
-        up = lambda a: t.as_tensor(np.ascontiguousarray(a, dtype=np.float32), device=self.device)
-        self.W["e0"].copy_(up(params["encoder/hidden_0/kernel"])); self.b["e0"].copy_(up(params["encoder/hidden_0/bias"]))
-        self.W["e1"].copy_(up(params["encoder/hidden_1/kernel"])); self.b["e1"].copy_(up(params["encoder/hidden_1/bias"]))
-        self.W["eh"].copy_(t.cat([up(params["encoder/fc2_mean/kernel"]), up(params["encoder/fc2_logvar/kernel"])], 1))
-        self.b["eh"].copy_(t.cat([up(params["encoder/fc2_mean/bias"]), up(params["encoder/fc2_logvar/bias"])]))
-        for k, n in (("d0", "decoder/hidden_0"), ("d1", "decoder/hidden_1"), ("d2", "decoder/hidden_2")):
-            self.W[k].copy_(up(params[n + "/kernel"])); self.b[k].copy_(up(params[n + "/bias"]))
-        for k, n in (("e0", "encoder/LayerNorm_0"), ("e1", "encoder/LayerNorm_1"), ("d0", "decoder/LayerNorm_0"), ("d1", "decoder/LayerNorm_1")):
-            self.ln[k][0].copy_(up(params[n + "/scale"])); self.ln[k][1].copy_(up(params[n + "/bias"]))
+        lrn.pack_policy(self.p, params)
         if self.x3:
-            for k, w in self.W.items():
-                self.tk.split_into(w, *self.Wsplit[k])
+            tk.split_into(self.blob_dev, *self.blob_split)
 
     def set_normalizer(self, mean, std) -> None:
         """None = identity.  Tensors already on the device are ADOPTED when first given (shared with normalizer.RunningStatistics),
@@ -280,45 +266,10 @@ class PrecisePolicy:
     def pin_operands(self) -> None:
         self._norm_pinned = True
 
-    def alloc_outputs(self, B: int, heads: bool = False):
-        t, nu = self.torch, self.action_size
-        f = lambda *s: t.empty(*s, dtype=t.float32, device=self.device)
-        out = {"action": f(B, nu), "raw_action": f(B, nu), "logits": f(B, 2 * nu), "log_prob": f(B), "rand_log_prob": f(B)}
-        if heads:
-            out["z_mean"], out["z_logvar"] = f(B, self.latent), f(B, self.latent)
-        return out
-
-    def _buffers(self, B: int):
-        if B not in self.bufs:
-            t = self.torch
-            f = lambda *s: t.zeros(*s, dtype=t.float32, device=self.device)
-            fp = lambda rows, n: self.tk.padded(rows, n, self.device)  # GEMM operands: row stride tk.ld4(n)
-            e1, e2, h2, d1, d2, nlog = self.widths
-            b = dict(traj=f(B, self.tk.ld4(self.traj_size)), idx=t.arange(B, dtype=t.int32, device=self.device), pre0=fp(B, e1), h0=fp(B, e1), pre1=fp(B, e2),
-                     h1=fp(B, e2), heads=f(B, h2), dec_in=fp(B, self.latent + self.obs_size), pre2=fp(B, d1), h2=fp(B, d1), pre3=fp(B, d2), h3=fp(B, d2),
-                     st=f(B, 2))
-            if self.x3:
-                for k in ("traj", "h0", "h1", "dec_in", "h2", "h3"):
-                    b[k + "_hi"], b[k + "_lo"] = self.tk.like(b[k]), self.tk.like(b[k])
-            self.bufs[B] = b
-        return self.bufs[B]
-
-    def _dense(self, b, xname, rows, wname, out):
-        tk = self.tk
-        W = self.W[wname]
-        K, N = W.shape
-        parts, sk = None, 1
-        if self.x3:
-            tk.split_into(b[xname], b[xname + "_hi"], b[xname + "_lo"])
-            parts = ((b[xname + "_hi"], b[xname + "_lo"]), self.Wsplit[wname])
-            sk = max(1, ((K + 31) // 32 + 7) // 8)  # accumulation chains of <= 8 K blocks (the tensor core's accumulator truncates)
-        tk.gemm(b[xname], 0, W, 1, out, rows, N, K, bias=self.b[wname], x3=self.x3, splitk=sk, parts=parts)
-
     def __call__(self, traj, obs, eps_z, eps_a, rand_action=None, out: Optional[dict] = None, heads: bool = False):
         """(action [B, nu], extras) as IntentionPolicy.__call__; rand_action: the reference's ONE uniform draw of shape (nu,)
         (a [B, nu] tensor is accepted for compatibility: its first row is used)."""
-        t, tk = self.torch, self.tk
-        L_ = tk.lib()
+        t, L_, chk = self.torch, tk.lib(), tk.check
         B = traj.shape[0]
         for x, w in ((traj, self.traj_size), (obs, self.obs_size), (eps_z, self.latent)):
             if x.dtype != t.float32 or not x.is_contiguous() or x.shape != (B, w) or x.device != self.device:
@@ -327,28 +278,21 @@ class PrecisePolicy:
             out = self.alloc_outputs(B, heads)
         if B == 0:
             return out["action"], out
-        b, st, ptr = self._buffers(B), tk.stream(traj), (lambda x: None if x is None else x.data_ptr())
-        chk = tk.check
+        if B not in self.bufs:  # the forward's workspaces, and traj rows padded to tk.ld4 floats (a TMA row stride)
+            self.bufs[B] = dict(fwd=lrn.PolicyForward(self.widths, B, self.device, self.x3), idx=t.arange(B, dtype=t.int32, device=self.device),
+                                traj=t.zeros(B, tk.ld4(self.traj_size), dtype=t.float32, device=self.device))
+        b, st, ptr = self.bufs[B], tk.stream(traj), (lambda x: None if x is None else x.data_ptr())
         with t.cuda.device(self.device):
-            ld = lambda x: x.stride(0)  # row strides come from the tensors (padded operands: tk.ld4 of the width)
-            dec_in = b["dec_in"]
-            chk(L_.vnl_gather_rows(ptr(traj), 1, B, self.traj_size, ptr(b["idx"]), B, ptr(b["traj"]), ld(b["traj"]), st), "pad traj")
-            chk(L_.vnl_obs_normalize(ptr(obs), ld(obs), B, self.obs_size, ptr(self.obs_mean), ptr(self.obs_std), ptr(dec_in) + 4 * self.latent, ld(dec_in), st), "normalize")
-            relu_ln = lambda pre, name, dst: chk(L_.vnl_relu_ln_fwd(ptr(pre), ld(pre), B, pre.shape[1], ptr(self.ln[name][0]), ptr(self.ln[name][1]), ptr(dst), ld(dst), ptr(b["st"]), st), "relu_ln")
-            self._dense(b, "traj", B, "e0", b["pre0"]); relu_ln(b["pre0"], "e0", b["h0"])
-            self._dense(b, "h0", B, "e1", b["pre1"]); relu_ln(b["pre1"], "e1", b["h1"])
-            self._dense(b, "h1", B, "eh", b["heads"])
-            chk(L_.vnl_reparam_fwd(ptr(b["heads"]), ptr(eps_z), B, self.latent, ptr(dec_in), ld(dec_in), st), "reparam")
-            self._dense(b, "dec_in", B, "d0", b["pre2"]); relu_ln(b["pre2"], "d0", b["h2"])
-            self._dense(b, "h2", B, "d1", b["pre3"]); relu_ln(b["pre3"], "d1", b["h3"])
-            self._dense(b, "h3", B, "d2", out["logits"])
+            chk(L_.vnl_gather_rows(ptr(traj), 1, B, self.traj_size, ptr(b["idx"]), B, ptr(b["traj"]), b["traj"].stride(0), st), "pad traj")
+            b["fwd"](self.p, b["traj"], obs, self.obs_mean, self.obs_std, eps_z, out["logits"], self.splits)
             if rand_action is not None and rand_action.dim() == 2:
                 rand_action = rand_action[0].contiguous()
-            chk(L_.vnl_policy_sample(ptr(out["logits"]), ld(out["logits"]), ptr(eps_a), ptr(rand_action), B, self.action_size, ptr(out["action"]),
+            chk(L_.vnl_policy_sample(ptr(out["logits"]), out["logits"].stride(0), ptr(eps_a), ptr(rand_action), B, self.action_size, ptr(out["action"]),
                                      ptr(out["raw_action"]), ptr(out["log_prob"]), ptr(out["rand_log_prob"]) if rand_action is not None else None, st),
                 "policy_sample")
             if heads:
-                out["z_mean"].copy_(b["heads"][:, :self.latent]); out["z_logvar"].copy_(b["heads"][:, self.latent:])
+                h = b["fwd"].ws["heads"]
+                out["z_mean"].copy_(h[:, :self.latent]); out["z_logvar"].copy_(h[:, self.latent:])
         self.launches += 1
         return out["action"], out
 
