@@ -117,6 +117,11 @@ int vnl_adam_tick(int* step_dev, float b1, float b2, float* bc_dev, void* stream
 int vnl_adam(float* params, const float* grads, float* m, float* v, size_t n, float lr, float b1, float b2, float eps, int step, float grad_scale,
              const float* bc_dev, void* stream);
 
+/* dst[i] += src[i] for i < n (n <= 1024), each entry by one thread in launch order, no atomics: the running sum of the loss metrics
+ * row of vnl_ppo_loss_bwd over the minibatch updates of an epoch (brax `training_epoch` reports their mean).  Enqueued after every
+ * loss evaluation, inside the captured gradient graph, so the sum costs no host sync per update. */
+int vnl_metrics_accumulate(const float* src, int n, float* dst, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

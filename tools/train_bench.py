@@ -24,7 +24,7 @@ import bench  # noqa: E402
 
 def build(dev, rank, world, B, unroll, nmb, nup, graph=True, x3=False, env_name="rodent", clip="standing"):
     P = lambda n: importlib.import_module("vnl-brax-imitation_b200." + n)
-    sh, pol, lrn = P("sharding"), P("policy"), P("learner")
+    sh, trn = P("sharding"), P("train")
     if env_name not in ("rodent", "humanoid") or clip not in ("standing", "moving"):
         raise ValueError("ENV must be rodent or humanoid, CLIP standing or moving")
     if env_name == "humanoid":
@@ -32,17 +32,12 @@ def build(dev, rank, world, B, unroll, nmb, nup, graph=True, x3=False, env_name=
         env = P("envs").HumanoidTracking(model=model, reference_clip=ref, device=str(dev))
     else:
         env = bench.make_env("rodent", str(dev))
-    eng = env.engine
     qpos, qvel, start = bench.workload_draws(env_name, env, B * world, *sh.shard_range(B * world, rank, world))
     s0 = env.reset_from(qpos, qvel, start)
-    rng = np.random.default_rng(0)  # the same initial networks on every rank (key_policy / key_value are global, train.py:190-192)
-    pp = pol.init_params(rng, pol.param_shapes(eng.traj_size, eng.obs_size, env.action_size))
-    vp = lrn.init_value_params(rng, lrn.value_param_shapes(eng.obs_size))
-    stats = P("normalizer").RunningStatistics(eng.obs_size, str(dev))
-    policy = (pol.IntentionPolicy if os.environ.get("POLICY") == "bf16" else pol.PrecisePolicy)(pp, str(dev), stats.mean, stats.std)
-    ro = P("rollout").Rollout(env, policy, s0, unroll, 150.0, use_graph=True)
-    learner = lrn.PPOLearner(pp, vp, unroll, B // nmb, device=str(dev), x3=x3, clipping_epsilon=0.2, kl_weight=1e-4, learning_rate=6e-4)
-    tr = P("trainer").Trainer(env, policy, learner, ro, stats, nmb, nup, use_graph=graph, seed=rank)
+    # train()'s assembly (the same seeds: identical initial networks on every rank, the trainer's noise seeded by its rank)
+    cfg = dict(trn.DEFAULTS, num_envs=B * world, batch_size=B * world // nmb, unroll_length=unroll, num_minibatches=nmb, num_updates_per_batch=nup,
+               policy="bf16" if os.environ.get("POLICY") == "bf16" else "3xtf32")
+    tr = trn.Run(env, cfg, rank=rank, world_size=world, first_state=s0, use_graph=graph, learner_x3=x3, accumulate_metrics=False, evaluate=False).trainer
     return tr
 
 

@@ -389,6 +389,11 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
   }
 }
 
+// dst[i] += src[i]: one thread per entry of a short metrics row, so every sum is added in update order (no atomics)
+__global__ void metrics_accumulate_kernel(const float* __restrict__ src, int n, float* __restrict__ dst) {
+  for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] += src[i];
+}
+
 inline int grid_for(size_t n, int threads) {
   size_t b = (n + threads - 1) / threads;
   if (b > 148 * 8) b = 148 * 8;
@@ -551,6 +556,12 @@ int vnl_adam(float* params, const float* grads, float* m, float* v, size_t n, fl
   if (n == 0) return 0;
   const float bc1 = bc_dev ? 1.0f : 1.0f - powf(b1, (float)step), bc2 = bc_dev ? 1.0f : 1.0f - powf(b2, (float)step);
   adam_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(params, grads, m, v, n, lr, b1, b2, eps, bc1, bc2, grad_scale, bc_dev);
+  return rc();
+}
+
+int vnl_metrics_accumulate(const float* src, int n, float* dst, void* stream) {
+  if (!src || !dst || n <= 0 || n > 1024) return -1;
+  metrics_accumulate_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(src, n, dst);
   return rc();
 }
 

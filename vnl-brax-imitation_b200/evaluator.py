@@ -10,6 +10,7 @@ wrappers fused in the step launch, the unroll replayed as one CUDA graph), then 
 recorded [T, B] metrics / reward / done (one thread per env).  `deterministic_eval` = the policy's mode (eps_a = None)."""
 from __future__ import annotations
 
+import json
 import time
 from typing import Dict
 
@@ -42,6 +43,16 @@ class Evaluator:
         self.metric_keys = tuple(getattr(eval_env, "metric_keys", METRIC_KEYS))
         self.episode_metrics, self.active, self.episode_steps = f(self.B, len(METRIC_KEYS) + 1), f(self.B), f(self.B)
         self.rollout = None
+
+    def state_dict(self) -> Dict[str, object]:
+        """The two random streams (numpy for the reset draws, torch for the policy noise) and the accumulated eval walltime."""
+        return {"rng": np.array(json.dumps(self.rng.bit_generator.state)), "gen": self.gen.get_state().numpy().copy(),
+                "walltime": np.float64(self._eval_walltime)}
+
+    def load_state_dict(self, sd) -> None:
+        self.rng.bit_generator.state = json.loads(str(sd["rng"]))
+        self.gen.set_state(self.torch.as_tensor(np.asarray(sd["gen"]), dtype=self.torch.uint8).cpu())
+        self._eval_walltime = float(sd["walltime"])
 
     def _unroll(self):
         t = self.torch

@@ -198,6 +198,13 @@ class PPOLearner:
     `loss_and_grads(batch)` -> metrics; `apply_gradients()` = all-reduce (if a process group exists) + Adam; `update(batch)` =
     both.  `policy_params()` / `value_params()` export the flax trees (the rollout policy re-packs from them)."""
 
+    @staticmethod
+    def check(widths: Dict[str, int], value_hidden) -> None:
+        # the backward kernels' limits (PolicyForward checks the forward's): any policy width up to 256 (tk.ld4 row strides), value
+        # hidden widths multiples of 4 (the swish passes are elementwise over dense rows)
+        if max(widths["e1"], widths["e2"], widths["d1"], widths["d2"]) > 256 or any(v % 4 for v in value_hidden):
+            raise ValueError("layer sizes not supported by the update kernels")
+
     def __init__(self, policy_params: Dict[str, np.ndarray], value_params: Dict[str, np.ndarray], T: int, Bm: int, device: str = "cuda:0",
                  learning_rate: float = 6e-4, entropy_cost: float = 1e-4, discounting: float = 0.9, reward_scaling: float = 1.0,
                  gae_lambda: float = 0.95, clipping_epsilon: float = 0.3, normalize_advantage: bool = True, kl_weight: float = 1e-4,
@@ -217,10 +224,7 @@ class PPOLearner:
         self.traj, self.obs, self.L, self.nu = w["traj"], w["obs"], w["latent"], w["nu"]
         e1, e2, d1, d2 = w["e1"], w["e2"], w["d1"], w["d2"]
         self.vh = [value_params["hidden_0/kernel"].shape[1], value_params["hidden_1/kernel"].shape[1]]
-        # the backward kernels' limits (PolicyForward checks the forward's): any policy width up to 256 (tk.ld4 row strides), value
-        # hidden widths multiples of 4 (the swish passes are elementwise over dense rows)
-        if max(e1, e2, d1, d2) > 256 or any(v % 4 for v in self.vh):
-            raise ValueError("layer sizes not supported by the update kernels")
+        self.check(w, self.vh)
         self.fwd = PolicyForward(w, self.R, dev, self.x3)
         # ---- flat buffers -------------------------------------------------------------------------------------------------
         shapes = learner_shapes({k: v.shape for k, v in policy_params.items()}, {k: v.shape for k, v in value_params.items()})
@@ -281,6 +285,22 @@ class PPOLearner:
 
     def value_grads(self):
         return self._value(self.g)
+
+    # ---- checkpoint ------------------------------------------------------------------------------------------------------------
+    STATE_KEYS = ("params", "m", "v", "step_dev", "bc_dev")
+
+    def state_dict(self) -> Dict[str, np.ndarray]:
+        """The optimiser state on the host: the flat params and Adam moments (padding included) and the device step counter /
+        bias corrections."""
+        return {k: getattr(self, k).detach().cpu().numpy().copy() for k in self.STATE_KEYS}
+
+    def load_state_dict(self, sd) -> None:
+        """Copies into the existing buffers (captured SGD graphs keep their addresses)."""
+        for k in self.STATE_KEYS:
+            x, a = getattr(self, k), np.asarray(sd[k])
+            if tuple(a.shape) != tuple(x.shape) or a.dtype != np.dtype(str(x.dtype).replace("torch.", "")):
+                raise ValueError(f"learner state {k}: {a.dtype}{tuple(a.shape)} does not match this learner's {x.dtype}{tuple(x.shape)}")
+            x.copy_(self.torch.from_numpy(np.ascontiguousarray(a)))
 
     # ---- the three products of a dense layer -------------------------------------------------------------------------------
     def _fwd(self, x, rows, W, b, out, act):  # out[rows, out] = x[rows, in] . W[in, out] + b;  act = swish(out) from the same epilogue

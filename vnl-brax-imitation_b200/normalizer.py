@@ -60,6 +60,22 @@ class RunningStatistics:
         self.sums = f(2 * self.width + 1)
         self.std_min_value, self.std_max_value = float(std_min_value), float(std_max_value)
 
+    STATE_KEYS = ("count", "mean", "summed_variance", "std")
+
+    def state_dict(self):
+        """`RunningStatisticsState` on the host as numpy arrays."""
+        return {k: getattr(self, k).detach().cpu().numpy().copy() for k in self.STATE_KEYS}
+
+    def load_state_dict(self, sd) -> None:
+        """Copies into the existing tensors: a policy that adopted `mean` / `std` (and the graphs it was captured into) sees the
+        restored values."""
+        import numpy as np
+        for k in self.STATE_KEYS:
+            x, a = getattr(self, k), np.asarray(sd[k], dtype=np.float32)
+            if tuple(a.shape) != tuple(x.shape):
+                raise ValueError(f"normaliser {k}: shape {a.shape} does not match {tuple(x.shape)}")
+            x.copy_(self.torch.from_numpy(np.ascontiguousarray(a)))
+
     def update(self, batch, group_reduce: bool = True) -> None:
         """`running_statistics.update(state, batch, pmap_axis_name=...)`: batch [..., width] fp32 on this rank's GPU.
         `group_reduce=False` is brax's `pmap_axis_name=None` (statistics of this rank's batch only)."""

@@ -141,6 +141,36 @@ class Rollout:
         self.traj[0].copy_(first_state.info["traj"])
         self._fresh = True
 
+    # ---- checkpoint --------------------------------------------------------------------------------------------------
+    def state_dict(self) -> Dict[str, "np.ndarray"]:
+        """The carry into the next unroll, on the host: the env state the captured launches read first ("state/<key>", clip_id only
+        where the env has one), the AutoReset state ("first/<key>", "first_obs"), the obs / traj the next unroll starts from, the
+        episode step counters and the last step's done flags."""
+        carried = self.launches and not getattr(self, "_fresh", False)  # generate_unroll would copy obs[T] / traj[T] to row 0
+        h = lambda x: x.detach().cpu().numpy().copy()
+        out = {"state/" + k: h(v) for k, v in self.state[self.cur].items()}
+        out.update(("first/" + k, h(v)) for k, v in self.first.items())
+        out.update(first_obs=h(self.first_obs), obs=h(self.obs[self.T] if carried else self.obs[0]),
+                   traj=h(self.traj[self.T] if carried else self.traj[0]), steps=h(self.steps), done_prev=h(self.done_prev))
+        return out
+
+    def load_state_dict(self, sd) -> None:
+        """Copies a state_dict() into the existing buffers, as reset_to does: no address changes, so a captured unroll graph stays
+        valid, and the reset kernel does not run."""
+        import numpy as np
+        t = self.torch
+        dst = {"state/" + k: v for k, v in self.state[self.cur].items()}
+        dst.update(("first/" + k, v) for k, v in self.first.items())
+        dst.update(first_obs=self.first_obs, obs=self.obs[0], traj=self.traj[0], steps=self.steps, done_prev=self.done_prev)
+        if set(dst) != set(sd):
+            raise ValueError(f"rollout state keys differ: missing {sorted(set(dst) - set(sd))}, unexpected {sorted(set(sd) - set(dst))}")
+        for k, x in dst.items():
+            a = np.asarray(sd[k])
+            if tuple(a.shape) != tuple(x.shape) or a.dtype != np.dtype(str(x.dtype).replace("torch.", "")):
+                raise ValueError(f"rollout state {k}: {a.dtype}{tuple(a.shape)} does not match {x.dtype}{tuple(x.shape)}")
+            x.copy_(t.from_numpy(np.ascontiguousarray(a)))
+        self._fresh = True  # the next unroll starts from obs[0] / traj[0]
+
     # -----------------------------------------------------------------------------------------------------------------
     def _snapshot(self):
         s = self.state[self.cur]

@@ -8,7 +8,8 @@ from . import _lib
 
 TRAIN_EXPORTS = ("vnl_gemm_tf32", "vnl_gemm_tf32_ex", "vnl_split_tf32", "vnl_gather_rows", "vnl_obs_normalize", "vnl_relu_ln_fwd", "vnl_relu_ln_bwd",
                  "vnl_swish_fwd", "vnl_swish_bwd", "vnl_reparam_fwd", "vnl_heads_bwd", "vnl_colsum", "vnl_rowdot", "vnl_outer", "vnl_outer_swish_bwd", "vnl_gather_scalars",
-                 "vnl_ppo_rows", "vnl_ppo_loss_bwd", "vnl_adam_tick", "vnl_adam", "vnl_policy_sample", "vnl_eval_metrics")
+                 "vnl_ppo_rows", "vnl_ppo_loss_bwd", "vnl_adam_tick", "vnl_adam", "vnl_policy_sample", "vnl_eval_metrics",
+                 "vnl_metrics_accumulate")
 _bound = None
 
 
@@ -40,6 +41,7 @@ def lib():
         L.vnl_eval_metrics.argtypes = [i, i, i, v, v, v, v, v, v, v]
         L.vnl_adam_tick.argtypes = [v, f, f, v, v]
         L.vnl_adam.argtypes = [v, v, v, v, sz, f, f, f, f, i, f, v, v]
+        L.vnl_metrics_accumulate.argtypes = [v, i, v, v]
         _bound = L
     return _bound
 

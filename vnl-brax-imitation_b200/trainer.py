@@ -23,7 +23,9 @@ from . import train_kernels as tk
 
 class Trainer:
     def __init__(self, env, policy, learner: "lrn.PPOLearner", rollout, stats, num_minibatches: int, num_updates_per_batch: int,
-                 use_graph: bool = True, seed: int = 0):
+                 use_graph: bool = True, seed: int = 0, accumulate_metrics: bool = False):
+        """`accumulate_metrics`: sum the loss metrics of every minibatch update on the device (`vnl_metrics_accumulate`, one 8-float
+        launch per update, inside the captured gradient graph); `epoch_metrics()` returns their mean."""
         import torch
 
         self.torch = t = torch
@@ -53,6 +55,9 @@ class Trainer:
         self.discount_buf = f(self.T, self.B)
         self.env_steps = 0
         self.sgd_launches = 0
+        self.accumulate_metrics = bool(accumulate_metrics)
+        self.metric_sum = f(8) if self.accumulate_metrics else None
+        self._acc_updates0 = 0  # learner.updates when the sum was last reset
 
     # ---- one minibatch ----------------------------------------------------------------------------------------------------
     def _gather(self, tr):
@@ -73,10 +78,21 @@ class Trainer:
                  "vnl_gather_scalars")
         self.sgd_launches += 5
 
+    def _accumulate(self):
+        """metric_sum += this update's metrics row (enqueued right after loss_and_grads, on the same stream)."""
+        m = self.learner.ws["metrics"]
+        tk.check(tk.lib().vnl_metrics_accumulate(m.data_ptr(), m.numel(), self.metric_sum.data_ptr(), tk.stream(m)), "vnl_metrics_accumulate")
+        self.sgd_launches += 1
+
     def _minibatch(self, tr):
         n0 = self.learner.launches
         self._gather(tr)
-        self.learner.update(self.mb)
+        if self.accumulate_metrics:  # update() = loss_and_grads + apply_gradients, with the accumulation between them
+            self.learner.loss_and_grads(self.mb)
+            self._accumulate()
+            self.learner.apply_gradients()
+        else:
+            self.learner.update(self.mb)
         self.sgd_launches += self.learner.launches - n0
 
     def _capture(self, fn):
@@ -121,6 +137,8 @@ class Trainer:
                         def grads_only():
                             self._gather(tr)
                             lr.loss_and_grads(self.mb, exchange=False)
+                            if self.accumulate_metrics:
+                                self._accumulate()
                         self.graph = (self._capture(grads_only), self._capture(lambda: lr.apply_gradients(exchange=False, scale=1.0 / dist.get_world_size())))
                     lr.updates, self.sgd_launches = n0, l1  # the capture passes went through the host-side counters without executing
                     continue  # this minibatch was the warm-up run
@@ -143,3 +161,30 @@ class Trainer:
         self.policy.load_params(self.learner.policy_params())
         self.env_steps += self.B * self.T
         return self.learner.metrics_dict()
+
+    def epoch_metrics(self, reset: bool = True) -> Dict[str, float]:
+        """Mean of the loss metrics over every minibatch update since the last reset (brax `training_epoch`:
+        `tree_map(jnp.mean, loss_metrics)`), named as learner.metrics_dict names them.  Needs `accumulate_metrics=True`."""
+        if not self.accumulate_metrics:
+            raise RuntimeError("epoch_metrics needs a Trainer built with accumulate_metrics=True")
+        n = self.learner.updates - self._acc_updates0
+        out = self.learner.metrics_dict(self.metric_sum / max(n, 1))
+        if reset:
+            self.metric_sum.zero_()
+            self._acc_updates0 = self.learner.updates
+        return out
+
+    # ---- checkpoint ---------------------------------------------------------------------------------------------------------
+    def state_dict(self) -> Dict[str, object]:
+        """This rank's host-side training state: the noise generator and the counters (the device buffers live in the learner,
+        the normaliser and the rollout)."""
+        return {"gen": self.gen.get_state().numpy().copy(), "env_steps": self.env_steps, "updates": self.learner.updates}
+
+    def load_state_dict(self, sd) -> None:
+        t = self.torch
+        self.gen.set_state(t.as_tensor(sd["gen"], dtype=t.uint8).cpu())
+        self.env_steps = int(sd["env_steps"])
+        self.learner.updates = int(sd["updates"])
+        self._acc_updates0 = self.learner.updates
+        if self.metric_sum is not None:
+            self.metric_sum.zero_()
