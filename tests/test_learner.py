@@ -3,7 +3,7 @@ loss forward / backward through the intention policy network and the value MLP o
 torch-autograd restatement of `compute_ppo_intention_loss` (learner.reference_loss, float64).  Tolerances (written here):
   * 3xTF32 mode (the parity mode): every loss term 1e-5 absolute, every gradient tensor 1e-4 of its largest entry;
   * TF32 mode (one tensor-core pass, the reference's own GPU arithmetic): loss 2e-3, gradients 3e-2.
-The gradient exchange (two buckets, SUM + 1 / world folded into Adam = lax.pmean) is driven on CPU by a 2-rank gloo group."""
+The gradient exchange (one SUM all-reduce + 1 / world folded into Adam = lax.pmean) is driven on CPU by a 2-rank gloo group."""
 import os
 
 import numpy as np
@@ -171,17 +171,15 @@ def _gloo_worker(rank, world, port, q):
     dist.init_process_group("gloo", rank=rank, world_size=world)
     lrn = pkg("learner")
     g = torch.Generator().manual_seed(100 + rank)
-    n, n_first = 1000, 384
-    grads = torch.randn(n, generator=g)
+    grads = torch.randn(1000, generator=g)
     mine = grads.clone()
-    pending = lrn.start_bucket(dist, grads, 0, n_first)      # the policy bucket, asynchronous
-    scale = lrn.finish_buckets(dist, grads, n_first, pending)
+    scale = lrn.all_reduce_gradients(grads)
     q.put((rank, mine.numpy(), (grads * scale).numpy()))
     dist.destroy_process_group()
 
 
-def test_gradient_buckets_reduce_to_the_mean_over_ranks_gloo():
-    """world_size 2, gloo, CPU: the two-bucket exchange (async policy bucket + value bucket, scale folded into Adam) == lax.pmean."""
+def test_gradient_all_reduce_is_the_mean_over_ranks_gloo():
+    """world_size 2, gloo, CPU: the whole-buffer SUM all-reduce with its scale (folded into Adam) == lax.pmean."""
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
     q = ctx.Queue()

@@ -243,6 +243,75 @@ def test_epoch_metrics_are_the_mean_of_every_update(gpu_env):
     assert acc.sgd_launches - plain.sgd_launches == 2 * 2 * 4 and acc._launches_per_update == plain._launches_per_update + 1
 
 
+def _two_rank_worker(rank, port, q):
+    """One rank of a 2-rank gloo group on cuda:0: a training step of `train.Run` in graph mode, then in eager mode."""
+    import hashlib
+    import traceback
+
+    import torch
+    import torch.distributed as dist
+    try:
+        dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=2)
+        trn, rod = pkg("train"), pkg("envs.rodent")
+        model, clip = rod.packaged_rodent()  # as conftest's gpu_env: spawned processes do not see fixtures
+        env = pkg("envs").RodentTracking(reference_clip=clip, model=model, device="cuda:0", **rod.RODENT_ENV_ARGS)
+        out = {}
+        for graph in (True, False):
+            run = trn.Run(env, dict(trn.DEFAULTS, **SMALL), rank=rank, world_size=2, use_graph=graph, evaluate=False)
+            p0 = run.learner.params.clone()
+            run.trainer.training_step()
+            torch.cuda.synchronize()
+            p = run.learner.params.cpu().numpy()
+            out[graph] = dict(start=hashlib.sha256(p0.cpu().numpy().tobytes()).hexdigest(), params=hashlib.sha256(p.tobytes()).hexdigest(),
+                              moved=float(np.abs(p - p0.cpu().numpy()).max()), finite=bool(np.isfinite(p).all()),
+                              updates=run.learner.updates, graphs=len(run.trainer.graph or ()))
+        q.put((rank, out))
+        dist.destroy_process_group()
+    except BaseException:
+        q.put((rank, traceback.format_exc()))
+
+
+@pytest.mark.gpu
+def test_trainer_under_a_two_rank_process_group():
+    """Two ranks share cuda:0 through a gloo group over CUDA tensors (NCCL refuses two ranks on one device).  After one training
+    step both ranks hold the same parameters to the bit, in graph mode (a gradient graph, the eager all-reduce, an Adam graph)
+    and in eager mode."""
+    import queue
+    import socket
+
+    import torch.multiprocessing as mp
+    s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
+    ctx = mp.get_context("spawn")
+    q = ctx.Queue()
+    procs = [ctx.Process(target=_two_rank_worker, args=(r, port, q)) for r in range(2)]
+    for p in procs:
+        p.start()
+    res = {}
+    try:
+        for _ in procs:
+            r, got = q.get(timeout=900)
+            res[r] = got
+            if not isinstance(got, dict):
+                break  # a rank failed: the other may wait in a collective until it is terminated
+    except queue.Empty:
+        pass
+    finally:
+        for p in procs:
+            p.join(timeout=60)
+            if p.is_alive():
+                p.terminate()
+                p.join()
+    for r in (0, 1):
+        assert isinstance(res.get(r), dict), res
+    updates = SMALL["num_updates_per_batch"] * SMALL["num_minibatches"]
+    for graph in (True, False):
+        a, b = res[0][graph], res[1][graph]
+        assert a["start"] == b["start"] and a["params"] == b["params"], graph  # the same mean gradient on both ranks
+        assert a["params"] != a["start"] and a["moved"] > 1e-4 and a["finite"], graph
+        assert a["updates"] == b["updates"] == updates, graph
+        assert a["graphs"] == b["graphs"] == (2 if graph else 0), graph
+
+
 def _host(sd):
     return {k: np.asarray(v) for k, v in sd.items()}
 

@@ -99,16 +99,17 @@ def main():
     nparams = sum(int(np.prod(s)) for s in tr.learner.shapes.values())  # 1630397 for the rodent
     flops = 6.0 * nparams * (unroll * B // nmb)  # fwd + bwd of both networks per minibatch update
     res["sgd_tflops_dense"] = flops * nup * nmb / (red["sgd"] / steps * 1e-3) / 1e12
-    if world > 1:
+    if world > 1:  # the one whole-buffer gradient all-reduce the trainer issues per update, on its own
         import torch.distributed as dist
+        lrn = importlib.import_module("vnl-brax-imitation_b200.learner")
         g = tr.learner.grads
         for _ in range(5):
-            dist.all_reduce(g[:tr.learner.n_policy]); dist.all_reduce(g[tr.learner.n_policy:])
+            lrn.all_reduce_gradients(g)
         torch.cuda.synchronize()
         a0, a1 = ev(), ev()
         a0.record()
         for _ in range(50):
-            dist.all_reduce(g[:tr.learner.n_policy]); dist.all_reduce(g[tr.learner.n_policy:])
+            lrn.all_reduce_gradients(g)
         a1.record()
         torch.cuda.synchronize()
         us = sh.reduce_scalars(dict(us=a0.elapsed_time(a1) / 50 * 1e3), op="max", device=dev)["us"]

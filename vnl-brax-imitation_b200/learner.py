@@ -1,8 +1,8 @@
 """The PPO update on the GPU (SURVEY section 8 row f2): one `minibatch_step` of the reference (ppo_imitation/train.py:251-268) =
 `jax.value_and_grad(compute_ppo_intention_loss)` (ppo_imitation/intention_losses.py:91-202) over the intention policy network
 (intention_policy_network.py:20-105) and the brax value MLP (ppo_networks.py:114-118: hidden (1024, 1024), swish), the gradient
-`pmean` over devices (one NCCL all-reduce of the flat gradient buffer, overlapped: the policy bucket is reduced while the value
-network is still in its backward pass) and `optax.adam` (train.py:231-232).
+`pmean` over devices (`all_reduce_gradients`: one SUM all-reduce of the whole flat gradient buffer, 1 / world applied by Adam) and
+`optax.adam` (train.py:231-232).
 
 Everything numeric runs in libvnl_b200.so (include/vnl_train.h): the dense contractions on the tensor cores
 (`vnl_gemm_tf32`: tcgen05 kind::tf32, TMA tensor maps, K-major / MN-major operands so that forward, dgrad and wgrad need no
@@ -22,6 +22,7 @@ from typing import Dict, Optional
 import numpy as np
 
 from . import ppo as gae_mod
+from . import sharding
 from . import train_kernels as tk
 
 VALUE_ORDER = ("hidden_0/kernel", "hidden_0/bias", "hidden_1/kernel", "hidden_1/bias", "hidden_2/kernel", "hidden_2/bias")
@@ -195,8 +196,9 @@ class PolicyForward:
 class PPOLearner:
     """Flat parameter / gradient / Adam buffers + the workspaces of one minibatch shape (T x Bm rows).
 
-    `loss_and_grads(batch)` -> metrics; `apply_gradients()` = all-reduce (if a process group exists) + Adam; `update(batch)` =
-    both.  `policy_params()` / `value_params()` export the flax trees (the rollout policy re-packs from them)."""
+    `loss_and_grads(batch)` -> metrics; `apply_gradients(scale)` = Adam; `update(batch)` = loss_and_grads, all_reduce_gradients
+    (if a process group exists), apply_gradients.  `policy_params()` / `value_params()` export the flax trees (the rollout policy
+    re-packs from them)."""
 
     @staticmethod
     def check(widths: Dict[str, int], value_hidden) -> None:
@@ -231,7 +233,7 @@ class PPOLearner:
         self.shapes = shapes
         self.offsets, self.strides, off = flat_layout(shapes)
         self.nparams = off
-        self.n_policy = self.offsets["value/hidden_0/kernel"]  # the policy bucket = [0, n_policy)
+        self.n_policy = self.offsets["value/hidden_0/kernel"]  # the policy tensors = [0, n_policy)
         z = lambda n, dt=t.float32: t.zeros(n, dtype=dt, device=dev)
         self.params, self.grads, self.m, self.v = z(off), z(off), z(off), z(off)
         self.step_dev, self.bc_dev = z(1, t.int32), z(2)
@@ -254,11 +256,9 @@ class PPOLearner:
         self.obs_mean, self.obs_std = f(self.obs), t.ones(self.obs, dtype=t.float32, device=dev)
         self.updates = 0
         self.launches = 0
-        self.side = t.cuda.Stream(device=dev)    # gradient exchange of the policy bucket
         self.branch = t.cuda.Stream(device=dev)  # the value network's forward / backward, beside the policy's
         self.leaf_p, self.leaf_v = t.cuda.Stream(device=dev), t.cuda.Stream(device=dev)  # weight / bias gradients: leaves of the backward chains
         self._gae = gae_mod._bind(tk.lib())
-        self._pending = None
 
     # ---- parameters -----------------------------------------------------------------------------------------------------
     @staticmethod
@@ -340,7 +340,7 @@ class PPOLearner:
         self.launches += 1
 
     # ---- one loss + gradient evaluation ------------------------------------------------------------------------------------
-    def loss_and_grads(self, batch: Dict[str, "torch.Tensor"], exchange: bool = True):
+    def loss_and_grads(self, batch: Dict[str, "torch.Tensor"]):
         """batch (time-major, contiguous fp32 CUDA tensors, R = T * Bm rows):
         traj [R, ld_traj] (row stride padded to a multiple of 4: vnl_gather_rows does it), observation [R, obs],
         next_observation_last [Bm, obs], reward / discount / truncation / log_prob [R], raw_action [R, nu],
@@ -420,7 +420,7 @@ class PPOLearner:
             self._wgrad(vin, ws["dv0pre"], R, GV("hidden_0/kernel"))
             colsum(ws["dv0pre"], self.vh[0], GV("hidden_0/bias"))
 
-        # policy (its gradient bucket goes to the exchange as soon as it is complete)
+        # policy
         def relu_ln_bwd(dy, pre, stats, name, dpre, dense):  # also leaves the bias gradient of the dense layer in front (column sums of dpre)
             n = pre.shape[1]
             chk(L_.vnl_relu_ln_bwd(ptr(dy), ld(dy), ptr(pre), ld(pre), ptr(stats), ptr(P(name + "/scale")), R, n, ptr(dpre), ld(dpre), ptr(G(name + "/scale")),
@@ -444,42 +444,17 @@ class PPOLearner:
         self._dgrad(ws["dh1pre"], R, P("encoder/hidden_1/kernel"), ws["dh0"])
         relu_ln_bwd(ws["dh0"], ws["h0pre"], ws["s0"], "encoder/LayerNorm_0", ws["dh0pre"], "encoder/hidden_0")
         self._wgrad(traj, ws["dh0pre"], R, G("encoder/hidden_0/kernel"))
-        main.wait_stream(self.leaf_p)  # the policy bucket is complete
-        self._pending = None
-        if exchange:
-            self._policy_bucket_ready()
-        main.wait_stream(self.branch)  # join: all gradients are in self.grads
+        main.wait_stream(self.leaf_p)  # join: all gradients are in self.grads
+        main.wait_stream(self.branch)
         main.wait_stream(self.leaf_v)
         self.launches += 12  # row kernels of the backward pass
         return ws["metrics"]
 
-    # ---- gradient exchange + optimiser ---------------------------------------------------------------------------------------
-    def _dist(self):
-        import torch.distributed as dist
-        return dist if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1 else None
-
-    def _policy_bucket_ready(self):
-        """`pmean` of the policy gradients (gradients.gradient_update_fn, ppo_imitation/train.py:251) starts on a side stream as soon
-        as the policy backward has been enqueued; the value backward runs beside it."""
-        self._pending = None
-        dist = self._dist()
-        if dist is None:
-            return
-        t = self.torch
-        self.side.wait_stream(t.cuda.current_stream(self.device))
-        with t.cuda.stream(self.side):
-            self._pending = start_bucket(dist, self.grads, 0, self.n_policy)
-
-    def apply_gradients(self, exchange: bool = True, scale: float = 1.0):
-        """value bucket all-reduce + join the policy bucket, then optax.adam on the flat buffers (mean over ranks folded into Adam).
-        `exchange=False`: the caller has already all-reduced self.grads (trainer.Trainer: eager NCCL call between two CUDA graphs)
-        and passes `scale` = 1 / world."""
-        t, L_ = self.torch, tk.lib()
-        dist = self._dist() if exchange else None
-        if dist is not None:
-            scale = finish_buckets(dist, self.grads, self.n_policy, self._pending)
-            t.cuda.current_stream(self.device).wait_stream(self.side)
-            self._pending = None
+    # ---- optimiser -------------------------------------------------------------------------------------------------------------
+    def apply_gradients(self, scale: float = 1.0):
+        """optax.adam on the flat buffers, the gradients multiplied by `scale` (1 / world after all_reduce_gradients: the mean over
+        ranks folded into Adam)."""
+        L_ = tk.lib()
         st = tk.stream(self.params)
         hp = self.hp
         tk.check(L_.vnl_adam_tick(self.step_dev.data_ptr(), float(hp["b1"]), float(hp["b2"]), self.bc_dev.data_ptr(), st), "adam_tick")
@@ -490,7 +465,7 @@ class PPOLearner:
 
     def update(self, batch):
         m = self.loss_and_grads(batch)
-        self.apply_gradients()
+        self.apply_gradients(all_reduce_gradients(self.grads))
         return m
 
     def metrics_dict(self, m=None) -> Dict[str, float]:
@@ -501,19 +476,16 @@ class PPOLearner:
 
 
 # -------------------------------------------------------------------------------------------------------------------------------
-# gradient exchange (device-agnostic: the 2-rank gloo test on CPU drives the same two functions)
+# gradient exchange (device-agnostic: the 2-rank gloo test on CPU drives it on a CPU tensor)
 # -------------------------------------------------------------------------------------------------------------------------------
-def start_bucket(dist, grads, lo: int, hi: int):
-    """Asynchronous SUM all-reduce of grads[lo:hi] in place (the policy bucket, started while the value backward still runs)."""
-    return dist.all_reduce(grads[lo:hi], op=dist.ReduceOp.SUM, async_op=True)
-
-
-def finish_buckets(dist, grads, n_first: int, pending) -> float:
-    """All-reduces the remaining bucket grads[n_first:], joins the pending one and returns the factor that turns the SUMs into
-    `lax.pmean` (gradients.gradient_update_fn with pmap_axis_name): Adam applies it (vnl_adam grad_scale)."""
-    dist.all_reduce(grads[n_first:], op=dist.ReduceOp.SUM)
-    if pending is not None:
-        pending.wait()
+def all_reduce_gradients(grads) -> float:
+    """`lax.pmean` of the gradients (gradients.gradient_update_fn with pmap_axis_name, ppo_imitation/train.py:251): one in-place
+    SUM all-reduce of the whole flat buffer over the process group.  Returns the factor that turns the SUMs into the mean, which
+    Adam applies (vnl_adam grad_scale): 1 / world, or 1.0 without a group (nothing is exchanged)."""
+    dist = sharding.group()
+    if dist is None:
+        return 1.0
+    dist.all_reduce(grads, op=dist.ReduceOp.SUM)
     return 1.0 / dist.get_world_size()
 
 

@@ -14,7 +14,7 @@ from __future__ import annotations
 
 import ctypes
 
-from . import _lib
+from . import _lib, sharding
 
 NORMALIZER_EXPORTS = ("vnl_obs_stats_workspace_bytes", "vnl_obs_stats_partial", "vnl_obs_stats_finish",
                       "vnl_xla_obs_stats_partial", "vnl_xla_obs_stats_finish")
@@ -34,9 +34,8 @@ def _bind(lib):
 
 def all_reduce_sums(sums):
     """The one exchange of the update: sum the [S1 | S2 | rows] vector over the process group (identity without one)."""
-    import torch.distributed as dist
-
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+    dist = sharding.group()
+    if dist is not None:
         dist.all_reduce(sums, op=dist.ReduceOp.SUM)
     return sums
 

@@ -17,6 +17,8 @@ from __future__ import annotations
 
 from typing import Dict, Optional
 
+from . import train_kernels as tk
+
 
 class Rollout:
     def __init__(self, env, policy, first_state, unroll_length: int, episode_length: float, use_graph: bool = True):
@@ -82,7 +84,6 @@ class Rollout:
     def generate_unroll(self, eps_z=None, eps_a=None) -> Dict[str, "torch.Tensor"]:
         """One unroll; returns views of the transition buffers, named as brax's Transition (acting.py:50-57):
         observation / next_observation [T,B,obs], action [T,B,nu], reward, discount [T,B], policy extras, state extras."""
-        t = self.torch
         if eps_z is not None:
             self.eps_z.copy_(eps_z)
         if eps_a is not None:
@@ -94,20 +95,9 @@ class Rollout:
             self._enqueue()
         else:
             if self.graph is None:
-                # warm-up outside capture (function attributes, lazy module load), on a snapshot that is restored after
+                # the warm-up unroll runs on a snapshot of the carry that is restored after it (the capture executes nothing)
                 snap = self._snapshot()
-                side = t.cuda.Stream(device=self.eng.device)
-                side.wait_stream(t.cuda.current_stream(self.eng.device))
-                with t.cuda.stream(side):
-                    self._enqueue()
-                t.cuda.current_stream(self.eng.device).wait_stream(side)
-                self._restore(snap)
-                t.cuda.synchronize(self.eng.device)
-                self.graph = t.cuda.CUDAGraph()
-                # thread_local: event queries of other threads (NCCL's watchdog when a process group exists) do not invalidate the capture
-                with t.cuda.graph(self.graph, capture_error_mode="thread_local"):
-                    self._enqueue()
-                self._restore(snap)
+                self.graph, = tk.capture(self.eng.device, lambda: (self._enqueue(), self._restore(snap)), self._enqueue)
                 # the graph holds the policy's operand addresses: `load_params` / `set_normalizer` copy into them from now on
                 self._captured = (self.policy.blob_dev.data_ptr(), None if self.policy.obs_mean is None else self.policy.obs_mean.data_ptr(),
                                   None if self.policy.obs_std is None else self.policy.obs_std.data_ptr())

@@ -43,19 +43,26 @@ def init_process_group(backend: str = "nccl"):
     return rank, local_rank, world
 
 
-def barrier():
+def group():
+    """`torch.distributed` when a process group with more than one rank is initialised, else None: the one test of whether
+    there is anybody to exchange with."""
     import torch.distributed as dist
 
-    if dist.is_available() and dist.is_initialized():
+    return dist if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1 else None
+
+
+def barrier():
+    dist = group()
+    if dist is not None:
         dist.barrier()
 
 
 def reduce_scalars(values: Dict[str, float], op: str = "sum", device=None) -> Dict[str, float]:
     """All-reduce a small dict of python floats (metric / timing reduction); identity at world size 1."""
     import torch
-    import torch.distributed as dist
 
-    if not (dist.is_available() and dist.is_initialized()):
+    dist = group()
+    if dist is None:
         return dict(values)
     keys = sorted(values)
     t = torch.tensor([float(values[k]) for k in keys], dtype=torch.float64, device=device)

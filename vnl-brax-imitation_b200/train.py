@@ -274,7 +274,5 @@ def train(environment, num_timesteps: int, episode_length: int = 150, num_envs: 
 
 
 def _rank_world() -> Tuple[int, int]:
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized():
-        return dist.get_rank(), dist.get_world_size()
-    return 0, 1
+    dist = sharding.group()
+    return (dist.get_rank(), dist.get_world_size()) if dist is not None else (0, 1)

@@ -56,6 +56,28 @@ def check(rc: int, what: str):
         raise RuntimeError(f"{what} failed with code {rc}")
 
 
+def capture(device, warmup, *fns):
+    """One CUDA graph per function in `fns`, for the rollout's unroll and the trainer's minibatch update.  `warmup()` runs first,
+    eagerly on a side stream (lazy module loads, ctypes bindings and allocations happen outside the capture); then the device is
+    synchronised and each fn is captured with capture_error_mode="thread_local", so calls from other threads -- NCCL's watchdog
+    querying its events -- do not invalidate the capture.  No fn may issue a collective: an 8-GPU run hung when the gradient
+    all-reduce was captured with the update (DESIGN §3d)."""
+    import torch
+    main = torch.cuda.current_stream(device)
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(main)
+    with torch.cuda.stream(side):
+        warmup()
+    main.wait_stream(side)
+    torch.cuda.synchronize(device)
+    graphs = []
+    for fn in fns:
+        graphs.append(torch.cuda.CUDAGraph())
+        with torch.cuda.graph(graphs[-1], capture_error_mode="thread_local"):
+            fn()
+    return graphs
+
+
 def _ptrs(ts):
     return (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
 

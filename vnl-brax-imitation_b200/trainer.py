@@ -8,8 +8,8 @@
     policy <- new parameters                                            policy.load_params (same device blob: captured graphs keep working)
 
 The transition buffers stay on the device from the env kernel to the loss: a minibatch is an index list over the env axis
-(`vnl_gather_rows`, which also pads traj rows 795 -> 796 floats for TMA).  One minibatch update (gathers + ~80 launches + the two
-gradient exchange + Adam) is captured once into CUDA graphs (collective-free: with a process group the NCCL all-reduce runs eagerly
+(`vnl_gather_rows`, which also pads traj rows 795 -> 796 floats for TMA).  One minibatch update (gathers + ~80 launches, the
+gradient exchange, Adam) is captured once into CUDA graphs (collective-free: with a process group the NCCL all-reduce runs eagerly
 between the gradient graph and the Adam graph) and replayed with fresh indices / noise.  torch = memory, streams,
 RNG for the noise operands and `torch.distributed`; no torch math on the data path, no CPU fallback.
 """
@@ -18,6 +18,7 @@ from __future__ import annotations
 from typing import Dict
 
 from . import learner as lrn
+from . import sharding
 from . import train_kernels as tk
 
 
@@ -84,33 +85,32 @@ class Trainer:
         tk.check(tk.lib().vnl_metrics_accumulate(m.data_ptr(), m.numel(), self.metric_sum.data_ptr(), tk.stream(m)), "vnl_metrics_accumulate")
         self.sgd_launches += 1
 
-    def _minibatch(self, tr):
+    def _grads(self, tr):
+        """The update up to the gradient exchange: gather, loss + gradients, and the metric accumulation when enabled."""
         n0 = self.learner.launches
         self._gather(tr)
-        if self.accumulate_metrics:  # update() = loss_and_grads + apply_gradients, with the accumulation between them
-            self.learner.loss_and_grads(self.mb)
+        self.learner.loss_and_grads(self.mb)
+        if self.accumulate_metrics:
             self._accumulate()
-            self.learner.apply_gradients()
-        else:
-            self.learner.update(self.mb)
         self.sgd_launches += self.learner.launches - n0
 
-    def _capture(self, fn):
-        """Capture `fn` into a CUDA graph.  The graphs of the SGD phase never contain a collective: with a process group the gradient
-        all-reduce runs eagerly BETWEEN two graphs (loss + gradients | Adam), so NCCL's watchdog thread and the capture never meet
-        (`capture_error_mode="thread_local"`: calls from other threads -- the watchdog's event queries -- do not invalidate it)."""
-        t = self.torch
-        t.cuda.synchronize(self.idx.device)
-        g = t.cuda.CUDAGraph()
-        with t.cuda.graph(g, capture_error_mode="thread_local"):
-            fn()
-        return g
+    def _adam(self, scale: float):
+        n0 = self.learner.launches
+        self.learner.apply_gradients(scale)
+        self.sgd_launches += self.learner.launches - n0
+
+    def _minibatch(self, tr):
+        """One eager update: gradients, their exchange over the process group (if any), Adam."""
+        self._grads(tr)
+        self._adam(lrn.all_reduce_gradients(self.learner.grads))
 
     def sgd_phase(self, tr) -> None:
-        """num_updates_per_batch x num_minibatches gradient updates on the unroll `tr` (train.py:336-341)."""
+        """num_updates_per_batch x num_minibatches gradient updates on the unroll `tr` (train.py:336-341).  Graph mode captures the
+        update once: one graph of gradients + Adam on one rank; with a process group a graph of the gradients, the all-reduce eagerly
+        (the graphs never contain a collective, see tk.capture), then a graph of Adam."""
         t = self.torch
         lr = self.learner
-        dist = lr._dist()
+        dist = sharding.group()
         self.discount_buf.copy_(tr["discount"])  # `1 - done` view materialised once per unroll
         # the policy's INPUT trajectory of step t is traj[t] (acting.py:47: state.info["traj"]), i.e. rollout.traj[:T]
         tr = dict(tr, state_extras_traj_in=self.rollout.traj[:self.T])
@@ -123,28 +123,22 @@ class Trainer:
                     self._minibatch(tr)
                     continue
                 if self.graph is None:
-                    side = t.cuda.Stream(device=self.idx.device)  # warm-up outside capture (lazy module loads, attribute sets)
-                    side.wait_stream(t.cuda.current_stream(self.idx.device))
-                    l0 = self.sgd_launches
-                    with t.cuda.stream(side):
+                    n0, l0 = lr.updates, self.sgd_launches
+
+                    def warmup():  # a real update of this minibatch
                         self._minibatch(tr)
-                    t.cuda.current_stream(self.idx.device).wait_stream(side)
-                    self._launches_per_update = self.sgd_launches - l0  # kernels one replay of the captured update launches
-                    n0, l1 = lr.updates, self.sgd_launches
+                        self._launches_per_update = self.sgd_launches - l0  # kernels one replay of the captured update launches
                     if dist is None:
-                        self.graph = (self._capture(lambda: self._minibatch(tr)),)
+                        fns = (lambda: (self._grads(tr), self._adam(1.0)),)
                     else:
-                        def grads_only():
-                            self._gather(tr)
-                            lr.loss_and_grads(self.mb, exchange=False)
-                            if self.accumulate_metrics:
-                                self._accumulate()
-                        self.graph = (self._capture(grads_only), self._capture(lambda: lr.apply_gradients(exchange=False, scale=1.0 / dist.get_world_size())))
-                    lr.updates, self.sgd_launches = n0, l1  # the capture passes went through the host-side counters without executing
+                        fns = (lambda: self._grads(tr), lambda: self._adam(1.0 / dist.get_world_size()))
+                    self.graph = tk.capture(self.idx.device, warmup, *fns)
+                    # the warm-up was one update; the capture passes went through the host-side counters without executing
+                    lr.updates, self.sgd_launches = n0 + 1, l0 + self._launches_per_update
                     continue  # this minibatch was the warm-up run
                 self.graph[0].replay()
                 if dist is not None:
-                    dist.all_reduce(lr.grads, op=dist.ReduceOp.SUM)  # lax.pmean of the gradients: one NCCL call, 6.5 MB; 1 / world in Adam
+                    lrn.all_reduce_gradients(lr.grads)  # lax.pmean: one 6.5 MB SUM all-reduce; its 1 / world is in the Adam graph
                     self.graph[1].replay()
                 lr.updates += 1  # host-side counter (the device-side step counter advanced inside the graph)
                 self.sgd_launches += self._launches_per_update
