@@ -47,11 +47,12 @@ int vnl_obs_normalize(const float* obs, int ld_obs, int rows, int width, const f
                       void* stream);
 
 /* h = LayerNorm(relu(pre)) (intention_policy_network.py:36-40, 64-68; flax LayerNorm: eps 1e-6, fast variance).
- * stats [rows, 2] = (mean, rstd) of relu(pre), kept for the backward pass. */
+ * stats [rows, 2] = (mean, rstd) of relu(pre), kept for the backward pass.  n <= 1024 (one warp per row, 32 values per lane). */
 int vnl_relu_ln_fwd(const float* pre, int ld_pre, int rows, int n, const float* scale, const float* bias, float* out, int ld_out,
                     float* stats, void* stream);
 /* dpre from dy; dscale / dbias [n] are ACCUMULATED (caller zeroes).  dbias_pre (may be NULL) [n] += column sums of dpre = the bias
- * gradient of the dense layer in front of the relu, so that it needs no pass of its own. */
+ * gradient of the dense layer in front of the relu, so that it needs no pass of its own.  n <= 256 (the per-column partials of a
+ * warp live in registers: 8 per lane); ld_dy, ld_pre, ld_dpre >= n. */
 int vnl_relu_ln_bwd(const float* dy, int ld_dy, const float* pre, int ld_pre, const float* stats, const float* scale, int rows, int n,
                     float* dpre, int ld_dpre, float* dscale, float* dbias, float* dbias_pre, void* stream);
 

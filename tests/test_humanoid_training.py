@@ -146,18 +146,21 @@ def test_gemm_with_padded_row_strides(case):
 T, BM = 5, 96  # 480 rows: ragged last tile
 
 
-def _params(seed, enc=(256, 128), dec=(128, 256)):
+def _params(seed, enc=(256, 128), dec=(128, 256), last_scale=1.0):
     pol, lrn = pkg("policy"), pkg("learner")
     rng = np.random.default_rng(seed)
     P = pol.init_params(rng, pol.param_shapes(630, 55, 21, encoder_layer_sizes=enc, decoder_layer_sizes=dec), perturb=0.05)
+    P["decoder/hidden_2/kernel"] = P["decoder/hidden_2/kernel"] * np.float32(last_scale)
     V = lrn.init_value_params(rng, lrn.value_param_shapes(55), perturb=0.05)
     return P, V
 
 
-def _batch(seed, P, V):
+def _batch(seed, P, V, T=T, BM=BM, clip=0.3):
     """A humanoid minibatch as tests/test_learner.py builds the rodent's: actions sampled from the policy's own distribution,
-    behaviour log-probs = the target's plus noise (rho on both sides of the clip range), some truncations / terminations."""
+    behaviour log-probs = the target's plus noise (rho on both sides of the clip range, no row within 2e-3 of a clip boundary in
+    log rho), some truncations / terminations."""
     import torch
+    from test_learner import keep_off_clip_edges
     lrn = pkg("learner")
     g = torch.Generator(device="cuda").manual_seed(seed)
     R, nu = T * BM, 21
@@ -173,7 +176,8 @@ def _batch(seed, P, V):
     loc, scale = aux["logits"][:, :nu], torch.nn.functional.softplus(aux["logits"][:, nu:]) + 0.001
     batch["raw_action"] = (loc + scale * rn(R, nu).double()).float().contiguous()
     _, _, _, _, aux = lrn.reference_loss(P, V, batch, T, BM, mean, std)
-    batch["log_prob"] = (aux["target_lp"].reshape(-1) + 0.25 * rn(R).double()).float().contiguous()
+    log_rho = keep_off_clip_edges(-0.25 * rn(R).double(), clip)
+    batch["log_prob"] = (aux["target_lp"].reshape(-1) - log_rho).float().contiguous()
     return batch, mean, std
 
 
@@ -193,39 +197,43 @@ def _padding(L, flat):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("T_,BM_", [(T, BM), (20, 256)], ids=["480rows", "5120rows"])
+@pytest.mark.parametrize("x3", [True, False], ids=["3xtf32", "tf32"])
 @pytest.mark.parametrize("sizes", [((256, 128), (128, 256)), ((250, 126), (126, 250))], ids=["humanoid", "odd-hidden-widths"])
-def test_humanoid_loss_and_gradients_match_autograd(sizes):
-    """3xTF32 against learner.reference_loss in float64: loss terms 1e-5, every gradient tensor 5e-4 of its largest entry, on a
-    batch without relu sign flips (the first such seed, as test_loss_and_gradients_match_autograd chooses it).  The second case
-    also pads the hidden activations and kernels (widths 250 / 126)."""
+def test_humanoid_loss_and_gradients_match_autograd(sizes, x3, T_, BM_):
+    """Against learner.reference_loss in float64 on the kernel's relu branches (test_learner.reference_on_kernel_branches), with
+    test_learner's tolerances: 3xTF32 loss terms 1e-5, every gradient tensor 5e-4 of its largest entry; TF32 (what train() runs) loss
+    2e-3, gradients 1e-1 in Frobenius norm, logits of std 0.2 and the clip range opened wide (the reasons are given there).  The second
+    case also pads the hidden activations and kernels (widths 250 / 126); 5120 rows is the minibatch training runs."""
     import torch
+    from test_learner import reference_on_kernel_branches
     lrn = pkg("learner")
-    P, V = _params(1, *sizes)
-    for seed in range(2, 10):
-        batch, mean, std = _batch(seed, P, V)
-        L = lrn.PPOLearner(P, V, T, BM, x3=True, clipping_epsilon=0.3)
-        L.set_normalizer(mean, std)
-        m = L.metrics_dict(L.loss_and_grads(batch))
-        torch.cuda.synchronize()
-        _, want, gP, gV, aux = lrn.reference_loss(P, V, batch, T, BM, mean, std, clipping_epsilon=0.3)
-        flips = sum(int(((L.ws[n].double() > 0) != (ref > 0)).sum()) for n, ref in zip(("h0pre", "h1pre", "d0pre", "d1pre"), aux["pre"]))
-        if flips == 0:
-            break
-    assert flips == 0, "no seed without a relu sign flip"
+    P, V = _params(1, *sizes, last_scale=1.0 if x3 else 0.2)
+    clip = 0.3 if x3 else 1e3
+    tol_loss, tol_grad, tol_fwd = (1e-5, 5e-4, 2e-5) if x3 else (2e-3, 1e-1, 5e-3)
+    batch, mean, std = _batch(2, P, V, T=T_, BM=BM_, clip=clip)
+    L = lrn.PPOLearner(P, V, T_, BM_, x3=x3, clipping_epsilon=clip)
+    L.set_normalizer(mean, std)
+    m = L.metrics_dict(L.loss_and_grads(batch))
+    torch.cuda.synchronize()
+    want, gP, gV, aux, flips = reference_on_kernel_branches(L, P, V, batch, T_, BM_, mean, std, x3, clip)
     assert L.ws["logits"].stride(0) == 44 and L.ws["dec_in"].stride(0) == 120 and L.ws["vin"].stride(0) == 56
     for k in ("total_loss", "policy_loss", "v_loss", "entropy_loss", "kl_loss_intention", "mean_rho"):
-        assert abs(m[k] - want[k]) < 1e-5 * max(1.0, abs(want[k])), (k, m[k], want[k])
-    assert 0.05 < m["clip_fraction"] < 0.95
-    assert _rel(L.ws["logits"].cpu().numpy(), aux["logits"].cpu().numpy()) < 2e-5
-    assert _rel(L.ws["val"][:T * BM].cpu().numpy(), aux["baseline"].reshape(-1).cpu().numpy()) < 2e-5
-    assert _rel(L.ws["dlogits"].cpu().numpy(), aux["dlogits"].cpu().numpy()) < 5e-4
+        assert abs(m[k] - want[k]) < tol_loss * max(1.0, abs(want[k])), (k, m[k], want[k])
+    assert (0.05 < m["clip_fraction"] < 0.95) if x3 else m["clip_fraction"] == 0
+    assert _rel(L.ws["logits"].cpu().numpy(), aux["logits"].cpu().numpy()) < tol_fwd
+    assert _rel(L.ws["val"][:T_ * BM_].cpu().numpy(), aux["baseline"].reshape(-1).cpu().numpy()) < tol_fwd
+    assert _rel(L.ws["dlogits"].cpu().numpy(), aux["dlogits"].cpu().numpy()) < tol_grad
     got_p, got_v = L.policy_grads(), L.value_grads()
-    worst = {"policy/" + k: _rel(got_p[k], g.cpu().numpy()) for k, g in gP.items()}
-    worst.update({"value/" + k: _rel(got_v[k], g.cpu().numpy()) for k, g in gV.items()})
-    bad = {k: v for k, v in worst.items() if v > 5e-4}
+    fro = lambda a, b: float(np.linalg.norm(np.asarray(a, np.float64) - np.asarray(b, np.float64)) / (np.linalg.norm(np.asarray(b, np.float64)) + 1e-30))
+    err = _rel if x3 else fro
+    worst = {"policy/" + k: err(got_p[k], g.cpu().numpy()) for k, g in gP.items()}
+    worst.update({"value/" + k: err(got_v[k], g.cpu().numpy()) for k, g in gV.items()})
+    bad = {k: v for k, v in worst.items() if v > tol_grad}
     assert not bad, bad
     assert len(worst) == 28
-    print("sizes %s seed %d: worst gradient error %.2e" % (sizes, seed, max(worst.values())))
+    print("sizes %s x3=%s rows %d: %d relu flips, worst gradient error %.2e (%s)" % (sizes, x3, T_ * BM_, flips, max(worst.values()),
+                                                                                     max(worst, key=worst.get)))
 
 
 @pytest.mark.gpu

@@ -435,6 +435,7 @@ int vnl_relu_ln_fwd(const float* pre, int ld_pre, int rows, int n, const float* 
 int vnl_relu_ln_bwd(const float* dy, int ld_dy, const float* pre, int ld_pre, const float* stats, const float* scale, int rows, int n,
                     float* dpre, int ld_dpre, float* dscale, float* dbias, float* dbias_pre, void* stream) {
   if (!dy || !pre || !stats || !scale || !dpre || !dscale || !dbias || rows <= 0 || n <= 0 || n > 256) return -1;
+  if (ld_dy < n || ld_pre < n || ld_dpre < n) return -1;
   const int threads = 256, grid = grid_for((size_t)rows * 32, threads) < 148 ? grid_for((size_t)rows * 32, threads) : 148;
   const size_t smem = (size_t)(threads / 32) * 3 * n * sizeof(float);
   relu_ln_bwd_kernel<8><<<grid, threads, smem, (cudaStream_t)stream>>>(dy, ld_dy, pre, ld_pre, stats, scale, rows, n, dpre, ld_dpre, dscale, dbias, dbias_pre);
@@ -443,12 +444,14 @@ int vnl_relu_ln_bwd(const float* dy, int ld_dy, const float* pre, int ld_pre, co
 
 int vnl_swish_fwd(const float* pre, size_t n, float* out, void* stream) {
   if (!pre || !out) return -1;
-  if (n) swish_fwd_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(pre, n, out);
+  if (n == 0) return 0;  // as split and Adam: nothing to enqueue, and an earlier launch's error is not this call's to report
+  swish_fwd_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(pre, n, out);
   return rc();
 }
 int vnl_swish_bwd(const float* dy, const float* pre, size_t n, float* dpre, void* stream) {
   if (!dy || !pre || !dpre) return -1;
-  if (n) swish_bwd_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(dy, pre, n, dpre);
+  if (n == 0) return 0;
+  swish_bwd_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(dy, pre, n, dpre);
   return rc();
 }
 

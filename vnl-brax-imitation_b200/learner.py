@@ -493,11 +493,14 @@ def all_reduce_gradients(grads) -> float:
 # checker: torch-autograd restatement of the reference loss (tests / tools only)
 # -------------------------------------------------------------------------------------------------------------------------------
 def reference_loss(policy_params, value_params, batch, T: int, Bm: int, obs_mean, obs_std, *, entropy_cost=1e-4, discounting=0.9,
-                   reward_scaling=1.0, gae_lambda=0.95, clipping_epsilon=0.3, normalize_advantage=True, kl_weight=1e-4, dtype=None):
+                   reward_scaling=1.0, gae_lambda=0.95, clipping_epsilon=0.3, normalize_advantage=True, kl_weight=1e-4, dtype=None,
+                   relu_masks=None):
     """`compute_ppo_intention_loss` (ppo_imitation/intention_losses.py:91-202) restated in torch with autograd, line by line:
     policy_apply (intention_policy_network.py:82-105 with the reparameterisation noise `eps_z`), value_apply (brax MLP, swish),
     NormalTanhDistribution.log_prob / entropy (sample from `eps_ent`), compute_gae (:26-89, stop-gradient), advantage
     normalisation, clipped surrogate, v_loss * 0.5 * 0.5, entropy_cost, kl_weight * kl_divergence.
+    relu_masks: optional [h0pre, h1pre, d0pre, d1pre] sign masks (pre-activation > 0) of another evaluation, the kernels' own: relu(x)
+    becomes x * mask, so that an element whose pre-activation lies within rounding of zero takes the same branch in both.
     Returns (total, metrics dict, policy grads dict, value grads dict) with parameters as leaf tensors."""
     import torch
 
@@ -517,17 +520,18 @@ def reference_loss(policy_params, value_params, batch, T: int, Bm: int, obs_mean
         var = torch.clamp((x * x).mean(-1, keepdim=True) - m * m, min=0.0)
         return (x - m) * torch.rsqrt(var + 1e-6) * Pp[name + "/scale"] + Pp[name + "/bias"]
     dense = lambda x, name: x @ Pp[name + "/kernel"] + Pp[name + "/bias"]
+    relu = lambda x: torch.relu(x) if relu_masks is None else x * c(relu_masks[len(pres) - 1])
     h = traj
     pres = []
     for i in range(2):
         pres.append(dense(h, f"encoder/hidden_{i}"))
-        h = ln(torch.relu(pres[-1]), f"encoder/LayerNorm_{i}")
+        h = ln(relu(pres[-1]), f"encoder/LayerNorm_{i}")
     zm, zlv = dense(h, "encoder/fc2_mean"), dense(h, "encoder/fc2_logvar")
     z = zm + c(batch["eps_z"]) * torch.exp(0.5 * zlv)
     h = torch.cat([z, obs_n], -1)
     for i in range(2):
         pres.append(dense(h, f"decoder/hidden_{i}"))
-        h = ln(torch.relu(pres[-1]), f"decoder/LayerNorm_{i}")
+        h = ln(relu(pres[-1]), f"decoder/LayerNorm_{i}")
     logits = dense(h, "decoder/hidden_2")
     logits.retain_grad()
 
