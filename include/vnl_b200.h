@@ -344,6 +344,31 @@ int vnl_step_training(const VnlContext* ctx, const void* model, const void* task
                       const VnlState* out, const VnlOutputs* outputs, const VnlState* first, const float* first_obs,
                       const VnlEpisode* episode, void* stream);
 
+/* Resampling AutoReset (DESIGN §3h): where an episode ends, the env starts a new one from a fresh draw instead of the cached
+ * first state.  The draw: Philox4x32-10 with key (seed low 32 bits, seed high 32 bits) and counter (g, n, j, 0), g =
+ * env_offset + e the global env index, n = reset_count[e], j the block.  Block 0: clip = (x0 * nclips) >> 32, start =
+ * (x1 * start_frame_hi) >> 32 (64-bit products).  Blocks j >= 1, only when noise_scale != 0: u = ((x >> 8) + 1) 2^-24,
+ * Box-Muller on (u0, u1) and (u2, u3) -> (r cos t, r sin t), r = sqrt(-2 ln u_a), t = 2 pi u_b: the normals of qpos
+ * coordinates 4 (j - 1) .. 4 (j - 1) + 3. */
+typedef struct VnlResample {
+  uint64_t seed;          /* Philox key */
+  int32_t env_offset;     /* global index of env 0 of this call (a shard's first env): a sharded run draws what one process would */
+  int32_t start_frame_hi; /* start frame uniform in [0, start_frame_hi); 0 < start_frame_hi <= clip length - ref_traj_length, so
+                             that the reset's reference window lies inside the clip */
+  float noise_scale;      /* qpos += noise_scale * N(0, 1) on every coordinate (finite, >= 0; 0 = no noise) */
+  int32_t* reset_count;   /* [B] resets of each env so far (the draw's counter n); incremented on every env reset */
+  int32_t* scratch;       /* [B + 1] caller-owned device scratch: the count of done envs, then their indices */
+} VnlResample;
+
+/* vnl_step_training without the first-state restore, then, where the final done flag is set, the env reset in place to a fresh
+ * draw (clip, start frame, qpos noise): what vnl_reset of the drawn qpos / qvel / start frame / clip would write goes to the
+ * state leaves of `out`, cur_frame = start, sub_clip_frame = 0, clip_id = clip (where `out` has one), and to the obs / traj rows
+ * of `outputs`.  The step's reward, done, metrics, stats, steps and truncation are kept.  Three launches (step, compaction of
+ * the done envs into rs->scratch, reset of the listed envs): enqueue-only, no allocation, capturable. */
+int vnl_step_training_resample(const VnlContext* ctx, const void* model, const void* task, int B, const VnlState* in,
+                               const float* action, const VnlState* out, const VnlOutputs* outputs, const VnlEpisode* episode,
+                               const VnlResample* rs, void* stream);
+
 /* Reset tail for B envs: qpos/qvel/cur_frame(start_frame) are read from `in` (act, ctrl and
  * qacc_warmstart are zero as in mjx.make_data), `out` receives the mjx.forward state, obs,
  * traj and info["termination_error"] (metrics[6]).  Replaces envs/rodent.py:148-176. */

@@ -8,6 +8,8 @@
   POLICY=kernel (default): the repo's tcgen05 policy kernel (vnl_policy_forward, one launch, row f1), normal draws
   pre-generated for the whole unroll (the caller owns the RNG stream, like the reference's key argument);
   POLICY=torch: the same network through torch / cuBLAS (library kernels, ~25 launches) -- the comparison line.
+  GRAPH=1: the packaged loop (rollout.Rollout); there AUTORESET=first|resample (first) selects how finished episodes restart
+  (brax's first-state restore, or a fresh draw of clip, start frame and noise on the device: DESIGN §3h).
 
 Also times the PPO gradient all-reduce message (policy 341 k + value 1.289 M fp32 parameters = 6.5 MB,
 ppo_imitation/train.py:251-253) over NCCL when launched under torchrun.
@@ -77,6 +79,7 @@ def main():
     first, first_obs = dict(s0.pipeline_state), s0.obs
     torch.manual_seed(rank)
     which = os.environ.get("POLICY", "kernel")
+    autoreset = os.environ.get("AUTORESET", "first")  # GRAPH=1 only: "resample" restarts finished episodes from fresh draws
     if which == "torch":
         policy = IntentionPolicy(eng.traj_size, eng.obs_size, env.action_size).to(dev).eval()
     else:
@@ -90,7 +93,8 @@ def main():
     if os.environ.get("GRAPH") == "1" and which != "torch":
         # the packaged loop: rollout.Rollout = generate_unroll over vnl_policy_forward + vnl_step_training (Episode + AutoReset
         # wrappers fused, episode_length 150), 2 x 20 launches replayed as one CUDA graph, draws refilled per unroll
-        ro = importlib.import_module("vnl-brax-imitation_b200.rollout").Rollout(env, kpol, s0, unroll, 150.0, use_graph=True)
+        ro = importlib.import_module("vnl-brax-imitation_b200.rollout").Rollout(env, kpol, s0, unroll, 150.0, use_graph=True,
+                                                                                  autoreset=autoreset, env_offset=B * rank)
         stats = importlib.import_module("vnl-brax-imitation_b200.normalizer").RunningStatistics(eng.obs_size, str(dev))
         kpol.set_normalizer(stats.mean, stats.std)  # shared tensors: every update is seen by the next policy launch
         stats.update(ro.generate_unroll(eps_z, eps_a)["observation"])
@@ -111,7 +115,7 @@ def main():
             dist.destroy_process_group()
         if rank == 0:
             print(json.dumps({"config": "rodent PPO rollout (rollout.Rollout, CUDA graph of 2 x %d launches; draws generated and the obs normaliser updated + all-reduced inside the timed region): %d envs/GPU" % (unroll, B),
-                              "n_gpus": world, "rollout_env_steps_per_s": world * B * unroll * reps / (ms * 1e-3), "ms_per_unroll": ms / reps}), flush=True)
+                              "autoreset": autoreset, "n_gpus": world, "rollout_env_steps_per_s": world * B * unroll * reps / (ms * 1e-3), "ms_per_unroll": ms / reps}), flush=True)
         return
     a_st = {k: v.clone() for k, v in first.items()}
     a_st["cur_frame"], a_st["sub_clip_frame"] = s0.info["cur_frame"].clone(), s0.info["sub_clip_frame"].clone()

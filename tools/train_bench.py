@@ -7,6 +7,7 @@ GEMMs, Adam) with the gradient all-reduce over NCCL at N > 1 -- timed phase by p
   env: ENVS (8192) MINIBATCHES (32) UPDATES (16) STEPS (2) GRAPH (1) X3 (0)
        ENV=rodent|humanoid (rodent) -- the tracking env; CLIP=standing|moving (standing) -- the humanoid's packaged stand-in clip
        (`envs.humanoid.packaged_humanoid(moving=...)`; the rodent always tracks its packaged clip)
+  AUTORESET=first|resample (first) -- how finished training episodes restart: brax's first-state restore, or a fresh draw (DESIGN §3h)
   PROFILE=1 (with GRAPH=0): after the warm-up step, ONE eager minibatch update between cudaProfilerStart / Stop and exit -- the region
   `ncu --profile-from-start off --metrics gpu__time_duration.sum` lists (tools/make_profiles.py summarises the csv)."""
 import importlib
@@ -36,7 +37,7 @@ def build(dev, rank, world, B, unroll, nmb, nup, graph=True, x3=False, env_name=
     s0 = env.reset_from(qpos, qvel, start)
     # train()'s assembly (the same seeds: identical initial networks on every rank, the trainer's noise seeded by its rank)
     cfg = dict(trn.DEFAULTS, num_envs=B * world, batch_size=B * world // nmb, unroll_length=unroll, num_minibatches=nmb, num_updates_per_batch=nup,
-               policy="bf16" if os.environ.get("POLICY") == "bf16" else "3xtf32")
+               policy="bf16" if os.environ.get("POLICY") == "bf16" else "3xtf32", autoreset=os.environ.get("AUTORESET", "first"))
     tr = trn.Run(env, cfg, rank=rank, world_size=world, first_state=s0, use_graph=graph, learner_x3=x3, accumulate_metrics=False, evaluate=False).trainer
     return tr
 

@@ -31,6 +31,11 @@ class VnlEpisode(ctypes.Structure):
                 ("truncation_out", ctypes.c_void_p), ("episode_length", ctypes.c_float)]
 
 
+class VnlResample(ctypes.Structure):
+    _fields_ = [("seed", ctypes.c_uint64), ("env_offset", ctypes.c_int32), ("start_frame_hi", ctypes.c_int32),
+                ("noise_scale", ctypes.c_float), ("reset_count", ctypes.c_void_p), ("scratch", ctypes.c_void_p)]
+
+
 class VnlOutputs(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in OUT_F + ("stats",)]
 
@@ -51,7 +56,7 @@ EXPORTS = ("vnl_step", "vnl_reset", "vnl_pipeline_step", "vnl_forward_dump", "vn
            "vnl_check_task", "vnl_context_init", "vnl_step_smem_bytes", "vnl_xla_step", "vnl_xla_reset", "vnl_xla_step_rc",
            "vnl_xla_reset_rc", "vnl_xla_make_opaque", "vnl_version", "vnl_ffma_probe", "vnl_step_profiled",
            "vnl_step_autoreset", "vnl_envs_per_cta", "vnl_resident_envs", "vnl_workspace_bytes", "vnl_step_training",
-           "vnl_debug_layout", "vnl_process_clip")
+           "vnl_debug_layout", "vnl_process_clip", "vnl_step_training_resample")
 
 
 IEEE_LIB_PATH = os.path.join(_HERE, "libvnl_b200_ieee.so")  # A/B twin: IEEE div / sqrt in the physics kernels (tests only)
@@ -79,6 +84,7 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.vnl_step.argtypes = [CTX, v, v, i, ST, v, ST, OUT, v]
     lib.vnl_step_autoreset.argtypes = [CTX, v, v, i, ST, v, ST, OUT, ST, v, v]
     lib.vnl_step_training.argtypes = [CTX, v, v, i, ST, v, ST, OUT, ST, v, ctypes.POINTER(VnlEpisode), v]
+    lib.vnl_step_training_resample.argtypes = [CTX, v, v, i, ST, v, ST, OUT, ctypes.POINTER(VnlEpisode), ctypes.POINTER(VnlResample), v]
     lib.vnl_reset.argtypes = [CTX, v, v, i, ST, ST, OUT, v]
     lib.vnl_pipeline_step.argtypes = [CTX, v, i, i, ST, v, ST, v, v]
     lib.vnl_forward_dump.argtypes = [CTX, v, i, ST, v, v, v]
@@ -246,6 +252,27 @@ class Engine:
         self._check(self.lib.vnl_step_training(self._cref, self.model_dev.data_ptr(), self.task_dev.data_ptr(), B, ctypes.byref(a),
                                                action.data_ptr(), ctypes.byref(b), ctypes.byref(o), ctypes.byref(f),
                                                first_obs.data_ptr(), ctypes.byref(ep), self._stream()), "vnl_step_training")
+
+    def step_training_resample(self, state: Dict, action, out_state: Dict, outputs: Dict, steps, done_in, steps_out, truncation,
+                               episode_length: float, reset_count, scratch, seed: int, env_offset: int, start_frame_hi: int,
+                               noise_scale: float):
+        """`vnl_step_training_resample`: the training step without the first-state restore; done envs are reset in place to a
+        fresh draw (clip, start frame in [0, start_frame_hi), qpos noise), keyed by `seed`, the global env index
+        (`env_offset` + row) and `reset_count` (int32 [B], incremented per reset).  `scratch`: int32 [B + 1] for the done list."""
+        t = self.torch
+        B = state["qpos"].shape[0]
+        a, b, o = self._state(state), self._state(out_state), self._outputs(outputs)
+        assert action.is_contiguous() and action.shape == (B, self.dims["nu"])
+        for x in (steps, done_in, steps_out, truncation):
+            assert x.is_contiguous() and x.shape == (B,) and x.element_size() == 4 and x.dtype.is_floating_point
+        assert reset_count.is_contiguous() and reset_count.shape == (B,) and reset_count.dtype == t.int32
+        assert scratch.is_contiguous() and scratch.numel() >= B + 1 and scratch.dtype == t.int32
+        ep = VnlEpisode(steps.data_ptr(), done_in.data_ptr(), steps_out.data_ptr(), truncation.data_ptr(), float(episode_length))
+        rs = VnlResample(int(seed) & 0xFFFFFFFFFFFFFFFF, int(env_offset), int(start_frame_hi), float(noise_scale), reset_count.data_ptr(),
+                         scratch.data_ptr())
+        self._check(self.lib.vnl_step_training_resample(self._cref, self.model_dev.data_ptr(), self.task_dev.data_ptr(), B, ctypes.byref(a),
+                                                        action.data_ptr(), ctypes.byref(b), ctypes.byref(o), ctypes.byref(ep),
+                                                        ctypes.byref(rs), self._stream()), "vnl_step_training_resample")
 
     def reset(self, state: Dict, out_state: Dict, outputs: Dict):
         B = state["qpos"].shape[0]

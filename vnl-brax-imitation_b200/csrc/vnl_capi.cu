@@ -6,6 +6,7 @@
 // task blobs are plain device operands that may sit at a different address on every call.  No call on the step path
 // copies, allocates or synchronises.
 #include <cuda_runtime.h>
+#include <math.h>
 #include <string.h>
 
 #include "../../include/vnl_blob.h"
@@ -136,6 +137,31 @@ __global__ void clip_velocity_kernel(const float* __restrict__ qpos, int nclips,
   }
 }
 
+// The envs a step finished, in ascending order: list[0] = their count, list[1 ..] = their indices (the work list of the
+// resampling reset, env-kernel mode 5).  One CTA walks the batch 1024 envs at a time with a block-wide ballot scan, so the
+// list -- and with it which warp resets which env -- is the same on every run.
+__global__ void __launch_bounds__(1024) done_list_kernel(const float* __restrict__ done, int B, int32_t* __restrict__ list) {
+  __shared__ int wsum[32];
+  __shared__ int base;
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  if (tid == 0) base = 0;
+  __syncthreads();
+  for (int i0 = 0; i0 < B; i0 += 1024) {
+    const int i = i0 + tid;
+    const bool f = i < B && done[i] > 0.0f;
+    const unsigned m = __ballot_sync(0xffffffffu, f);
+    if (lane == 0) wsum[w] = __popc(m);
+    __syncthreads();
+    int off = base;
+    for (int k = 0; k < w; ++k) off += wsum[k];
+    if (f) list[1 + off + __popc(m & ((1u << lane) - 1u))] = i;
+    __syncthreads();
+    if (tid == 0) { int t = base; for (int k = 0; k < 32; ++k) t += wsum[k]; base = t; }
+    __syncthreads();
+  }
+  if (tid == 0) list[0] = base;
+}
+
 extern "C" {
 
 const char* vnl_version(void) { return "vnl_b200 0.1 (sm_100a)"; }
@@ -242,6 +268,31 @@ int vnl_step_training(const VnlContext* ctx, const void* model, const void* task
   p.B = B; p.nsteps = vnl_hdr_i(ctx->task_hdr, VNL_TH_NFRAMES); p.in = *in; p.out = *out; p.ctrl = action; p.outputs = *outputs;
   p.first = *first; p.first_obs = first_obs; p.episode = *episode;
   return (int)vnl::any_launch(0, p, (cudaStream_t)stream);
+}
+
+int vnl_step_training_resample(const VnlContext* ctx, const void* model, const void* task, int B, const VnlState* in, const float* action,
+                               const VnlState* out, const VnlOutputs* outputs, const VnlEpisode* episode, const VnlResample* rs,
+                               void* stream) {
+  if (B <= 0 || !in || !out || !outputs || !outputs->done || !action || !episode || !rs) return -1;
+  if (!episode->steps_in || !episode->done_in || !episode->steps_out || !episode->truncation_out) return -1;
+  if (!rs->reset_count || !rs->scratch || rs->start_frame_hi <= 0 || !(rs->noise_scale >= 0.0f) || !isfinite(rs->noise_scale)) return -1;
+  // every drawn start must have its whole reference window (frames start + 1 .. start + ref_len) inside the clip, so that no
+  // lookup of the reset has to be clamped: start_frame_hi <= clip length - ref_len (host-side header, no CUDA call)
+  if (ctx && rs->start_frame_hi > vnl_hdr_i(ctx->task_hdr, VNL_TH_CLIP_LEN) - vnl_hdr_i(ctx->task_hdr, VNL_TH_REF_LEN)) return -1;
+  vnl::Params p;
+  memset(&p, 0, sizeof(p));
+  int rc = prepare(ctx, model, task, true, B, p);
+  if (rc) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  p.B = B; p.nsteps = vnl_hdr_i(ctx->task_hdr, VNL_TH_NFRAMES); p.in = *in; p.out = *out; p.ctrl = action; p.outputs = *outputs;
+  p.episode = *episode;  // p.first stays empty: no first-state restore
+  cudaError_t err = vnl::any_launch(0, p, st);
+  if (err != cudaSuccess) return (int)err;
+  done_list_kernel<<<1, 1024, 0, st>>>(outputs->done, B, rs->scratch);
+  err = cudaGetLastError();
+  if (err != cudaSuccess) return (int)err;
+  p.rs = *rs;  // the launch geometry stays that of B envs; the kernel walks only the listed ones
+  return (int)vnl::any_launch(5, p, st);
 }
 
 // Developer hook: vnl_step with per-phase clock64 accumulation for CTA `block` into prof[32].

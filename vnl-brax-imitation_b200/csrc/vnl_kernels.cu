@@ -1629,13 +1629,28 @@ __device__ __noinline__ RewardTerms reward_state_terms(const uint32_t* tb, int n
   return r;
 }
 
+// Philox4x32-10 (Salmon et al., SC 2011; the constants of Random123): the draws of the resampling reset (DESIGN §3h)
+__device__ __forceinline__ uint4 philox4x32_10(uint4 x, uint32_t k0, uint32_t k1) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t lo0 = 0xD2511F53u * x.x, hi0 = __umulhi(0xD2511F53u, x.x);
+    const uint32_t lo1 = 0xCD9E8D57u * x.z, hi1 = __umulhi(0xCD9E8D57u, x.z);
+    x = make_uint4(hi1 ^ x.y ^ k0, lo1, hi0 ^ x.w ^ k1, lo0);
+    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+  }
+  return x;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // one env, one env group.  MODE 0 = env step, 1 = env reset tail, 2 = physics only, 3 = forward stage dump,
-// 4 = kinematics only (clip preprocessing: qpos -> normalised qpos, xpos, xquat)
+// 4 = kinematics only (clip preprocessing: qpos -> normalised qpos, xpos, xquat), 5 = reset to a fresh draw (the envs
+// listed in p.rs.scratch: the resampling AutoReset, DESIGN §3h) -- mode 1 with the qpos / qvel / clip / start frame drawn
+// in-kernel, no reward / done / metrics / stats writes
 // ---------------------------------------------------------------------------------------------------------------------
 template <int MODE>
 __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool active) {
   VNL_SMEM
+  constexpr bool kReset = MODE == 1 || MODE == 5;
   const Dims& d = c.d;
   const Lay& L = c.L;
   const int lane = LANE, tid = ETID;
@@ -1651,8 +1666,8 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
   }
   if (!active) {  // a warp without an env in this round only keeps the CTA's phase barriers company
     if (p.lockstep) {
-      const int ns = (MODE == 1 || MODE == 3) ? 1 : p.nsteps;
-      for (int st = 0; st < ns; ++st) { group_sync(p.lsgroups); if (MODE == 1 || MODE == 3) break; if (p.lockstep > 1) group_sync(p.lsgroups); }
+      const int ns = (kReset || MODE == 3) ? 1 : p.nsteps;
+      for (int st = 0; st < ns; ++st) { group_sync(p.lsgroups); if (kReset || MODE == 3) break; if (p.lockstep > 1) group_sync(p.lsgroups); }
     }
     return;
   }
@@ -1663,10 +1678,50 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
   if (lane < 16) ints[lane] = 0;
   if (pf.p) { env_sync(); if (ETID == 0) *reinterpret_cast<long long*>(smem + pf.t0o) = clock64(); }
 
+  const uint32_t* tb = p.task;
   // ---- load state -------------------------------------------------------------------------------------------------------
-  for (int i = tid; i < d.nq; i += kEnvThreads) s[L.qpos + i] = p.in.qpos[(size_t)e * d.nq + i];
-  for (int i = tid; i < d.nv; i += kEnvThreads) s[L.qvel + i] = p.in.qvel[(size_t)e * d.nv + i];
-  if (MODE == 1) {
+  int rclip = 0, rstart = 0, rcount = 0;
+  if (MODE == 5) {
+    // the draw (include/vnl_b200.h, VnlResample): block 0 = clip and start frame, blocks 1 .. = four qpos normals each;
+    // qpos / qvel = the clip row (clip, start) as the env classes' reset() stack it, plus the noise
+    const VnlResample& rs = p.rs;
+    const uint32_t k0 = (uint32_t)rs.seed, k1 = (uint32_t)(rs.seed >> 32), g = (uint32_t)(rs.env_offset + e);
+    rcount = rs.reset_count[e];
+    const uint4 x = philox4x32_10(make_uint4(g, (uint32_t)rcount, 0u, 0u), k0, k1);
+    rclip = (int)(((uint64_t)x.x * (uint64_t)max(1, vnl_hdr_i(tb, VNL_TH_NCLIPS))) >> 32);
+    rstart = (int)(((uint64_t)x.y * (uint64_t)rs.start_frame_hi) >> 32);
+    const size_t row = (size_t)rclip * vnl_hdr_i(tb, VNL_TH_CLIP_LEN) + rstart;
+    const int nj = d.nq - 7, nvj = d.nv - 6;
+    for (int i = tid; i < d.nq; i += kEnvThreads)
+      s[L.qpos + i] = i < 3 ? vnl_field_f(tb, VNL_T_POSITION)[row * 3 + i]
+                      : i < 7 ? vnl_field_f(tb, VNL_T_QUATERNION)[row * 4 + i - 3] : vnl_field_f(tb, VNL_T_JOINTS)[row * nj + i - 7];
+    for (int i = tid; i < d.nv; i += kEnvThreads)
+      s[L.qvel + i] = i < 3 ? vnl_field_f(tb, VNL_T_VELOCITY)[row * 3 + i]
+                      : i < 6 ? vnl_field_f(tb, VNL_T_ANGULAR_VELOCITY)[row * 3 + i - 3] : vnl_field_f(tb, VNL_T_JOINTS_VELOCITY)[row * nvj + i - 6];
+    env_sync();
+    if (rs.noise_scale != 0.0f) {
+      for (int j = 1 + tid; 4 * (j - 1) < d.nq; j += kEnvThreads) {  // the lanes draw the noise blocks in parallel
+        const uint4 y = philox4x32_10(make_uint4(g, (uint32_t)rcount, (uint32_t)j, 0u), k0, k1);
+        const float u[4] = {(float)((y.x >> 8) + 1u) * 0x1p-24f, (float)((y.y >> 8) + 1u) * 0x1p-24f,
+                            (float)((y.z >> 8) + 1u) * 0x1p-24f, (float)((y.w >> 8) + 1u) * 0x1p-24f};
+        float nrm[4];
+        for (int h = 0; h < 2; ++h) {
+          const float r = sqrtf(-2.0f * logf(u[2 * h]));
+          float sn, cs;
+          sincospif(2.0f * u[2 * h + 1], &sn, &cs);
+          nrm[2 * h] = r * cs; nrm[2 * h + 1] = r * sn;
+        }
+        for (int k = 0; k < 4; ++k) {
+          const int i = 4 * (j - 1) + k;
+          if (i < d.nq) s[L.qpos + i] = fmaf(rs.noise_scale, nrm[k], s[L.qpos + i]);
+        }
+      }
+    }
+  } else {
+    for (int i = tid; i < d.nq; i += kEnvThreads) s[L.qpos + i] = p.in.qpos[(size_t)e * d.nq + i];
+    for (int i = tid; i < d.nv; i += kEnvThreads) s[L.qvel + i] = p.in.qvel[(size_t)e * d.nv + i];
+  }
+  if (kReset) {
     for (int i = tid; i < d.na; i += kEnvThreads) s[L.act + i] = 0.0f;
     for (int i = tid; i < d.nv; i += kEnvThreads) s[L.warm + i] = 0.0f;
     for (int i = tid; i < d.nu; i += kEnvThreads) s[L.ctrl + i] = 0.0f;
@@ -1682,16 +1737,15 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
     }
   }
   env_sync();
-  const uint32_t* tb = p.task;
   // termination error of the PREVIOUS state and frame (envs/rodent.py:241-264, quirks Q2 / Q9): depends only on
   // inputs, so evaluate it before the physics overwrites them.
   float rtrunk = 0.0f;
   int frame_old = 0;
   // multi-clip task tables (SURVEY 8 row f4): every clip table is [nclips, T, ...]; the env's clip only offsets the row
   int fbase = 0, clip = 0;
-  if (MODE == 0 || MODE == 1) {
+  if (MODE == 0 || kReset) {
     const int nclips = max(1, vnl_hdr_i(tb, VNL_TH_NCLIPS));
-    clip = p.in.clip_id ? min(max(p.in.clip_id[e], 0), nclips - 1) : 0;
+    clip = MODE == 5 ? rclip : p.in.clip_id ? min(max(p.in.clip_id[e], 0), nclips - 1) : 0;
     fbase = clip * vnl_hdr_i(tb, VNL_TH_CLIP_LEN);
   }
   RewardTerms rt;
@@ -1722,7 +1776,7 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
 
   int* stats = ints + 4;  // [4..7]
   float* dump = (MODE == 3) ? p.dump + (size_t)e * d.dump_total : nullptr;
-  const int nsteps = (MODE == 1 || MODE == 3) ? 1 : p.nsteps;
+  const int nsteps = (kReset || MODE == 3) ? 1 : p.nsteps;
   for (int st = 0; st < nsteps; ++st) {
     // Optional lockstep: the warps of a CTA start each substep together, so that they walk the (large) instruction
     // footprint of a substep as one group instead of seven independent streams.
@@ -1732,7 +1786,7 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
       forward<MODE == 3>(so, dump, pf, last ? p.out.xpos + (size_t)e * d.nbody * 3 : nullptr,
                          last ? p.out.xquat + (size_t)e * d.nbody * 4 : nullptr, last ? p.out.qfrc_actuator + (size_t)e * d.nv : nullptr);
     }
-    if (MODE == 1 || MODE == 3) break;
+    if (kReset || MODE == 3) break;
     if (p.lockstep > 1) group_sync(p.lsgroups);
     euler(so, pf);
   }
@@ -1785,7 +1839,7 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
   const float* rjoints = vnl_field_f(tb, VNL_T_JOINTS);
   int cur_frame, sub_clip_frame;
   if (MODE == 0) { cur_frame = frame_old + 1; sub_clip_frame = p.in.sub_clip_frame[e] + 1; }
-  else { cur_frame = p.in.cur_frame[e]; sub_clip_frame = 0; }
+  else { cur_frame = MODE == 5 ? rstart : p.in.cur_frame[e]; sub_clip_frame = 0; }
   if (lane == 0) { o.cur_frame[e] = cur_frame; o.sub_clip_frame[e] = sub_clip_frame; if (o.clip_id) o.clip_id[e] = clip; }
   {
     float* obs = p.outputs.obs + (size_t)e * obs_size;
@@ -1827,6 +1881,11 @@ __device__ __forceinline__ void env_run(int so, const Params& p, int e, bool act
       }
       traj[i] = v;
     }
+  }
+  if (MODE == 5) {  // the step's reward, done, metrics and stats stay; the env's next draw takes the next counter
+    env_sync();
+    if (tid == 0) p.rs.reset_count[e] = rcount + 1;
+    return;
   }
   if (MODE == 1) {
     // info["termination_error"] of the fresh state (rodent.py:169)
@@ -1954,12 +2013,15 @@ __global__ void __launch_bounds__(kMaxEnvs * kEnvThreads, 1) vnl_env_kernel(Para
   __syncthreads();
   const int W = nt / kEnvThreads, warp = tid / kEnvThreads;  // env slots of this CTA, this thread's slot
   const int so = kCtaFloats + align4(c.d.ktab_words) + warp * c.L.total;
-  const int stride = gridDim.x * W, rounds = (p.B + stride - 1) / stride;
+  // mode 5 walks the list of envs to reset (count, then the env indices), the other modes envs 0 .. B-1.  Every CTA reads
+  // the same count, so all warps of a CTA agree on the number of rounds and the lockstep barriers stay matched.
+  const int n = MODE == 5 ? p.rs.scratch[0] : p.B;
+  const int stride = gridDim.x * W, rounds = (n + stride - 1) / stride;
   for (int r = 0; r < rounds; ++r) {
     // slot-major env numbering: a partial last round thins out EVERY CTA (fewer co-resident envs each, all faster)
     // instead of leaving whole SMs idle next to full ones
-    const int e = r * stride + warp * gridDim.x + blockIdx.x;
-    env_run<MODE>(so, p, e, e < p.B);
+    const int i = r * stride + warp * gridDim.x + blockIdx.x;
+    env_run<MODE>(so, p, MODE == 5 ? (i < n ? p.rs.scratch[1 + i] : 0) : i, i < n);
   }
 }
 
@@ -1968,6 +2030,7 @@ template __global__ void vnl_env_kernel<1>(Params);
 template __global__ void vnl_env_kernel<2>(Params);
 template __global__ void vnl_env_kernel<3>(Params);
 template __global__ void vnl_env_kernel<4>(Params);
+template __global__ void vnl_env_kernel<5>(Params);
 
 // (name, offset, size) of every array of the per-env layout, for tests/test_layout.py (sizes as make_layout reserves them)
 int layout_table(const Dims& d, LayoutEntry* out, int cap) {
@@ -2054,7 +2117,8 @@ cudaError_t launch(int mode, const Params& p, cudaStream_t stream) {
   if (li.warps_per_cta < 1) return cudaErrorInvalidConfiguration;  // one env does not fit in shared memory
   if (p.dims.env_warps != kEnvWarps) return cudaErrorInvalidValue;   // the blob's lane programs are for another group width
   if ((p.dims.stream != 0) != kStream) return cudaErrorInvalidValue;  // dispatched to the wrong instantiation
-  void (*k)(Params) = mode == 0 ? vnl_env_kernel<0> : mode == 1 ? vnl_env_kernel<1> : mode == 2 ? vnl_env_kernel<2> : mode == 3 ? vnl_env_kernel<3> : vnl_env_kernel<4>;
+  void (*k)(Params) = mode == 0 ? vnl_env_kernel<0> : mode == 1 ? vnl_env_kernel<1> : mode == 2 ? vnl_env_kernel<2> : mode == 3 ? vnl_env_kernel<3>
+                      : mode == 4 ? vnl_env_kernel<4> : vnl_env_kernel<5>;
   cudaError_t err = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, li.smem_bytes);
   if (err != cudaSuccess) return err;
   static int lockstep = -1;

@@ -56,6 +56,8 @@ struct Params {
   int work_stride;
   int lsgroups;     // lockstep groups per CTA (1 = the whole CTA)
   int lockstep;     // 0 = warps free-run, 1 = CTA barrier at every substep start, 2 = also before the integrator, 3 = at every phase boundary (default)
+  VnlResample rs;   // mode 5 (reset over a list): the draw's key and counters, the list of envs to reset in rs.scratch (last: the
+                    // parameter offsets of the other modes stay as they were)
 };
 
 struct LaunchInfo { int smem_bytes, warps_per_cta, ctas; };  // warps_per_cta = env groups per CTA

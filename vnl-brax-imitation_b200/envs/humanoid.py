@@ -124,6 +124,10 @@ class HumanoidTracking:
         qvel = np.hstack([rt.velocity[start_frame], rt.angular_velocity[start_frame], rt.joints_velocity[start_frame]]).astype(np.float32)
         return self.reset_from(qpos, qvel, start_frame)
 
+    def resample_spec(self):
+        """(start_frame_hi, noise_scale) of `reset`'s draws for the resampling AutoReset: no noise, as the reference."""
+        return self._clip_length - self._episode_length - self._ref_traj_length, 0.0
+
     def reset_from(self, qpos, qvel, start_frame) -> State:
         import torch
         dev = self.device

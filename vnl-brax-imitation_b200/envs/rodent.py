@@ -166,6 +166,12 @@ class RodentTracking:
         qvel = np.hstack([rt.velocity[start_frame], rt.angular_velocity[start_frame], rt.joints_velocity[start_frame]]).astype(np.float32)
         return self.reset_from(qpos + noise, qvel, start_frame)
 
+    def resample_spec(self):
+        """(start_frame_hi, noise_scale) of `reset`'s draws, for the resampling AutoReset on the GPU (rollout.Rollout(...,
+        autoreset="resample")): start frame uniform in [0, start_frame_hi), qpos += noise_scale * N(0, 1), clip uniform over
+        the task's clips."""
+        return self._clip_length - self._sub_clip_length - self._ref_traj_length, float(self._reset_noise_scale)
+
     def reset_from(self, qpos, qvel, start_frame, clip_id=None) -> State:
         """Reset tail after the random draws: `pipeline_init` + traj / obs / termination error."""
         import torch

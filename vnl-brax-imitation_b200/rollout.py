@@ -12,6 +12,9 @@ Both kernels write straight into the `[T(+1), B, ...]` transition buffers (each 
 them), so collecting the data costs no copies; the 2 T launches are captured once into a CUDA graph and replayed.  The
 random draws are operands (`eps_z`, `eps_a`): the caller fills the static draw buffers before every unroll, as the
 reference splits a fresh key per step (`acting.py:72-73`).  No CPU fallback: both kernels are required.
+
+`autoreset="resample"` replaces brax's AutoReset (restore the cached first state) by a fresh reset of every finished episode:
+new clip, start frame and reset noise, drawn on the device inside the env step (`vnl_step_training_resample`, DESIGN §3h).
 """
 from __future__ import annotations
 
@@ -21,9 +24,12 @@ from . import train_kernels as tk
 
 
 class Rollout:
-    def __init__(self, env, policy, first_state, unroll_length: int, episode_length: float, use_graph: bool = True):
-        """`first_state`: the State returned by env.reset(...) — it is also the state AutoReset restores (brax caches
-        `first_pipeline_state` / `first_obs` in info at reset)."""
+    def __init__(self, env, policy, first_state, unroll_length: int, episode_length: float, use_graph: bool = True,
+                 autoreset: str = "first", seed: int = 0, env_offset: int = 0):
+        """`first_state`: the State returned by env.reset(...).  `autoreset="first"`: it is also the state AutoReset restores (brax
+        caches `first_pipeline_state` / `first_obs` in info at reset).  `autoreset="resample"`: a finished episode restarts from a
+        fresh draw of `env.resample_spec()`'s distribution, keyed by `seed`, the global env index (`env_offset` + row: this
+        process's first env in a sharded run) and the env's own reset counter."""
         import torch
 
         self.torch = t = torch
@@ -36,10 +42,23 @@ class Rollout:
         if (obs, traj) != (policy.obs_size, policy.traj_size):
             raise ValueError("policy and env disagree on obs / traj sizes")
         f = lambda *s: t.zeros(*s, dtype=t.float32, device=dev)
-        self.first = {k: v.clone() for k, v in first_state.pipeline_state.items()}
-        self.first_obs = first_state.obs.clone()
+        if autoreset not in ("first", "resample"):
+            raise ValueError(f"autoreset must be 'first' or 'resample', not {autoreset!r}")
+        self.autoreset = autoreset
+        self.first = self.first_obs = self.reset_count = None
+        if autoreset == "first":
+            self.first = {k: v.clone() for k, v in first_state.pipeline_state.items()}
+            self.first_obs = first_state.obs.clone()
+        else:
+            if not hasattr(env, "resample_spec"):
+                raise ValueError(f"autoreset='resample': {type(env).__name__} has no resample_spec()")
+            self.start_frame_hi, self.noise_scale = env.resample_spec()
+            self.seed, self.env_offset = int(seed), int(env_offset)
+            # fixed addresses for the captured graph: each env's resets so far (the draw's counter) and the done list
+            self.reset_count = t.zeros(B, dtype=t.int32, device=dev)
+            self.scratch = t.zeros(B + 1, dtype=t.int32, device=dev)
         # env state ping-pong + episode counters of EpisodeWrapper / AutoResetWrapper
-        self.state = [dict({k: v.clone() for k, v in self.first.items()}, cur_frame=first_state.info["cur_frame"].clone(),
+        self.state = [dict({k: v.clone() for k, v in first_state.pipeline_state.items()}, cur_frame=first_state.info["cur_frame"].clone(),
                            sub_clip_frame=first_state.info["sub_clip_frame"].clone()), self.eng.alloc_state(B)]
         if first_state.info.get("clip_idx") is not None:  # multi-clip env: every env keeps tracking its own clip
             self.state[0]["clip_id"] = first_state.info["clip_idx"].clone()
@@ -70,9 +89,14 @@ class Rollout:
             self.policy(self.traj[t], self.obs[t], self.eps_z[t], None if self.eps_a is None else self.eps_a[t], out=pout)  # eps_a None: the mode
             out = {"obs": self.obs[t + 1], "traj": self.traj[t + 1], "reward": self.reward[t], "done": self.done[t],
                    "metrics": self.metrics[t]}
-            self.eng.step_training(self.state[cur], self.action[t], self.state[1 - cur], out, self.first, self.first_obs,
-                                   self.steps, self.done_prev if t == 0 else self.done[t - 1], self.steps, self.truncation[t],
-                                   self.episode_length)
+            done_in = self.done_prev if t == 0 else self.done[t - 1]
+            if self.autoreset == "first":
+                self.eng.step_training(self.state[cur], self.action[t], self.state[1 - cur], out, self.first, self.first_obs,
+                                       self.steps, done_in, self.steps, self.truncation[t], self.episode_length)
+            else:
+                self.eng.step_training_resample(self.state[cur], self.action[t], self.state[1 - cur], out, self.steps, done_in, self.steps,
+                                                self.truncation[t], self.episode_length, self.reset_count, self.scratch, self.seed,
+                                                self.env_offset, self.start_frame_hi, self.noise_scale)
             cur = 1 - cur
         # carry: the next unroll starts from the last state / obs / traj / done
         self.done_prev.copy_(self.done[self.T - 1])
@@ -118,9 +142,11 @@ class Rollout:
         """Start over from a fresh `env.reset(...)` state WITHOUT changing any buffer address (a captured graph stays valid): the
         evaluator resets its envs before every evaluation (acting.py:111-113)."""
         for k, v in first_state.pipeline_state.items():
-            self.first[k].copy_(v)
+            if self.first is not None:
+                self.first[k].copy_(v)
             self.state[self.cur][k].copy_(v)
-        self.first_obs.copy_(first_state.obs)
+        if self.first_obs is not None:
+            self.first_obs.copy_(first_state.obs)
         self.state[self.cur]["cur_frame"].copy_(first_state.info["cur_frame"])
         self.state[self.cur]["sub_clip_frame"].copy_(first_state.info["sub_clip_frame"])
         if "clip_id" in self.state[self.cur] and first_state.info.get("clip_idx") is not None:
@@ -134,14 +160,21 @@ class Rollout:
     # ---- checkpoint --------------------------------------------------------------------------------------------------
     def state_dict(self) -> Dict[str, "np.ndarray"]:
         """The carry into the next unroll, on the host: the env state the captured launches read first ("state/<key>", clip_id only
-        where the env has one), the AutoReset state ("first/<key>", "first_obs"), the obs / traj the next unroll starts from, the
-        episode step counters and the last step's done flags."""
+        where the env has one), the AutoReset state ("first/<key>", "first_obs"; "reset_count" in resample mode), the obs / traj
+        the next unroll starts from, the episode step counters and the last step's done flags."""
         carried = self.launches and not getattr(self, "_fresh", False)  # generate_unroll would copy obs[T] / traj[T] to row 0
         h = lambda x: x.detach().cpu().numpy().copy()
-        out = {"state/" + k: h(v) for k, v in self.state[self.cur].items()}
-        out.update(("first/" + k, h(v)) for k, v in self.first.items())
-        out.update(first_obs=h(self.first_obs), obs=h(self.obs[self.T] if carried else self.obs[0]),
-                   traj=h(self.traj[self.T] if carried else self.traj[0]), steps=h(self.steps), done_prev=h(self.done_prev))
+        return {k: h(v) for k, v in self._carry(carried).items()}
+
+    def _carry(self, carried=False) -> Dict[str, "torch.Tensor"]:
+        out = {"state/" + k: v for k, v in self.state[self.cur].items()}
+        if self.autoreset == "first":
+            out.update(("first/" + k, v) for k, v in self.first.items())
+            out["first_obs"] = self.first_obs
+        else:
+            out["reset_count"] = self.reset_count
+        out.update(obs=self.obs[self.T] if carried else self.obs[0], traj=self.traj[self.T] if carried else self.traj[0], steps=self.steps,
+                   done_prev=self.done_prev)
         return out
 
     def load_state_dict(self, sd) -> None:
@@ -149,9 +182,7 @@ class Rollout:
         valid, and the reset kernel does not run."""
         import numpy as np
         t = self.torch
-        dst = {"state/" + k: v for k, v in self.state[self.cur].items()}
-        dst.update(("first/" + k, v) for k, v in self.first.items())
-        dst.update(first_obs=self.first_obs, obs=self.obs[0], traj=self.traj[0], steps=self.steps, done_prev=self.done_prev)
+        dst = self._carry()
         if set(dst) != set(sd):
             raise ValueError(f"rollout state keys differ: missing {sorted(set(dst) - set(sd))}, unexpected {sorted(set(sd) - set(dst))}")
         for k, x in dst.items():
@@ -164,14 +195,17 @@ class Rollout:
     # -----------------------------------------------------------------------------------------------------------------
     def _snapshot(self):
         s = self.state[self.cur]
-        return ({k: v.clone() for k, v in s.items()}, self.steps.clone(), self.done_prev.clone())
+        return ({k: v.clone() for k, v in s.items()}, self.steps.clone(), self.done_prev.clone(),
+                None if self.reset_count is None else self.reset_count.clone())
 
     def _restore(self, snap):
-        st, steps, done_prev = snap
+        st, steps, done_prev, reset_count = snap
         for k, v in st.items():
             self.state[self.cur][k].copy_(v)
         self.steps.copy_(steps)
         self.done_prev.copy_(done_prev)
+        if reset_count is not None:
+            self.reset_count.copy_(reset_count)
 
     @property
     def env_state(self) -> Dict[str, "torch.Tensor"]:

@@ -9,6 +9,8 @@ the Evaluator.  Schedule (`schedule`): brax's -- an optional evaluation at step 
 `checkpoint_dir` is set), rank 0 evaluates and calls `progress_fn`.  `restore_checkpoint_path` resumes a run from a checkpoint of the
 same configuration: the state is copied into the freshly built buffers and the remaining epochs of the schedule run (DESIGN §3g).
 
+`autoreset="resample"` restarts finished training episodes from fresh draws (DESIGN §3h) instead of the first states.
+
 Out of scope: several unrolls per training step (batch_size * num_minibatches must equal num_envs), action_repeat other than 1,
 num_resets_per_eval, network depths other than 2 + 2, re-sharding a checkpoint to another world size.
 """
@@ -25,13 +27,14 @@ from . import policy as pol
 from . import sharding
 
 POLICIES = ("3xtf32", "tf32", "bf16")
+AUTORESETS = ("first", "resample")
 
 # train()'s keyword arguments after num_timesteps (brax PPO names) and their defaults
 DEFAULTS = dict(
     episode_length=150, num_envs=8192, num_eval_envs=128, unroll_length=20, batch_size=256, num_minibatches=32, num_updates_per_batch=16,
     num_evals=2, learning_rate=6e-4, entropy_cost=1e-4, discounting=0.9, reward_scaling=1.0, gae_lambda=0.95, clipping_epsilon=0.2,
     kl_weight=1e-4, normalize_advantage=True, deterministic_eval=False, encoder_layer_sizes=(256, 128), decoder_layer_sizes=(128, 256),
-    latent_size=64, value_layer_sizes=(1024, 1024), policy="3xtf32", seed=0)
+    latent_size=64, value_layer_sizes=(1024, 1024), policy="3xtf32", seed=0, autoreset="first")
 
 # meta.json entries a checkpoint must share with the run that restores it (buffer sizes, sharding, schedule)
 MATCH_FIELDS = ("format", "env", "obs_size", "traj_size", "action_size", "policy_shapes", "value_shapes", "world_size", "num_envs",
@@ -68,6 +71,10 @@ def check_config(environment, cfg, world_size: int, eval_env=None) -> None:
         raise ValueError("eval_env: obs / traj / action sizes differ from environment's")
     if cfg["policy"] not in POLICIES:
         raise ValueError(f"policy must be one of {POLICIES}, not {cfg['policy']!r}")
+    if cfg["autoreset"] not in AUTORESETS:
+        raise ValueError(f"autoreset must be one of {AUTORESETS}, not {cfg['autoreset']!r}")
+    if cfg["autoreset"] == "resample" and not hasattr(environment, "resample_spec"):
+        raise ValueError(f"autoreset='resample': {type(environment).__name__} has no resample_spec() (the draws of its reset)")
     if cfg["batch_size"] * cfg["num_minibatches"] != cfg["num_envs"]:
         raise ValueError("batch_size * num_minibatches must equal num_envs: one unroll per training step (several unrolls per "
                          f"training step are not supported); got {cfg['batch_size']} * {cfg['num_minibatches']} != {cfg['num_envs']}")
@@ -95,9 +102,12 @@ def run_meta(environment, cfg, sched, world_size: int) -> dict:
     """meta.json of a checkpoint of this run, without the schedule position."""
     obs, traj, nu = _sizes(environment)
     shapes, vshapes = network_shapes(environment, cfg)
+    layout = {k: cfg[k] for k in LAYOUT_KEYS}
+    if cfg["autoreset"] == "resample":  # only then: checkpoints of the default mode keep the layout they always had
+        layout["autoreset"] = "resample"
     return dict(format=ckpt.FORMAT_VERSION, env=type(environment).__name__, obs_size=obs, traj_size=traj, action_size=nu,
                 policy_shapes={k: list(s) for k, s in shapes.items()}, value_shapes={k: list(s) for k, s in vshapes.items()},
-                world_size=int(world_size), num_envs=int(cfg["num_envs"]), layout={k: cfg[k] for k in LAYOUT_KEYS},
+                world_size=int(world_size), num_envs=int(cfg["num_envs"]), layout=layout,
                 schedule=dict(sched), hyperparameters={k: list(v) if isinstance(v, tuple) else v for k, v in cfg.items()})
 
 
@@ -122,8 +132,8 @@ class Run:
         self.env, self.cfg, self.rank, self.world = environment, dict(cfg), int(rank), int(world_size)
         self.device = dev = str(environment.device)
         B = cfg["num_envs"] // self.world
+        lo, hi = sharding.shard_range(cfg["num_envs"], self.rank, self.world)
         if first_state is None:
-            lo, hi = sharding.shard_range(cfg["num_envs"], self.rank, self.world)
             first_state = environment.reset(np.random.default_rng(cfg["seed"]), batch_size=cfg["num_envs"])
             if (lo, hi) != (0, cfg["num_envs"]):
                 first_state = _shard(first_state, lo, hi)
@@ -133,7 +143,8 @@ class Run:
         vp = lrn.init_value_params(rng, vshapes)
         self.stats = normalizer.RunningStatistics(environment.engine.obs_size, dev)
         self.policy = self._new_policy(pp, dev, self.stats.mean, self.stats.std)
-        self.rollout = rollout.Rollout(environment, self.policy, first_state, cfg["unroll_length"], float(cfg["episode_length"]), use_graph=True)
+        self.rollout = rollout.Rollout(environment, self.policy, first_state, cfg["unroll_length"], float(cfg["episode_length"]), use_graph=True,
+                                       autoreset=cfg["autoreset"], seed=cfg["seed"], env_offset=lo)
         hp = {k: cfg[k] for k in ("learning_rate", "entropy_cost", "discounting", "reward_scaling", "gae_lambda", "clipping_epsilon",
                                   "normalize_advantage", "kl_weight")}
         self.learner = lrn.PPOLearner(pp, vp, cfg["unroll_length"], B // cfg["num_minibatches"], device=dev, x3=learner_x3, **hp)
@@ -249,7 +260,7 @@ def train(environment, num_timesteps: int, episode_length: int = 150, num_envs: 
           learning_rate: float = 6e-4, entropy_cost: float = 1e-4, discounting: float = 0.9, reward_scaling: float = 1.0,
           gae_lambda: float = 0.95, clipping_epsilon: float = 0.2, kl_weight: float = 1e-4, normalize_advantage: bool = True,
           deterministic_eval: bool = False, encoder_layer_sizes=(256, 128), decoder_layer_sizes=(128, 256), latent_size: int = 64,
-          value_layer_sizes=(1024, 1024), policy: str = "3xtf32", seed: int = 0, eval_env=None,
+          value_layer_sizes=(1024, 1024), policy: str = "3xtf32", seed: int = 0, autoreset: str = "first", eval_env=None,
           progress_fn: Callable = lambda step, metrics: None, policy_params_fn: Callable = lambda step, make_policy, params: None,
           checkpoint_dir: Optional[str] = None, restore_checkpoint_path: Optional[str] = None):
     """PPO training of the intention network on `environment` (RodentTracking / HumanoidTracking: an env whose info carries the
@@ -261,7 +272,9 @@ def train(environment, num_timesteps: int, episode_length: int = 150, num_envs: 
 
     Under torchrun with a process group, envs are sharded over the ranks and only rank 0 evaluates and calls the callbacks.
     `checkpoint_dir`: a checkpoint after every epoch (checkpoint.py); `restore_checkpoint_path`: resume from one (same
-    configuration and world size) and run the remaining epochs."""
+    configuration and world size) and run the remaining epochs.  `autoreset`: "first" (the reference: a finished episode restarts
+    from the env's first state, brax's AutoReset) or "resample" (from a fresh draw of clip, start frame and reset noise on the
+    device, DESIGN §3h); evaluation always resets to first states."""
     cfg = {k: v for k, v in locals().items() if k in DEFAULTS}
     cfg.update((k, tuple(cfg[k])) for k in ("encoder_layer_sizes", "decoder_layer_sizes", "value_layer_sizes"))
     rank, world = _rank_world()
