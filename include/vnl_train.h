@@ -95,6 +95,24 @@ int vnl_policy_sample(const float* logits, int ld, const float* eps_a, const flo
 int vnl_eval_metrics(int T, int B, int nm, const float* metrics, const float* reward, const float* done, float* episode_metrics, float* active,
                      float* episode_steps, void* stream);
 
+/* Per-clip evaluation over what vnl_eval_metrics produced.  clip_id [B] (int32) assigns each env a clip; NULL = every env is
+ * clip 0; an env whose id is outside [0, nclips) is counted nowhere.  Both run one CTA per clip, accumulate in double in a fixed
+ * order (no atomics): two calls on the same inputs are bit-identical.
+ *
+ * vnl_eval_clip_stats: per clip c, mean[c, k] and std[c, k] (population std, jnp.std) over the clip's envs of nm + 2 columns:
+ * episode_metrics[:, 0..nm] (each metric, then the reward) and episode_steps; count[c] = the clip's envs.  An empty clip gets
+ * count 0 and NaN mean / std.  episode_metrics [B, nm + 1], episode_steps [B]; mean / std [nclips, nm + 2], count [nclips]. */
+int vnl_eval_clip_stats(int B, int nm, const float* episode_metrics, const float* episode_steps, const int* clip_id, int nclips, float* mean,
+                        float* std, int* count, void* stream);
+/* vnl_eval_frame_profile: bins the first episode of each env by the clip frame its reward read.  Step t < min(episode_steps[b], T)
+ * of env b read frame f = clamp(start_frame[b] + t, 0, clip_len - 1); it adds metrics[t, b, 0..nm) and reward[t, b] to
+ * frame_sum[c, f, 0..nm] and 1 to frame_count[c, f], c = clip_id[b].  Every bin is written, the empty ones included; the sums run
+ * in ascending env order, then ascending t.  Summing a clip's frames gives its episode sums of vnl_eval_metrics.
+ * metrics [T, B, nm] (not NULL even when nm = 0), reward [T, B], episode_steps / start_frame [B];
+ * frame_sum [nclips, clip_len, nm + 1], frame_count [nclips, clip_len] (int32). */
+int vnl_eval_frame_profile(int T, int B, int nm, const float* metrics, const float* reward, const float* episode_steps, const int* start_frame,
+                           const int* clip_id, int nclips, int clip_len, float* frame_sum, int* frame_count, void* stream);
+
 /* Loss, part 1 (per row; intention_losses.py:149-166,189): brax NormalTanhDistribution on logits [rows, 2 nu]:
  *   target_lp[r] = log_prob(logits, raw_action), ent[r] = entropy(logits) with the sample loc + scale * eps_ent;
  *   termination[r] = (1 - discount[r]) * (1 - truncation[r]); rewards_s[r] = reward[r] * reward_scaling. */

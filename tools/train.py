@@ -5,7 +5,8 @@ summary: training env-steps/s, eval time per evaluation, checkpoint write time a
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/train.py
   env: ENV=rodent|humanoid (rodent)  CLIP=standing|moving (standing; the humanoid's packaged clip)  ENVS (8192, global)
        NUM_TIMESTEPS (2 training steps per epoch)  NUM_EVALS (3)  MINIBATCHES (32)  UPDATES (16)  EVAL_ENVS (128)
-       CKPT_DIR (none: no checkpoints)  RESUME (a step_<n> directory, or "latest" for the newest one in CKPT_DIR)"""
+       CKPT_DIR (none: no checkpoints)  RESUME (a step_<n> directory, or "latest" for the newest one in CKPT_DIR)
+       PER_CLIP_EVAL=1: per-clip evaluation (its per-clip / per-frame arrays are not printed)"""
 import importlib
 import json
 import os
@@ -50,7 +51,8 @@ def main():
     B, nmb = int(os.environ.get("ENVS", 8192)), int(os.environ.get("MINIBATCHES", 32))
     num_evals = int(os.environ.get("NUM_EVALS", 3))
     cfg = dict(num_envs=B, batch_size=B // nmb, num_minibatches=nmb, num_updates_per_batch=int(os.environ.get("UPDATES", 16)),
-               num_evals=num_evals, num_eval_envs=int(os.environ.get("EVAL_ENVS", 128)))
+               num_evals=num_evals, num_eval_envs=int(os.environ.get("EVAL_ENVS", 128)),
+               per_clip_eval=os.environ.get("PER_CLIP_EVAL", "0") == "1")
     per_step = B * 20
     num_timesteps = int(os.environ.get("NUM_TIMESTEPS", 2 * max(num_evals - 1, 1) * per_step))
     ckpt_dir, resume = os.environ.get("CKPT_DIR") or None, os.environ.get("RESUME") or None

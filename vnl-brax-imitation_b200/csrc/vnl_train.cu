@@ -1,7 +1,8 @@
 // vnl_train.cu -- the non-GEMM kernels of the PPO update (SURVEY section 8 row f2; C ABI in include/vnl_train.h):
 // minibatch gather, obs normalisation, relu + LayerNorm forward / backward, swish, reparameterisation and its backward with
 // the KL term, bias / weighted column sums, the value head, the PPO loss (brax NormalTanhDistribution log-prob / entropy,
-// advantage normalisation, clipped surrogate, value loss) with its gradients, Adam and the 3xTF32 operand split.
+// advantage normalisation, clipped surrogate, value loss) with its gradients, Adam and the 3xTF32 operand split; and the
+// evaluator's reductions (EvalWrapper's episode sums, their per-clip statistics and per-frame profiles).
 // All of them are HBM-bound row / elementwise passes: coalesced fp32, one warp per row where a row reduction is needed,
 // fixed reduction trees inside a block; cross-block accumulation (bias / LayerNorm parameter gradients, loss scalars) uses
 // red.global.add.  Reference: ppo_imitation/intention_losses.py:91-202, intention_policy_network.py:20-105, brax
@@ -305,6 +306,122 @@ __global__ void eval_metrics_kernel(int T, int B, int nm, const float* __restric
   episode_steps[b] = steps;
 }
 
+// Per-clip evaluation (vnl_eval_clip_stats / vnl_eval_frame_profile): one CTA per clip.  The CTA walks the batch kClipThreads envs
+// at a time and compacts the envs of its clip with a block ballot scan (ascending env order, as done_list_kernel).  Which thread adds
+// which value, and in what order, depends only on the inputs and the block size, never on launch timing: two calls are bit-identical.
+constexpr int kClipThreads = 256;
+constexpr int kClipWarps = kClipThreads / 32;
+
+// This thread's slot in the ascending list of the envs of chunk [i0, i0 + kClipThreads) that belong to clip c (-1: its env does
+// not); `len` = the list's length.  clip_id NULL: every env is clip 0.  The caller writes its slot, then synchronises.
+__device__ __forceinline__ int clip_chunk_slot(const int* __restrict__ clip_id, int B, int i0, int c, int* wsum, int& len) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, i = i0 + threadIdx.x;
+  const bool mine = i < B && (clip_id ? clip_id[i] == c : c == 0);
+  const unsigned bal = __ballot_sync(0xffffffffu, mine);
+  if (lane == 0) wsum[w] = __popc(bal);
+  __syncthreads();
+  int off = 0;
+  len = 0;
+  for (int q = 0; q < kClipWarps; ++q) { off += q < w ? wsum[q] : 0; len += wsum[q]; }
+  return mine ? off + __popc(bal & ((1u << lane) - 1u)) : -1;
+}
+
+// Per clip: mean and population std (two passes, double) of nm + 2 columns over the clip's envs: episode_metrics[:, 0..nm], then
+// episode_steps.  Lane k of every warp holds column k; warp w adds entries w, w + kClipWarps, ... of each chunk's list, and the
+// warps' partials are added in warp order.
+__global__ void __launch_bounds__(kClipThreads) eval_clip_stats_kernel(int B, int nm, const float* __restrict__ episode_metrics,
+                                                                      const float* __restrict__ episode_steps, const int* __restrict__ clip_id,
+                                                                      float* __restrict__ mean, float* __restrict__ sd, int* __restrict__ count) {
+  __shared__ int s_env[kClipThreads], wsum[kClipWarps];
+  __shared__ double red[kClipWarps][32], mom[2][32];
+  const int c = blockIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5, ncol = nm + 2, ld = nm + 1;
+  int total = 0;
+  for (int pass = 0; pass < 2; ++pass) {  // 0: sums -> means, 1: squared deviations from them
+    const double m = pass && lane < ncol ? mom[0][lane] : 0.0;
+    double s = 0.0;
+    total = 0;
+    for (int i0 = 0; i0 < B; i0 += kClipThreads) {
+      int len;
+      const int slot = clip_chunk_slot(clip_id, B, i0, c, wsum, len);
+      if (slot >= 0) s_env[slot] = i0 + threadIdx.x;
+      __syncthreads();
+      if (lane < ncol)
+        for (int j = w; j < len; j += kClipWarps) {
+          const int b = s_env[j];
+          const double d = (double)(lane < ld ? episode_metrics[(size_t)b * ld + lane] : episode_steps[b]) - m;
+          s += pass ? d * d : d;
+        }
+      total += len;
+      __syncthreads();  // s_env and wsum are rewritten by the next chunk
+    }
+    if (lane < ncol) red[w][lane] = s;
+    __syncthreads();
+    if (threadIdx.x < ncol) {
+      double a = 0.0;
+      for (int q = 0; q < kClipWarps; ++q) a += red[q][threadIdx.x];
+      mom[pass][threadIdx.x] = a / total;
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x < ncol) {
+    mean[(size_t)c * ncol + threadIdx.x] = total ? (float)mom[0][threadIdx.x] : nanf("");
+    sd[(size_t)c * ncol + threadIdx.x] = total ? (float)sqrt(mom[1][threadIdx.x]) : nanf("");
+  }
+  if (threadIdx.x == 0) count[c] = total;
+}
+
+// Per clip and clip frame: sums of the metrics and the reward over the first-episode steps whose reward read that frame.  Thread f
+// walks each chunk's list in order and adds, per env, its steps t (ascending) with clamp(start + t, 0, L - 1) == f: no two threads
+// write the same bin.  Clips longer than the block go round in groups of kClipThreads frames.
+__global__ void __launch_bounds__(kClipThreads) eval_frame_profile_kernel(int T, int B, int nm, const float* __restrict__ metrics,
+                                                                         const float* __restrict__ reward, const float* __restrict__ episode_steps,
+                                                                         const int* __restrict__ start_frame, const int* __restrict__ clip_id,
+                                                                         int L, float* __restrict__ frame_sum, int* __restrict__ frame_count) {
+  __shared__ int s_env[kClipThreads], s_start[kClipThreads], s_n[kClipThreads], wsum[kClipWarps];
+  const int c = blockIdx.x, ld = nm + 1;
+  for (int f0 = 0; f0 < L; f0 += kClipThreads) {
+    const int f = f0 + threadIdx.x;
+    double acc[15], racc = 0.0;  // static indices only: the metric sums stay in registers
+#pragma unroll
+    for (int k = 0; k < 15; ++k) acc[k] = 0.0;
+    int cnt = 0;
+    for (int i0 = 0; i0 < B; i0 += kClipThreads) {
+      int len;
+      const int slot = clip_chunk_slot(clip_id, B, i0, c, wsum, len);
+      if (slot >= 0) {
+        const int i = i0 + threadIdx.x;
+        s_env[slot] = i;
+        s_start[slot] = start_frame[i];
+        s_n[slot] = min((int)episode_steps[i], T);
+      }
+      __syncthreads();
+      if (f < L)
+        for (int j = 0; j < len; ++j) {
+          const int b = s_env[j], s = s_start[j], n = s_n[j];
+          // the steps that bin to f: t = f - s inside the clip, and every t that clamps to f at either end
+          const int lo = max(f == 0 ? 0 : f - s, 0), hi = min(f == L - 1 ? n - 1 : f - s, n - 1);
+          for (int t = lo; t <= hi; ++t) {
+            const size_t r = (size_t)t * B + b;
+#pragma unroll
+            for (int k = 0; k < 15; ++k)
+              if (k < nm) acc[k] += (double)metrics[r * nm + k];
+            racc += (double)reward[r];
+            ++cnt;
+          }
+        }
+      __syncthreads();  // the list is rebuilt for the next chunk
+    }
+    if (f < L) {
+      float* out = frame_sum + ((size_t)c * L + f) * ld;
+#pragma unroll
+      for (int k = 0; k < 15; ++k)
+        if (k < nm) out[k] = (float)acc[k];
+      out[nm] = (float)racc;
+      frame_count[(size_t)c * L + f] = cnt;
+    }
+  }
+}
+
 // mean and population std of `rows` values (jnp.mean / jnp.std), one block, fixed order
 __global__ void mean_std_kernel(const float* __restrict__ x, int rows, float* __restrict__ out2) {
   __shared__ double r1[32], r2[32];
@@ -517,6 +634,22 @@ int vnl_eval_metrics(int T, int B, int nm, const float* metrics, const float* re
                      float* episode_steps, void* stream) {
   if (T <= 0 || B <= 0 || nm < 0 || nm > 15 || !metrics || !reward || !done || !episode_metrics || !active || !episode_steps) return -1;
   eval_metrics_kernel<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(T, B, nm, metrics, reward, done, episode_metrics, active, episode_steps);
+  return rc();
+}
+
+int vnl_eval_clip_stats(int B, int nm, const float* episode_metrics, const float* episode_steps, const int* clip_id, int nclips, float* mean,
+                        float* std, int* count, void* stream) {
+  if (B < 1 || nm < 0 || nm > 15 || nclips < 1 || !episode_metrics || !episode_steps || !mean || !std || !count) return -1;
+  eval_clip_stats_kernel<<<nclips, kClipThreads, 0, (cudaStream_t)stream>>>(B, nm, episode_metrics, episode_steps, clip_id, mean, std, count);
+  return rc();
+}
+
+int vnl_eval_frame_profile(int T, int B, int nm, const float* metrics, const float* reward, const float* episode_steps, const int* start_frame,
+                           const int* clip_id, int nclips, int clip_len, float* frame_sum, int* frame_count, void* stream) {
+  if (T < 1 || B < 1 || nm < 0 || nm > 15 || nclips < 1 || clip_len < 1) return -1;
+  if (!metrics || !reward || !episode_steps || !start_frame || !frame_sum || !frame_count) return -1;
+  eval_frame_profile_kernel<<<nclips, kClipThreads, 0, (cudaStream_t)stream>>>(T, B, nm, metrics, reward, episode_steps, start_frame, clip_id,
+                                                                               clip_len, frame_sum, frame_count);
   return rc();
 }
 

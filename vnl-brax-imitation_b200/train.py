@@ -10,6 +10,7 @@ the Evaluator.  Schedule (`schedule`): brax's -- an optional evaluation at step 
 same configuration: the state is copied into the freshly built buffers and the remaining epochs of the schedule run (DESIGN §3g).
 
 `autoreset="resample"` restarts finished training episodes from fresh draws (DESIGN §3h) instead of the first states.
+`per_clip_eval=True` evaluates a fixed clip x start-frame sweep and adds per-clip and per-frame results (DESIGN §3i).
 
 Out of scope: several unrolls per training step (batch_size * num_minibatches must equal num_envs), action_repeat other than 1,
 num_resets_per_eval, network depths other than 2 + 2, re-sharding a checkpoint to another world size.
@@ -34,9 +35,10 @@ DEFAULTS = dict(
     episode_length=150, num_envs=8192, num_eval_envs=128, unroll_length=20, batch_size=256, num_minibatches=32, num_updates_per_batch=16,
     num_evals=2, learning_rate=6e-4, entropy_cost=1e-4, discounting=0.9, reward_scaling=1.0, gae_lambda=0.95, clipping_epsilon=0.2,
     kl_weight=1e-4, normalize_advantage=True, deterministic_eval=False, encoder_layer_sizes=(256, 128), decoder_layer_sizes=(128, 256),
-    latent_size=64, value_layer_sizes=(1024, 1024), policy="3xtf32", seed=0, autoreset="first")
+    latent_size=64, value_layer_sizes=(1024, 1024), policy="3xtf32", seed=0, autoreset="first", per_clip_eval=False)
 
-# meta.json entries a checkpoint must share with the run that restores it (buffer sizes, sharding, schedule)
+# meta.json entries a checkpoint must share with the run that restores it (buffer sizes, sharding, schedule); per_clip_eval is not
+# among them: it changes what an evaluation reports, not the state a checkpoint holds
 MATCH_FIELDS = ("format", "env", "obs_size", "traj_size", "action_size", "policy_shapes", "value_shapes", "world_size", "num_envs",
                 "layout", "schedule")
 LAYOUT_KEYS = ("episode_length", "num_eval_envs", "unroll_length", "batch_size", "num_minibatches", "num_updates_per_batch", "policy")
@@ -75,6 +77,12 @@ def check_config(environment, cfg, world_size: int, eval_env=None) -> None:
         raise ValueError(f"autoreset must be one of {AUTORESETS}, not {cfg['autoreset']!r}")
     if cfg["autoreset"] == "resample" and not hasattr(environment, "resample_spec"):
         raise ValueError(f"autoreset='resample': {type(environment).__name__} has no resample_spec() (the draws of its reset)")
+    if cfg["per_clip_eval"]:
+        from .evaluator import sweep_layout
+        try:
+            sweep_layout(eval_env or environment, cfg["num_eval_envs"])
+        except ValueError as e:
+            raise ValueError(f"per_clip_eval=True: {e}") from None
     if cfg["batch_size"] * cfg["num_minibatches"] != cfg["num_envs"]:
         raise ValueError("batch_size * num_minibatches must equal num_envs: one unroll per training step (several unrolls per "
                          f"training step are not supported); got {cfg['batch_size']} * {cfg['num_minibatches']} != {cfg['num_envs']}")
@@ -154,7 +162,7 @@ class Run:
         self.evaluator = None
         if (self.rank == 0) if evaluate is None else evaluate:
             self.evaluator = evaluator.Evaluator(eval_env or environment, self.policy, cfg["num_eval_envs"], cfg["episode_length"],
-                                                 seed=cfg["seed"], deterministic=cfg["deterministic_eval"])
+                                                 seed=cfg["seed"], deterministic=cfg["deterministic_eval"], per_clip=cfg["per_clip_eval"])
 
     def _new_policy(self, params, device, mean, std):
         if self.cfg["policy"] == "bf16":
@@ -260,7 +268,8 @@ def train(environment, num_timesteps: int, episode_length: int = 150, num_envs: 
           learning_rate: float = 6e-4, entropy_cost: float = 1e-4, discounting: float = 0.9, reward_scaling: float = 1.0,
           gae_lambda: float = 0.95, clipping_epsilon: float = 0.2, kl_weight: float = 1e-4, normalize_advantage: bool = True,
           deterministic_eval: bool = False, encoder_layer_sizes=(256, 128), decoder_layer_sizes=(128, 256), latent_size: int = 64,
-          value_layer_sizes=(1024, 1024), policy: str = "3xtf32", seed: int = 0, autoreset: str = "first", eval_env=None,
+          value_layer_sizes=(1024, 1024), policy: str = "3xtf32", seed: int = 0, autoreset: str = "first", per_clip_eval: bool = False,
+          eval_env=None,
           progress_fn: Callable = lambda step, metrics: None, policy_params_fn: Callable = lambda step, make_policy, params: None,
           checkpoint_dir: Optional[str] = None, restore_checkpoint_path: Optional[str] = None):
     """PPO training of the intention network on `environment` (RodentTracking / HumanoidTracking: an env whose info carries the
@@ -274,7 +283,9 @@ def train(environment, num_timesteps: int, episode_length: int = 150, num_envs: 
     `checkpoint_dir`: a checkpoint after every epoch (checkpoint.py); `restore_checkpoint_path`: resume from one (same
     configuration and world size) and run the remaining epochs.  `autoreset`: "first" (the reference: a finished episode restarts
     from the env's first state, brax's AutoReset) or "resample" (from a fresh draw of clip, start frame and reset noise on the
-    device, DESIGN §3h); evaluation always resets to first states."""
+    device, DESIGN §3h); evaluation always resets to first states.  `per_clip_eval`: every evaluation runs the same clip x
+    start-frame sweep (evaluator.clip_sweep; num_eval_envs a multiple of the clip count) and the metrics add eval/clip/* [nclips]
+    and eval/frame/* [nclips, clip_len] numpy arrays (DESIGN §3i)."""
     cfg = {k: v for k, v in locals().items() if k in DEFAULTS}
     cfg.update((k, tuple(cfg[k])) for k in ("encoder_layer_sizes", "decoder_layer_sizes", "value_layer_sizes"))
     rank, world = _rank_world()

@@ -9,7 +9,7 @@ from . import _lib
 TRAIN_EXPORTS = ("vnl_gemm_tf32", "vnl_gemm_tf32_ex", "vnl_split_tf32", "vnl_gather_rows", "vnl_obs_normalize", "vnl_relu_ln_fwd", "vnl_relu_ln_bwd",
                  "vnl_swish_fwd", "vnl_swish_bwd", "vnl_reparam_fwd", "vnl_heads_bwd", "vnl_colsum", "vnl_rowdot", "vnl_outer", "vnl_outer_swish_bwd", "vnl_gather_scalars",
                  "vnl_ppo_rows", "vnl_ppo_loss_bwd", "vnl_adam_tick", "vnl_adam", "vnl_policy_sample", "vnl_eval_metrics",
-                 "vnl_metrics_accumulate")
+                 "vnl_eval_clip_stats", "vnl_eval_frame_profile", "vnl_metrics_accumulate")
 _bound = None
 
 
@@ -39,6 +39,8 @@ def lib():
         L.vnl_ppo_loss_bwd.argtypes = [v, i, v, v, i, i, v, v, v, v, v, v, f, f, i, v, i, v, v, v, v]
         L.vnl_policy_sample.argtypes = [v, i, v, v, i, i, v, v, v, v, v]
         L.vnl_eval_metrics.argtypes = [i, i, i, v, v, v, v, v, v, v]
+        L.vnl_eval_clip_stats.argtypes = [i, i, v, v, v, i, v, v, v, v]
+        L.vnl_eval_frame_profile.argtypes = [i, i, i, v, v, v, v, v, i, i, v, v, v]
         L.vnl_adam_tick.argtypes = [v, f, f, v, v]
         L.vnl_adam.argtypes = [v, v, v, v, sz, f, f, f, f, i, f, v, v]
         L.vnl_metrics_accumulate.argtypes = [v, i, v, v]
