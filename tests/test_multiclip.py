@@ -110,6 +110,26 @@ def test_multiclip_step_equals_single_clip_step_of_each_envs_clip(rodent, oracle
 
 
 @pytest.mark.gpu
+def test_host_stepper_on_multiclip_env_equals_env_step(rodent):
+    """hostio.HostStepper steps every env against its own clip, as env.step does: the same obs / traj / reward / done, bit for bit."""
+    import torch
+    envs, rod = pkg("envs"), pkg("envs.rodent")
+    multi = envs.RodentMultiClipTracking(reference_clips=_variants(rodent["clip"], 4), model=rodent["model"], device="cuda:0",
+                                         **rod.RODENT_ENV_ARGS)
+    B, K = 96, 4
+    s = multi.reset(np.random.default_rng(8), batch_size=B)
+    assert set(s.info["clip_idx"].tolist()) == {0, 1, 2, 3}
+    stepper = pkg("hostio").HostStepper(multi, s, autoreset=False)
+    acts = torch.tensor(np.random.default_rng(9).uniform(-1, 1, size=(K, B, multi.action_size)).astype(np.float32)).pin_memory()
+    for t in range(K):
+        host = stepper.step(acts[t])
+        s = multi.step(s, acts[t].cuda())
+        torch.cuda.synchronize()
+        for k, want in (("obs", s.obs), ("traj", s.info["traj"]), ("reward", s.reward), ("done", s.done)):
+            assert torch.equal(host[k], want.cpu()), (t, k)
+
+
+@pytest.mark.gpu
 def test_process_clip_on_gpu_matches_host_restatement_and_reference_pickle(rodent, golden):
     """`vnl_process_clip` (kinematics pass of the env kernel per frame + finite-difference velocity kernel) against
     (a) `clip.process_clip_qpos` (float64 FK, the host restatement of mjx_preprocess.py:43-107) and (b) the fields of the

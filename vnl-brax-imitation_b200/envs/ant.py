@@ -29,7 +29,7 @@ import numpy as np
 from .. import clip as clipm
 from .. import mjcf
 from .. import model_blob as mb
-from .base import PipelineState, State
+from .base import State, TrackingEnv
 
 _DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "data")
 
@@ -61,7 +61,12 @@ def ant_task_tables(model: mjcf.Model, reference_clip, *, clip_length=250, episo
     return blob, state_size, traj_size
 
 
-class AntTracking:
+class AntTracking(TrackingEnv):
+    """`reset`: `AntTracking.reset` (`ant.py:76-123`), start frame 0 and no reset noise, no draws; `step`: `AntTracking.step`
+    (`ant.py:167-216`), one fused launch + the obs concatenation."""
+
+    metric_keys = ANT_METRIC_KEYS
+
     def __init__(self, params=None, healthy_z_range=(0.2, 1.0), reset_noise_scale=1e-2, clip_length: int = 250,
                  episode_length: int = 150, ref_traj_length: int = 5, termination_threshold: float = 0.9,
                  body_error_multiplier: float = 1.0, n_frames: int = 5, device: str = "cuda:0",
@@ -70,84 +75,26 @@ class AntTracking:
         if episode_length > clip_length:
             raise ValueError("episode_length cannot be greater than clip_length!")  # ant.py:73-74
         if model is None:
-            model = mjcf.load_ant(mjcf_path, params["solver"], params["iterations"], params["ls_iterations"])
-        else:
-            model.solver = {"cg": mjcf.SOLVER_CG, "newton": mjcf.SOLVER_NEWTON}[params["solver"].lower()]
-            model.iterations, model.ls_iterations = int(params["iterations"]), int(params["ls_iterations"])
+            model = mjcf.load_ant(mjcf_path)
         if reference_clip is None:
             if "clip_path" in params and os.path.exists(params["clip_path"]):
                 reference_clip = clipm.load_pickle(params["clip_path"])  # ant.py:70-71
             else:
                 reference_clip = clipm.tiled_clip(model, model.arrays["init_qpos"], 256)
-        self.model, self._ref_traj = model, reference_clip
-        self._clip_length, self._episode_length, self._ref_traj_length = clip_length, episode_length, ref_traj_length
-        self._n_frames = n_frames
-        self.task_blob, self._state_size, self._traj_size = ant_task_tables(
+        task_blob, state_size, traj_size = ant_task_tables(
             model, reference_clip, clip_length=clip_length, episode_length=episode_length, ref_traj_length=ref_traj_length,
             termination_threshold=termination_threshold, body_error_multiplier=body_error_multiplier,
             healthy_z_range=healthy_z_range, n_frames=n_frames)
-        self.model_blob = mb.build_model_blob(model)
-        from .._lib import Engine  # raises if the CUDA library / a GPU is missing: no CPU fallback
-        self.engine = Engine(self.model_blob, self.task_blob, device=device)
-        self.device = self.engine.device
-
-    @property
-    def dt(self) -> float:
-        return self.model.timestep * self._n_frames
-
-    @property
-    def action_size(self) -> int:
-        return self.model.nu
-
-    @property
-    def observation_size(self) -> int:
-        return self._traj_size + self._state_size
+        super().__init__(model, task_blob, reference_clip, traj_size + state_size, solver=params["solver"],
+                         iterations=params["iterations"], ls_iterations=params["ls_iterations"], n_frames=n_frames,
+                         start_frame_hi=None, reset_noise=None, device=device)
 
     def _wrap(self, st, out, step: bool) -> State:
         import torch
-        ps = PipelineState({k: st[k] for k in ("qpos", "qvel", "act", "qacc_warmstart", "xpos", "xquat", "subtree_com",
-                                              "qfrc_actuator")})
-        m = out["metrics"]
-        metrics = {"rcom": m[:, 0], "rvel": m[:, 1], "rtrunk": m[:, 2], "rquat": m[:, 3], "ract": m[:, 4],
-                   "termination_error": m[:, 6]}
-        traj = torch.nan_to_num(out["traj"]) if step else out["traj"]  # ant.py:199 nan_to_num(obs); reset applies none
-        obs = torch.cat([traj, out["obs"]], dim=1)                     # ant.py:300-309
-        info = dict(cur_frame=st["cur_frame"], sub_clip_frame=st["sub_clip_frame"], termination_error=m[:, 6],
-                    solver_stats=out["stats"])
-        return State(ps, obs, out["reward"], out["done"], metrics, info)
-
-    def reset(self, rng=None, batch_size: int = 1, start_frame=None) -> State:
-        """`AntTracking.reset` (`ant.py:76-123`): start_frame is fixed to 0 and no noise is applied by the reference."""
-        B = int(batch_size)
-        start_frame = np.zeros(B, dtype=np.int32) if start_frame is None else np.asarray(start_frame, dtype=np.int32).reshape(B)
-        rt = self._ref_traj
-        qpos = np.hstack([rt.position[start_frame], rt.quaternion[start_frame], rt.joints[start_frame]]).astype(np.float32)
-        qvel = np.hstack([rt.velocity[start_frame], rt.angular_velocity[start_frame], rt.joints_velocity[start_frame]]).astype(np.float32)
-        return self.reset_from(qpos, qvel, start_frame)
+        state = super()._wrap(st, out, step)
+        traj = state.info.pop("traj")
+        traj = torch.nan_to_num(traj) if step else traj  # ant.py:199 nan_to_num(obs); reset applies none
+        return state.replace(obs=torch.cat([traj, state.obs], dim=1))  # ant.py:300-309
 
     def reset_to_frame(self, start_frame, batch_size: int = 1) -> State:  # ant.py:125-165
         return self.reset(batch_size=batch_size, start_frame=np.full(int(batch_size), int(start_frame), dtype=np.int32))
-
-    def reset_from(self, qpos, qvel, start_frame) -> State:
-        import torch
-        dev = self.device
-        B = qpos.shape[0]
-        st_in = dict(qpos=torch.as_tensor(qpos, dtype=torch.float32, device=dev).contiguous(),
-                     qvel=torch.as_tensor(qvel, dtype=torch.float32, device=dev).contiguous(),
-                     cur_frame=torch.as_tensor(start_frame, dtype=torch.int32, device=dev).contiguous())
-        st, out = self.engine.alloc_state(B), self.engine.alloc_outputs(B)
-        self.engine.reset(st_in, st, out)
-        return self._wrap(st, out, step=False)
-
-    def step(self, state: State, action) -> State:
-        """`AntTracking.step` (`ant.py:167-216`): one fused launch + the obs concatenation."""
-        import torch
-        ps = state.pipeline_state
-        B = ps["qpos"].shape[0]
-        st_in = dict(ps)
-        st_in["cur_frame"] = state.info["cur_frame"]
-        st_in["sub_clip_frame"] = state.info["sub_clip_frame"]
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device).reshape(B, self.model.nu).contiguous()
-        st, out = self.engine.alloc_state(B), self.engine.alloc_outputs(B)
-        self.engine.step(st_in, action, st, out)
-        return self._wrap(st, out, step=True)

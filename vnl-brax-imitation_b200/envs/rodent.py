@@ -11,14 +11,14 @@ Differences from the reference that are forced by the host language, nothing els
 from __future__ import annotations
 
 import os
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, Optional, Sequence
 
 import numpy as np
 
 from .. import clip as clipm
 from .. import mjcf
 from .. import model_blob as mb
-from .base import PipelineState, State
+from .base import METRIC_KEYS, State, TrackingEnv  # noqa: F401  (METRIC_KEYS: imported from here by callers)
 
 # `configs/env_config.yaml:30-106` (rodent env_args)
 RODENT_ENV_ARGS = dict(
@@ -37,8 +37,6 @@ RODENT_ENV_ARGS = dict(
                  "wrist_R", "finger_R"],
     center_of_mass="torso",
 )
-
-METRIC_KEYS = ("rcom", "rvel", "rtrunk", "rquat", "ract", "rapp", "termination_error")
 
 _DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "data")
 
@@ -80,7 +78,10 @@ class _Sys:
         self.model = m
 
 
-class RodentTracking:
+class RodentTracking(TrackingEnv):
+    """`reset`: `RodentTracking.reset` (`envs/rodent.py:119-176`), start frame then reset noise; `step`: `RodentTracking.step`
+    (`envs/rodent.py:178-239`).  Every env carries `info["clip_idx"]`, the clip it tracks (0 on a single clip)."""
+
     def __init__(self, reference_clip=None, end_eff_names: Sequence[str] = (), appendage_names: Sequence[str] = (),
                  walker_body_names: Sequence[str] = (), joint_names: Sequence[str] = (), center_of_mass: str = "torso",
                  mjcf_path: str = "./assets/rodent.xml", scale_factor: float = 0.9, solver: str = "cg", iterations: int = 6,
@@ -91,116 +92,29 @@ class RodentTracking:
         if sub_clip_length > clip_length:
             raise ValueError("episode_length cannot be greater than clip_length!")  # rodent.py:116-117
         if model is None:
-            model = mjcf.load_rodent(mjcf_path, scale_factor, solver, iterations, ls_iterations)
-        else:
-            model.solver = {"cg": mjcf.SOLVER_CG, "newton": mjcf.SOLVER_NEWTON}[solver.lower()]
-            model.iterations, model.ls_iterations = int(iterations), int(ls_iterations)
-        self.model = model
+            model = mjcf.load_rodent(mjcf_path, scale_factor)
         self.sys = _Sys(model, n_frames)
-        self._n_frames = n_frames
-        self._healthy_z_range = healthy_z_range
-        self._reset_noise_scale = reset_noise_scale
-        self._termination_threshold = termination_threshold
-        self._body_error_multiplier = body_error_multiplier
-        self._clip_length = clip_length
-        self._sub_clip_length = sub_clip_length
-        self._ref_traj_length = ref_traj_length
-        self.task_blob, self._ref_traj, idx, self._obs_size, self._traj_size = rodent_task_tables(
+        task_blob, ref_traj, idx, obs_size, _ = rodent_task_tables(
             model, reference_clip, end_eff_names=end_eff_names, appendage_names=appendage_names,
             walker_body_names=walker_body_names, joint_names=joint_names, center_of_mass=center_of_mass,
             clip_length=clip_length, sub_clip_length=sub_clip_length, ref_traj_length=ref_traj_length,
             termination_threshold=termination_threshold, body_error_multiplier=body_error_multiplier,
             healthy_z_range=healthy_z_range, n_frames=n_frames)
-        self._end_eff_idx, self._app_idx, self._com_idx = idx["end_eff_idx"], idx["app_idx"], idx["com_idx"]
-        self._body_idxs, self._joint_idxs = idx["body_idxs"], idx["joint_idxs"]
-        self.model_blob = mb.build_model_blob(model)
-        from .._lib import Engine  # raises if the CUDA library / a GPU is missing: no CPU fallback
-        self.engine = Engine(self.model_blob, self.task_blob, device=device)
-        self.device = self.engine.device
+        self._body_idxs = idx["body_idxs"]
+        super().__init__(model, task_blob, ref_traj, obs_size, solver=solver, iterations=iterations, ls_iterations=ls_iterations,
+                         n_frames=n_frames, start_frame_hi=clip_length - sub_clip_length - ref_traj_length,
+                         reset_noise=reset_noise_scale, device=device)
 
-    # ---- brax Env surface --------------------------------------------------------------------
-    @property
-    def dt(self) -> float:
-        return self.sys.dt
-
-    @property
-    def action_size(self) -> int:
-        return self.sys.nu
-
-    @property
-    def observation_size(self) -> int:
-        return self._obs_size
-
-    @property
-    def metric_keys(self):
-        """Names of `State.metrics` (columns METRIC_KEYS.index(name) of the step kernel's metrics output)."""
-        return METRIC_KEYS
-
-    @property
-    def backend(self) -> str:
-        return "vnl_b200"
-
-    def _wrap(self, st: Dict, out: Dict) -> State:
-        ps = PipelineState({k: st[k] for k in ("qpos", "qvel", "act", "qacc_warmstart", "xpos", "xquat", "subtree_com",
-                                              "qfrc_actuator")})
-        m = out["metrics"]
-        metrics = {k: m[:, i] for i, k in enumerate(METRIC_KEYS)}
-        info = dict(cur_frame=st["cur_frame"], sub_clip_frame=st["sub_clip_frame"], traj=out["traj"],
-                    termination_error=m[:, 6], solver_stats=out["stats"], clip_idx=st["clip_id"])
-        return State(ps, out["obs"], out["reward"], out["done"], metrics, info)
-
-    def reset(self, rng, batch_size: int = 1, start_frame=None) -> State:
-        """`RodentTracking.reset` (`envs/rodent.py:119-176`) for `batch_size` envs."""
-        import torch
-
-        if not isinstance(rng, np.random.Generator):
-            rng = np.random.default_rng(rng)
-        B = int(batch_size)
-        hi = self._clip_length - self._sub_clip_length - self._ref_traj_length
-        if start_frame is None:
-            start_frame = rng.integers(0, hi, size=B)
-        start_frame = np.asarray(start_frame, dtype=np.int32).reshape(B)
-        noise = (self._reset_noise_scale * rng.standard_normal((B, self.sys.nq))).astype(np.float32)
-        rt = self._ref_traj
-        qpos = np.hstack([rt.position[start_frame], rt.quaternion[start_frame], rt.joints[start_frame]]).astype(np.float32)
-        qvel = np.hstack([rt.velocity[start_frame], rt.angular_velocity[start_frame], rt.joints_velocity[start_frame]]).astype(np.float32)
-        return self.reset_from(qpos + noise, qvel, start_frame)
+    def _wrap(self, st: Dict, out: Dict, step: bool) -> State:
+        state = super()._wrap(st, out, step)
+        state.info["clip_idx"] = st["clip_id"]
+        return state
 
     def resample_spec(self):
         """(start_frame_hi, noise_scale) of `reset`'s draws, for the resampling AutoReset on the GPU (rollout.Rollout(...,
         autoreset="resample")): start frame uniform in [0, start_frame_hi), qpos += noise_scale * N(0, 1), clip uniform over
         the task's clips."""
-        return self._clip_length - self._sub_clip_length - self._ref_traj_length, float(self._reset_noise_scale)
-
-    def reset_from(self, qpos, qvel, start_frame, clip_id=None) -> State:
-        """Reset tail after the random draws: `pipeline_init` + traj / obs / termination error."""
-        import torch
-
-        dev = self.device
-        B = qpos.shape[0]
-        st_in = dict(qpos=torch.as_tensor(qpos, dtype=torch.float32, device=dev).contiguous(),
-                     qvel=torch.as_tensor(qvel, dtype=torch.float32, device=dev).contiguous(),
-                     cur_frame=torch.as_tensor(start_frame, dtype=torch.int32, device=dev).contiguous())
-        if clip_id is not None:
-            st_in["clip_id"] = torch.as_tensor(clip_id, dtype=torch.int32, device=dev).contiguous()
-        st, out = self.engine.alloc_state(B), self.engine.alloc_outputs(B)
-        self.engine.reset(st_in, st, out)
-        return self._wrap(st, out)
-
-    def step(self, state: State, action) -> State:
-        """`RodentTracking.step` (`envs/rodent.py:178-239`): one fused launch."""
-        import torch
-
-        ps = state.pipeline_state
-        B = ps["qpos"].shape[0]
-        st_in = dict(ps)
-        st_in["cur_frame"] = state.info["cur_frame"]
-        st_in["sub_clip_frame"] = state.info["sub_clip_frame"]
-        st_in["clip_id"] = state.info.get("clip_idx")
-        action = torch.as_tensor(action, dtype=torch.float32, device=self.device).reshape(B, self.sys.nu).contiguous()
-        st, out = self.engine.alloc_state(B), self.engine.alloc_outputs(B)
-        self.engine.step(st_in, action, st, out)
-        return self._wrap(st, out)
+        return self._start_frame_hi, float(self._reset_noise)
 
 
 def stack_clips(clips):
@@ -225,24 +139,6 @@ class RodentMultiClipTracking(RodentTracking):
             reference_clips = stack_clips(reference_clips)
         super().__init__(reference_clip=reference_clips, **kw)
         self.nclips = int(np.asarray(self._ref_traj.position).shape[0])
-
-    def reset(self, rng, batch_size: int = 1, start_frame=None, clip_id=None) -> State:
-        if not isinstance(rng, np.random.Generator):
-            rng = np.random.default_rng(rng)
-        B = int(batch_size)
-        if clip_id is None:
-            clip_id = rng.integers(0, self.nclips, size=B)
-        clip_id = np.asarray(clip_id, dtype=np.int32).reshape(B)
-        hi = self._clip_length - self._sub_clip_length - self._ref_traj_length
-        if start_frame is None:
-            start_frame = rng.integers(0, hi, size=B)
-        start_frame = np.asarray(start_frame, dtype=np.int32).reshape(B)
-        noise = (self._reset_noise_scale * rng.standard_normal((B, self.sys.nq))).astype(np.float32)
-        rt = self._ref_traj
-        g = lambda a: np.asarray(a)[clip_id, start_frame]
-        qpos = np.hstack([g(rt.position), g(rt.quaternion), g(rt.joints)]).astype(np.float32)
-        qvel = np.hstack([g(rt.velocity), g(rt.angular_velocity), g(rt.joints_velocity)]).astype(np.float32)
-        return self.reset_from(qpos + noise, qvel, start_frame, clip_id)
 
 
 def process_clips_gpu(model: mjcf.Model, mocap_qpos, max_qvel: float = 20.0, dt: float = 0.02, device: str = "cuda:0"):

@@ -21,7 +21,7 @@ import numpy as np
 
 from . import model_blob as mb
 from . import train_kernels as tk
-from .envs.rodent import METRIC_KEYS
+from .envs.base import METRIC_KEYS
 
 
 def clip_sweep(nclips: int, num_eval_envs: int, start_frame_hi: int):
@@ -67,7 +67,7 @@ class Evaluator:
         f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)
         # the env's metric names (the humanoid has no appendage term); the step kernel writes every column of METRIC_KEYS, all of
         # which are folded, and only the env's own are reported
-        self.metric_keys = tuple(getattr(eval_env, "metric_keys", METRIC_KEYS))
+        self.metric_keys = tuple(eval_env.metric_keys)
         self.episode_metrics, self.active, self.episode_steps = f(self.B, len(METRIC_KEYS) + 1), f(self.B), f(self.B)
         self.rollout = None
         self.per_clip = bool(per_clip)

@@ -12,7 +12,8 @@ from __future__ import annotations
 
 from typing import Dict
 
-from ._lib import STATE_F, STATE_I
+from ._lib import STATE_F
+from .envs.base import engine_state
 
 HOST_FIELDS = ("obs", "traj", "reward", "done")
 
@@ -31,10 +32,7 @@ class HostStepper:
         self.first = {k: ps[k].clone() for k in STATE_F}
         self.first_obs = state0.obs.clone()
         self.autoreset = autoreset
-        cur = {k: ps[k].clone() for k in STATE_F}
-        cur["cur_frame"] = state0.info["cur_frame"].clone()
-        cur["sub_clip_frame"] = state0.info["sub_clip_frame"].clone()
-        self.bufs = [cur, eng.alloc_state(B)]
+        self.bufs = [{k: v.clone() for k, v in engine_state(state0).items()}, eng.alloc_state(B)]
         self.out = eng.alloc_outputs(B)
         self.episode_length = float(episode_length)
         if self.episode_length > 0 and not autoreset:

@@ -398,6 +398,19 @@ def _solref(vals: Optional[np.ndarray]) -> np.ndarray:
     return out
 
 
+def set_solver(m: Model, solver: Optional[str] = None, iterations: Optional[int] = None,
+               ls_iterations: Optional[int] = None) -> Model:
+    """The solver overrides the reference envs apply to a compiled model (`envs/rodent.py:55-63`, `envs/humanoid.py:43-54`);
+    None keeps the model's value."""
+    if solver is not None:
+        m.solver = {"cg": SOLVER_CG, "newton": SOLVER_NEWTON}[solver.lower()]
+    if iterations is not None:
+        m.iterations = int(iterations)
+    if ls_iterations is not None:
+        m.ls_iterations = int(ls_iterations)
+    return m
+
+
 def compile_model(root: ET.Element, *, name: str = "", solver: Optional[str] = None,
                   iterations: Optional[int] = None, ls_iterations: Optional[int] = None,
                   eulerdamp: Optional[bool] = None) -> Model:
@@ -427,18 +440,13 @@ def compile_model(root: ET.Element, *, name: str = "", solver: Optional[str] = N
         m.iterations = int(opt.get("iterations", m.iterations))
         m.ls_iterations = int(opt.get("ls_iterations", m.ls_iterations))
         if opt.get("solver"):
-            m.solver = {"cg": SOLVER_CG, "newton": SOLVER_NEWTON}[opt.get("solver").lower()]
+            set_solver(m, opt.get("solver"))
         if opt.get("cone", "pyramidal") != "pyramidal":
             raise NotImplementedError("only the pyramidal cone is on the reference path")
         flag = opt.find("flag")
         if flag is not None and flag.get("eulerdamp") == "disable":
             m.eulerdamp = False
-    if solver is not None:
-        m.solver = {"cg": SOLVER_CG, "newton": SOLVER_NEWTON}[solver.lower()]
-    if iterations is not None:
-        m.iterations = int(iterations)
-    if ls_iterations is not None:
-        m.ls_iterations = int(ls_iterations)
+    set_solver(m, solver, iterations, ls_iterations)
     if eulerdamp is not None:
         m.eulerdamp = bool(eulerdamp)
 

@@ -21,6 +21,7 @@ from __future__ import annotations
 from typing import Dict, Optional
 
 from . import train_kernels as tk
+from .envs.base import engine_state
 
 
 class Rollout:
@@ -58,10 +59,7 @@ class Rollout:
             self.reset_count = t.zeros(B, dtype=t.int32, device=dev)
             self.scratch = t.zeros(B + 1, dtype=t.int32, device=dev)
         # env state ping-pong + episode counters of EpisodeWrapper / AutoResetWrapper
-        self.state = [dict({k: v.clone() for k, v in first_state.pipeline_state.items()}, cur_frame=first_state.info["cur_frame"].clone(),
-                           sub_clip_frame=first_state.info["sub_clip_frame"].clone()), self.eng.alloc_state(B)]
-        if first_state.info.get("clip_idx") is not None:  # multi-clip env: every env keeps tracking its own clip
-            self.state[0]["clip_id"] = first_state.info["clip_idx"].clone()
+        self.state = [{k: v.clone() for k, v in engine_state(first_state).items()}, self.eng.alloc_state(B)]
         self.cur = 0
         self.steps, self.done_prev = f(B), f(B)
         # transition buffers (time-major, like `data` after the swapaxes of intention_losses.py:133)
@@ -101,7 +99,7 @@ class Rollout:
         # carry: the next unroll starts from the last state / obs / traj / done
         self.done_prev.copy_(self.done[self.T - 1])
         if cur != self.cur:  # odd T: bring the state back to the buffer the (captured) launches read first
-            # (its keys: without a clip index in the first state -- single-clip envs such as the humanoid -- there is no clip_id to restore)
+            # (its keys: engine_state's of the first state -- no clip_id where the env carries no clip index, as the humanoid)
             for k, v in self.state[self.cur].items():
                 v.copy_(self.state[cur][k])
 
@@ -141,16 +139,12 @@ class Rollout:
     def reset_to(self, first_state) -> None:
         """Start over from a fresh `env.reset(...)` state WITHOUT changing any buffer address (a captured graph stays valid): the
         evaluator resets its envs before every evaluation (acting.py:111-113)."""
-        for k, v in first_state.pipeline_state.items():
-            if self.first is not None:
-                self.first[k].copy_(v)
+        for k, v in engine_state(first_state).items():
             self.state[self.cur][k].copy_(v)
-        if self.first_obs is not None:
+        if self.first is not None:
+            for k, v in self.first.items():
+                v.copy_(first_state.pipeline_state[k])
             self.first_obs.copy_(first_state.obs)
-        self.state[self.cur]["cur_frame"].copy_(first_state.info["cur_frame"])
-        self.state[self.cur]["sub_clip_frame"].copy_(first_state.info["sub_clip_frame"])
-        if "clip_id" in self.state[self.cur] and first_state.info.get("clip_idx") is not None:
-            self.state[self.cur]["clip_id"].copy_(first_state.info["clip_idx"])
         self.steps.zero_()
         self.done_prev.zero_()
         self.obs[0].copy_(first_state.obs)

@@ -121,10 +121,8 @@ def run_meta(environment, cfg, sched, world_size: int) -> dict:
 
 def _shard(state, lo: int, hi: int):
     """The rows [lo, hi) of a reset State (the fields Rollout reads), as their own tensors."""
-    from .envs.base import PipelineState, State
-    info = {k: state.info[k][lo:hi].clone() for k in ("cur_frame", "sub_clip_frame", "traj")}
-    if state.info.get("clip_idx") is not None:
-        info["clip_idx"] = state.info["clip_idx"][lo:hi].clone()
+    from .envs.base import ENGINE_INFO, PipelineState, State
+    info = {k: state.info[k][lo:hi].clone() for k in (*ENGINE_INFO, "traj") if k in state.info}
     return State(PipelineState({k: v[lo:hi].clone() for k, v in state.pipeline_state.items()}), state.obs[lo:hi].clone(), None, None,
                  {}, info)
 
